@@ -21,7 +21,10 @@ on several GPUs (every rank must cut the minimizer space the same way).
 `cpu_baseline`  the unmodified reference's prlRead2HashTable (oracle/_ref) on a bounded sample of the same reads;
 `parity_checked`  the sliced build's table fingerprint equals the single-pass insert's on this workload (untimed).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--config C2] [--pairs P] [--impl reference]
+--dump-outputs DIR  writes the table the last timed step built (dump_outputs) as .npy files, so that two builds of the
+          project can be compared output for output on the same seeded inputs (one GPU).
+
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--config C2] [--pairs P] [--impl reference] [--dump-outputs DIR]
 """
 from __future__ import annotations
 
@@ -175,6 +178,67 @@ def reference_run(cfg_d: dict, sample_reads: np.ndarray, threads: int):
     return info
 
 
+def reference_built(cfg_d: dict) -> bool:
+    """oracle/_ref is built only where the SOAPdenovo-Trans sources are at hand (oracle/Makefile)."""
+    from oracle import oracle as O
+    return O.ref_binary(1 if cfg_d["key_words"] == 1 else 4) is not None
+
+
+DUMP_BYTES = 60_000_000     # all files of --dump-outputs together (under 64 MB)
+DUMP_SEED = 0x5D7D06B5E1EC7ED
+
+
+def _halves(a) -> np.ndarray:
+    """uint64 -> float64 [..., 2] (high, low 32 bits): exact, unlike a plain cast."""
+    a = np.asarray(a, dtype=np.uint64)
+    return np.stack([(a >> np.uint64(32)).astype(np.float64), (a & np.uint64(0xFFFFFFFF)).astype(np.float64)], axis=-1)
+
+
+def dump_outputs(pkg, g, out_dir: str) -> dict:
+    """Writes what the handle holds after a step, i.e. what a caller of the timed path receives, as float64 .npy:
+      stats           [n_instances, n_nodes, n_reads]
+      table_checksum  [4, 2] sdtgpu_table_checksum (include/sdtgpu.h) as 32-bit halves: the fingerprint of the whole table
+      nodes_key       [n, 2 x device key words] 32-bit halves, most significant first; nodes_count, nodes_l_links,
+      nodes_rword, nodes_ordinal [n]: the n nodes with the smallest seeded hash of their key, sorted by key.
+    The sample is chosen by content, so it does not depend on where a build keeps a node; n is as large as DUMP_BYTES allows.
+    Returns {name: shape}."""
+    st = g.stats()
+    W = int(st.device_key_words)
+    nodes = g.export_nodes(1)
+    cap = min(len(nodes), (DUMP_BYTES - (1 << 16)) // (8 * (2 * W + 4)))
+    hs, idx = [], []
+    chunk = 1 << 24
+    with np.errstate(over="ignore"):
+        for a in range(0, len(nodes), chunk):
+            key = nodes["key"][a:a + chunk]
+            h = np.full(len(key), DUMP_SEED, dtype=np.uint64)
+            for q in range(4 - W, 4):
+                h = pkg.synth.mix64(h ^ key[:, q])
+            keep = np.argpartition(h, cap - 1)[:cap] if len(h) > cap else np.arange(len(h))
+            hs.append(h[keep])
+            idx.append(keep + a)
+    if cap:
+        h, idx = np.concatenate(hs), np.concatenate(idx)
+        sel = nodes[idx[np.argsort(h, kind="stable")[:cap]]]
+        sel = sel[np.lexsort(tuple(sel["key"][:, q] for q in range(3, 3 - W, -1)))]
+    else:
+        sel = nodes[:0]
+    del nodes
+    out = {
+        "stats": np.array([st.n_instances, st.n_nodes, st.n_reads], dtype=np.float64),
+        "table_checksum": _halves(g.table_checksum()),
+        "nodes_key": _halves(sel["key"][:, 4 - W:]).reshape(len(sel), 2 * W),
+        "nodes_count": sel["count"].astype(np.float64),
+        "nodes_l_links": sel["l_links"].astype(np.float64),
+        "nodes_rword": sel["rword"].astype(np.float64),
+        "nodes_ordinal": sel["ordinal"].astype(np.float64),
+    }
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    return {name: list(a.shape) for name, a in out.items()}
+
+
 def host_sample(cfg_d: dict, n_pairs: int) -> np.ndarray:
     """The first n_pairs pairs of the workload, generated on the host (bit-identical to the device generator)."""
     import sdt_pkg
@@ -258,7 +322,13 @@ def main():
     ap.add_argument("--scaling", default="weak", choices=["weak", "strong"],
                     help="several GPUs: weak = the config's reads PER GPU (the driver's contract); strong = the config's reads in total, split over the GPUs")
     ap.add_argument("--hint", type=int, default=-1, help="capacity_hint for the handle (-1: none on one GPU, the closed-form estimate on several)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the table the last one built to DIR/<name>.npy (float64, one GPU, see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and (args.impl != "ours" or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        ap.error("--dump-outputs needs --impl ours on one GPU")
     if args.path == "auto":
         args.path = "sliced"
     import sdt_pkg
@@ -528,6 +598,9 @@ def main():
         if tj.get("key_words") == st.device_key_words:
             traffic = tj["dram_bytes_per_instance"] * inst_per_launch
             traffic_src = tj.get("source")
+    if args.dump_outputs:      # before e2e, which empties the handle again
+        shapes = dump_outputs(pkg, g, args.dump_outputs)
+        print(f"[bench] outputs of the last timed step written to {args.dump_outputs}: {shapes}", file=sys.stderr)
 
     # ---- e2e: HOST (pinned) buffers, H2D inside the timed region, counters read back (D2H) every step.
     # N = 1: straight through the C ABI's host entry point (sdtgpu_push_reads).  N > 1: every rank
@@ -583,7 +656,12 @@ def main():
 
     # ---- the reference on a bounded sample, and our whole path FROM FILES on the same sample (like for like)
     cpu, from_files = None, None
-    if rank == 0 and world == 1 and not args.no_cpu_baseline:
+    cpu_leg = rank == 0 and world == 1 and not args.no_cpu_baseline
+    if cpu_leg and not reference_built(cfg_d):
+        print("[bench] cpu_baseline and e2e_from_files skipped: the reference binaries (oracle/_ref) are not built; "
+              "oracle/Makefile builds them from the SOAPdenovo-Trans sources (REF=<src>)", file=sys.stderr)
+        cpu_leg = False
+    if cpu_leg:
         threads = ref_threads()
         sample = unpack_reads(d_packed[: 2 * sample_pairs].cpu().numpy(), L)
         info = reference_run(cfg_d, sample, threads)
