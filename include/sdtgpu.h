@@ -170,6 +170,44 @@ int sdtgpu_build_kmersets (const sdtgpu_node *nodes, uint64_t n_nodes, int key_w
 			   const uint64_t *set_last_ordinal /* [thrd_num] or NULL */, sdtgpu_kmerset **sets);
 void sdtgpu_free_kmersets (sdtgpu_kmerset **sets, int thrd_num);
 
+/* ---- lookups in the finished table (the reference's searchKmer / search_kmerset, prlRead2path.c:363, which
+ * prlRead2edge and prlRead2Ctg call once per read window).
+ * Valid only after sdtgpu_finalize: before it both calls return SDTGPU_ESTATE, and sdtgpu_reset puts the handle
+ * back into that state.  The first lookup after finalize builds a read-only index over the table (16 bytes per
+ * node; SDTGPU_ENOMEM if it does not fit, SDTGPU_ERANGE for a table of 2^32 - 1 slots or more), which is kept until
+ * sdtgpu_reset or sdtgpu_destroy; a lookup after reset, push and finalize sees the new table.
+ * Both calls only enqueue work on sdtgpu_stream(h): the hits are valid once that stream has been synchronised.
+ * Several GPUs: a handle answers for its own share of the table only, so a key is FOUND on exactly one rank (the
+ * one that owns it) and the others report it as absent; lookups are not routed between ranks.
+ *
+ * A hit reports count, l_links and rword exactly as sdtgpu_export_nodes would for the node: links after the -d
+ * cutoff of finalize, rword with the linear, deleted and single flags.  A window or key that is not in the table
+ * has status SDTGPU_HIT_WINDOW (plus SDTGPU_HIT_RC if it applies) and zero count, l_links and rword. */
+typedef struct sdtgpu_hit {
+	uint32_t count;		/* as sdtgpu_node */
+	uint32_t l_links;	/* as sdtgpu_node */
+	uint32_t rword;		/* as sdtgpu_node: r_links | linear | deleted | single */
+	uint32_t status;	/* SDTGPU_HIT_* bits; 0 = no such window / malformed key (all fields 0) */
+} sdtgpu_hit;		/* 16 bytes */
+#define SDTGPU_HIT_WINDOW 1u	/* a real window of the read, or a well-formed query key */
+#define SDTGPU_HIT_FOUND  2u	/* its canonical k-mer is in this handle's table */
+#define SDTGPU_HIT_RC     4u	/* the query / the window's forward k-mer is the reverse complement of the canonical key */
+
+/* n keys in the sdtgpu_node layout (4 u64 each, key[0] the most significant word, the k-mer in the low 2K bits;
+ * 16-byte aligned device memory) -> n hits (16-byte aligned device memory).  Each key is canonicalised as the chop
+ * does (KmerSmaller: the smaller of the k-mer and its reverse complement).  A key with any bit set at 2K or above
+ * is malformed: status 0, it matches nothing. */
+int sdtgpu_lookup_kmers_device (sdtgpu_t *h, const uint64_t *d_keys, uint64_t n, sdtgpu_hit *d_out);
+/* Every window of a batch of reads, under the conventions of sdtgpu_push_reads_device: tight-string packing,
+ * stride_bytes a multiple of 4, 16-byte aligned device buffers, lens == NULL means uniform_len, reads truncated
+ * to max_read_len, reads shorter than K+1 have no windows, nmask read only with SDTGPU_F_NKMER.  The windows are
+ * exactly those a push chops; with SDTGPU_F_NKMER a window that holds an N looks up key 0 without
+ * SDTGPU_HIT_RC, as it was inserted.  Window j of read r goes to d_out[r * maxwin + j], maxwin = max_read_len - K + 1
+ * (the ordinal convention of sdtgpu_node); entries for windows a read does not have are all zero. */
+int sdtgpu_lookup_reads_device (sdtgpu_t *h, const uint8_t *d_packed, const uint32_t *d_lens, const uint8_t *d_nmask,
+				uint64_t n_reads, uint32_t uniform_len, uint32_t stride_bytes,
+				sdtgpu_hit *d_out /* n_reads x (max_read_len - K + 1) */);
+
 /* pinned host memory for the caller's batch buffers (the reference's seqBuffer/lenBuffer role,
  * prlHashReads.c:387-395); plain pageable memory also works with push_reads, only slower */
 int sdtgpu_host_alloc (void **out, size_t bytes);
@@ -186,7 +224,7 @@ int sdtgpu_kernel_times (sdtgpu_t *h, int reset, double ms[3], uint64_t launches
 
 /* per kernel class since the last reset: [0] insert (single-pass, staged or records), [1] count
  * (staged path) or super-k-mer emit (sliced build), [2] scatter, [3] record dedupe (sliced build),
- * [4] slice build, [5] scans, [6] slice build, retried work items */
+ * [4] slice build, [5] scans, [6] slice build, retried work items, [7] lookups (index build and lookup kernels) */
 int sdtgpu_phase_times (sdtgpu_t *h, int reset, double ms[8], uint64_t launches[8]);
 /* SDTGPU_F_SLICED only: out = { slices, slots per slice image, minimizer length m, m-mers per window,
  * bytes per super-k-mer record, records held, nodes in the store, work items retried by the last build,

@@ -9,12 +9,15 @@
 //            the queue is drained with every lane issuing an upsert;
 //         0  upsert straight from the chop loop (kept for A/B, SDTGPU_NO_QUEUE=1);
 //         1  send side of the record exchange: records into per-owner bins;
-//         4  per reference set, the largest instance ordinal of the batch (hand-back helper).
+//         4  per reference set, the largest instance ordinal of the batch (hand-back helper);
+//         6  lookup: each window's canonical key in the finalized table's index (sdt_lookup.cuh), one
+//            sdtgpu_hit per window at read * maxwin + window.
 //   insert_records_kernel  receive side of the record exchange.
 //   init / rehash / finalize / export / checksum kernels: table maintenance, the post-pass
 //       (thread_delow prlHashReads.c:844-887, thread_mark :911-967) and verification.
 #pragma once
 #include "sdt_device.cuh"
+#include "sdt_lookup.cuh"
 
 namespace sdt {
 
@@ -85,10 +88,11 @@ __host__ __device__ inline u32 hash_kmer_impl (const uint64_t *key, int key_word
 	return (u32) crc & 0x00ffffffu;
 }
 
-// one window -> canonical key and the link bases in the stored orientation (SURVEY.md §8a-2)
+// one window -> canonical key and the link bases in the stored orientation (SURVEY.md §8a-2);
+// *flipped (if given): the canonical key is the reverse complement of the window's forward k-mer
 template <int W, bool NMODE>
 __device__ __forceinline__ void chop_window (const u32 *rd, const u32 *mk, int len, int j, int K,
-					     Key<W> &key, u32 &left, u32 &right)
+					     Key<W> &key, u32 &left, u32 &right, bool *flipped = nullptr)
 {
 	Key<W> f, rc;
 	extract_fwd<W> (rd, j + K, K, f);
@@ -121,10 +125,15 @@ __device__ __forceinline__ void chop_window (const u32 *rd, const u32 *mk, int l
 			for (int i = 0; i < W; i++)
 				key.w[i] = 0;
 			left = right = 4;
+			if (flipped)
+				*flipped = false;
 			return;
 		}
 	}
-	if (key_less<W> (f, rc))
+	const bool fwd = key_less<W> (f, rc);
+	if (flipped)
+		*flipped = !fwd;
+	if (fwd)
 	{
 		key = f;
 		left = prev;
@@ -175,7 +184,7 @@ template <int W> __device__ __forceinline__ void load_record (const u64 *rec, Ke
 // lines, warps parked at the barrier are not what limits it.
 template <int W, bool NMODE, int MODE>
 __global__ void __launch_bounds__ (BLOCK)
-insert_reads_kernel (typename SlotOf<W>::type *table, u64 cap, ReadBatch rb, Bins bins, Counters *ctr)
+insert_reads_kernel (typename SlotOf<W>::type *table, u64 cap, ReadBatch rb, Bins bins, Counters *ctr, Lookup lk)
 {
 	extern __shared__ __align__(16) u32 smem[];
 	const int tid = threadIdx.x;
@@ -321,9 +330,12 @@ insert_reads_kernel (typename SlotOf<W>::type *table, u64 cap, ReadBatch rb, Bin
 			}
 			Key<W> key;
 			u32 left, right;
-			chop_window<W, NMODE> (tile + r * sw, NMODE ? (mtile + r * mw) : nullptr, (int) len, (int) j, K, key, left, right);
+			bool flipped;
+			chop_window<W, NMODE> (tile + r * sw, NMODE ? (mtile + r * mw) : nullptr, (int) len, (int) j, K, key, left, right, MODE == 6 ? &flipped : nullptr);
 			const u64 ord = (rb.first_read_ordinal + r0 + r) * rb.maxwin + j;
-			if (MODE == 0)
+			if (MODE == 6)
+				store_hit (lk.out + (r0 + r) * (u64) rb.maxwin + j, index_probe<W> (table, lk, key, flipped ? HIT_RC : 0u));
+			else if (MODE == 0)
 				created += Table<W>::upsert (table, cap, key, left, right, ord);
 			else if (MODE == 5)
 			{	// replicated-reads sharding: every rank chops every read and keeps the k-mers it owns (the

@@ -6,6 +6,7 @@
 #include "sdt_skm.cuh"
 #include "sdt_merge.cuh"
 #include "sdt_build.cuh"
+#include "sdt_lookup.cuh"
 
 #include <algorithm>
 #include <cstdio>
@@ -39,7 +40,7 @@ struct LogSeg
 	u64 upper;	// windows of the batch at most
 };
 
-static constexpr int N_CAT = 8;	// timing classes: 0 insert, 1 count / emit, 2 scatter, 3 dedupe, 4 build, 5 scan, 6 build retries
+static constexpr int N_CAT = 8;	// timing classes: 0 insert, 1 count / emit, 2 scatter, 3 dedupe, 4 build, 5 scan, 6 build retries, 7 lookups
 
 }	// namespace
 
@@ -90,6 +91,8 @@ struct sdtgpu
 	u32 n_grows = 0;
 	bool finalized = false;
 	int deLowKmer = 0;
+	u64 *index = nullptr;	// lookup index over the finalized table (sdt_lookup.cuh): made by the first lookup, freed by reset
+	u64 idx_cap = 0;
 	u32 owner_rank = 0, owner_ranks = 1;	// sdtgpu_set_owner
 	// sliced build (SDTGPU_F_SLICED): reads of the open epoch are kept in a log and turned into super-k-mer
 	// records in the chains of their slices as they arrive; sliced_flush merges copies and builds the slices
@@ -272,7 +275,7 @@ size_t insert_smem_bytes (const ReadBatch &rb, bool nmode, size_t hist_bins)
 	return 4 * (2 * TILE_PAD + rb.tile_reads * sw + rb.tile_reads + 4 + rb.tile_reads * mw + hist_bins);
 }
 
-template <int W, bool NMODE, int MODE> int launch_insert_t (sdtgpu *h, const ReadBatch &rb, const Bins &bins)
+template <int W, bool NMODE, int MODE> int launch_insert_t (sdtgpu *h, const ReadBatch &rb, const Bins &bins, const Lookup &lk)
 {
 	typedef typename SlotOf<W>::type S;
 	auto kern = insert_reads_kernel<W, NMODE, MODE>;
@@ -288,40 +291,35 @@ template <int W, bool NMODE, int MODE> int launch_insert_t (sdtgpu *h, const Rea
 	cudaStream_t ls = h->launch_stream ? h->launch_stream : h->stream;
 	cudaEvent_t e0 = get_event (h), e1 = get_event (h);
 	CK (h, cudaEventRecord (e0, ls));
-	kern<<<grid, BLOCK, smem, ls>>> (static_cast<S *> (h->table), h->cap, rb, bins, h->d_ctr);
+	kern<<<grid, BLOCK, smem, ls>>> (static_cast<S *> (h->table), h->cap, rb, bins, h->d_ctr, lk);
 	CK (h, cudaGetLastError ());
 	CK (h, cudaEventRecord (e1, ls));
-	h->timing.push_back ({ e0, e1, (MODE == 0 || MODE == 5) ? 0 : 2 });
+	h->timing.push_back ({ e0, e1, (MODE == 0 || MODE == 5) ? 0 : (MODE == 6 ? 7 : 2) });
 	h->all_launches++;
 	return SDTGPU_OK;
 }
 
-template <int MODE> int launch_insert (sdtgpu *h, const ReadBatch &rb, const Bins &bins)
+template <int MODE> int launch_insert (sdtgpu *h, const ReadBatch &rb, const Bins &bins, const Lookup &lk = Lookup ())
 {
 	const bool nmode = (h->flags & SDTGPU_F_NKMER) && rb.nmask;
 	switch (h->W)
 	{
-	case 1: return nmode ? launch_insert_t<1, true, MODE> (h, rb, bins) : launch_insert_t<1, false, MODE> (h, rb, bins);
-	case 2: return nmode ? launch_insert_t<2, true, MODE> (h, rb, bins) : launch_insert_t<2, false, MODE> (h, rb, bins);
-	default: return nmode ? launch_insert_t<4, true, MODE> (h, rb, bins) : launch_insert_t<4, false, MODE> (h, rb, bins);
+	case 1: return nmode ? launch_insert_t<1, true, MODE> (h, rb, bins, lk) : launch_insert_t<1, false, MODE> (h, rb, bins, lk);
+	case 2: return nmode ? launch_insert_t<2, true, MODE> (h, rb, bins, lk) : launch_insert_t<2, false, MODE> (h, rb, bins, lk);
+	default: return nmode ? launch_insert_t<4, true, MODE> (h, rb, bins, lk) : launch_insert_t<4, false, MODE> (h, rb, bins, lk);
 	}
 }
 
+// a batch of device reads, validated (pushes and lookups)
 int make_batch (sdtgpu *h, ReadBatch &rb, const uint8_t *d_packed, const u32 *d_lens, const uint8_t *d_nmask,
 		u64 n_reads, u32 uniform_len, u32 stride_bytes, u64 first_read_ordinal)
 {
-	if (h->finalized)
-		return fail (h, SDTGPU_ESTATE, "push after finalize");
 	if (stride_bytes == 0 || (stride_bytes & 3) || (u64) stride_bytes * 4 < (u64) h->max_read_len)
 		return fail (h, SDTGPU_EINVAL, "stride_bytes must be a multiple of 4 and hold max_read_len bases");
 	if (((uintptr_t) d_packed & 15) || ((uintptr_t) d_lens & 3))
 		return fail (h, SDTGPU_EINVAL, "device read buffers must be 16-byte aligned");
 	if (!d_lens && uniform_len == 0 && n_reads)
 		return fail (h, SDTGPU_EINVAL, "lens == NULL needs uniform_len");
-	const u64 ord_limit = ORD40_NONE;	// the slot keeps 40 bits of ordinal
-	if ((first_read_ordinal + n_reads) >= ord_limit / h->maxwin)
-		return fail (h, SDTGPU_ERANGE, "instance ordinal would overflow the slot's ordinal field");
-	h->ord_end = std::max<u64> (h->ord_end, (first_read_ordinal + n_reads) * h->maxwin);
 	rb.packed = d_packed;
 	rb.lens = d_lens;
 	rb.nmask = (h->flags & SDTGPU_F_NKMER) ? d_nmask : nullptr;
@@ -340,6 +338,22 @@ int make_batch (sdtgpu *h, ReadBatch &rb, const uint8_t *d_packed, const u32 *d_
 	rb.queue_windows = h->owner_ranks > 1 ? std::min<u32> (QUEUE_CAP * h->owner_ranks * 3 / 4, 16384) : QUEUE_CAP;
 	rb.owner_rank = h->owner_rank;
 	rb.owner_ranks = h->owner_ranks;
+	return SDTGPU_OK;
+}
+
+// a batch that goes into the table: only before finalize, and its instance ordinals must fit the slot
+int make_push_batch (sdtgpu *h, ReadBatch &rb, const uint8_t *d_packed, const u32 *d_lens, const uint8_t *d_nmask,
+		     u64 n_reads, u32 uniform_len, u32 stride_bytes, u64 first_read_ordinal)
+{
+	if (h->finalized)
+		return fail (h, SDTGPU_ESTATE, "push after finalize");
+	int rc = make_batch (h, rb, d_packed, d_lens, d_nmask, n_reads, uniform_len, stride_bytes, first_read_ordinal);
+	if (rc)
+		return rc;
+	const u64 ord_limit = ORD40_NONE;	// the slot keeps 40 bits of ordinal
+	if ((first_read_ordinal + n_reads) >= ord_limit / h->maxwin)
+		return fail (h, SDTGPU_ERANGE, "instance ordinal would overflow the slot's ordinal field");
+	h->ord_end = std::max<u64> (h->ord_end, (first_read_ordinal + n_reads) * h->maxwin);
 	return SDTGPU_OK;
 }
 
@@ -419,22 +433,8 @@ export_kernel (const typename SlotOf<W>::type *table, u64 cap, int key_words, in
 #pragma unroll
 		for (int q = 0; q < 4; q++)
 			n.key[q] = q < 4 - W ? 0 : k.w[q - (4 - W)];
-		u32 in_num = 0, out_num = 0;
-#pragma unroll
-		for (int b = 0; b < 4; b++)
-		{
-			in_num += ((L >> (6 * b)) & 63) > 0;
-			out_num += ((R >> (6 * b)) & 63) > 0;
-		}
-		u32 rword = R;
-		if (in_num == 1 && out_num == 1)
-			rword |= 0x01000000u;	// linear  (thread_mark, prlHashReads.c:956-960)
-		if (deLowKmer > 0 && L == 0 && R == 0)
-			rword |= 0x02000000u;	// deleted (thread_delow, prlHashReads.c:876-880)
-		if (count == 1)
-			rword |= 0x08000000u;	// single  (newhash.c:39,103,445)
 		n.l_links = L;
-		n.rword = rword;
+		n.rword = node_rword (L, R, count, deLowKmer);
 		n.count = count;
 		n.set = hash_kmer_impl (n.key, key_words, c_crc) % (u32) thrd_num;
 		n.ordinal = ord;
@@ -1386,6 +1386,80 @@ int sliced_push (sdtgpu *h, const ReadBatch &rb, u64 upper)
 
 u64 iter_slots (const sdtgpu *h) { return h->sliced ? h->n_store : h->cap; }
 
+static_assert (sizeof (Hit) == sizeof (sdtgpu_hit) && SDTGPU_HIT_WINDOW == HIT_WINDOW && SDTGPU_HIT_FOUND == HIT_FOUND && SDTGPU_HIT_RC == HIT_RC, "sdtgpu_hit");
+
+void free_index (sdtgpu *h)
+{
+	cudaFree (h->index);
+	h->index = nullptr;
+	h->idx_cap = 0;
+}
+
+// The lookup index of the finalized table (sdt_lookup.cuh), made by the first lookup: one entry per node at load
+// <= 0.5, 16 bytes per node.  It is not made at finalize, so that a table nobody looks up costs nothing more.
+int ensure_index (sdtgpu *h)
+{
+	if (h->index)
+		return SDTGPU_OK;
+	const u64 slots = iter_slots (h);
+	if (slots >= 0xFFFFFFFFull)
+		return fail (h, SDTGPU_ERANGE, "lookup index: the table has 2^32 - 1 slots or more (entries hold 32-bit positions)");
+	int rc = read_counters (h);
+	if (rc)
+		return rc;
+	const u64 cap = std::max<u64> (1024, 2 * h->h_ctr->n_nodes);
+	if (cudaMalloc (&h->index, cap * sizeof (u64)) != cudaSuccess)
+	{
+		cudaGetLastError ();
+		h->index = nullptr;
+		char b[160];
+		snprintf (b, sizeof b, "device allocation of %.2f GB for the lookup index failed", cap * sizeof (u64) / 1e9);
+		return fail (h, SDTGPU_ENOMEM, b);
+	}
+	h->idx_cap = cap;
+	cudaError_t e;
+	{
+		TimedLaunch tl (h, 7);
+		e = cudaMemsetAsync (h->index, 0xFF, cap * sizeof (u64), h->stream);
+		const unsigned grid = (unsigned) std::min<u64> ((slots + BLOCK - 1) / BLOCK, (u64) h->sm_count * 16);
+		if (e == cudaSuccess && grid)
+		{
+			switch (h->W)
+			{
+			case 1: index_build_kernel<1><<<grid, BLOCK, 0, h->stream>>> (static_cast<const Slot1 *> (h->table), slots, h->index, cap); break;
+			case 2: index_build_kernel<2><<<grid, BLOCK, 0, h->stream>>> (static_cast<const Slot2 *> (h->table), slots, h->index, cap); break;
+			default: index_build_kernel<4><<<grid, BLOCK, 0, h->stream>>> (static_cast<const Slot4 *> (h->table), slots, h->index, cap); break;
+			}
+			e = cudaGetLastError ();
+		}
+	}
+	if (e != cudaSuccess)
+		free_index (h);
+	CK (h, e);
+	return SDTGPU_OK;
+}
+
+// what both lookups check first: a finalized table, and a hit buffer that takes 16-byte stores
+int lookup_prologue (sdtgpu *h, const void *d_out)
+{
+	CK (h, cudaSetDevice (h->device));
+	if (!h->finalized)
+		return fail (h, SDTGPU_ESTATE, "lookup before sdtgpu_finalize");
+	if ((uintptr_t) d_out & 15)
+		return fail (h, SDTGPU_EINVAL, "the hit buffer must be 16-byte aligned");
+	return SDTGPU_OK;
+}
+
+Lookup make_lookup (const sdtgpu *h, sdtgpu_hit *d_out)
+{
+	Lookup lk;
+	lk.index = h->index;
+	lk.idx_cap = h->idx_cap;
+	lk.out = reinterpret_cast<Hit *> (d_out);
+	lk.deLowKmer = h->deLowKmer;
+	return lk;
+}
+
 }	// namespace
 
 // =================================================================================================
@@ -1512,6 +1586,7 @@ void sdtgpu_destroy (sdtgpu_t *h)
 	if (h->h_small) cudaFreeHost (h->h_small);
 	if (h->h_failed) cudaFreeHost (h->h_failed);
 	cudaFree (h->table);
+	cudaFree (h->index);
 	cudaFree (h->d_ctr);
 	if (h->h_ctr) cudaFreeHost (h->h_ctr);
 	if (h->h_nodes_snap) cudaFreeHost (h->h_nodes_snap);
@@ -1527,6 +1602,11 @@ int sdtgpu_reset (sdtgpu_t *h)
 		return SDTGPU_EINVAL;
 	CK (h, cudaSetDevice (h->device));
 	Trace tr (h);
+	if (h->index)
+	{
+		CK (h, cudaStreamSynchronize (h->stream));	// (a lookup may still be reading it)
+		free_index (h);
+	}
 	CK (h, cudaMemsetAsync (h->d_ctr, 0, sizeof (Counters), h->stream));
 	tr.mark ("reset: counters");
 	if (h->sliced)
@@ -1597,7 +1677,7 @@ int sdtgpu_push_reads_device (sdtgpu_t *h, const uint8_t *d_packed, const uint32
 		return SDTGPU_EINVAL;
 	CK (h, cudaSetDevice (h->device));
 	ReadBatch rb;
-	int rc = make_batch (h, rb, d_packed, d_lens, d_nmask, n_reads, uniform_len, stride_bytes, first_read_ordinal);
+	int rc = make_push_batch (h, rb, d_packed, d_lens, d_nmask, n_reads, uniform_len, stride_bytes, first_read_ordinal);
 	if (rc || n_reads == 0)
 		return rc;
 	h->n_reads += n_reads;
@@ -1856,7 +1936,7 @@ int sdtgpu_bucket_reads_device (sdtgpu_t *h, const uint8_t *d_packed, const uint
 		return fail (h, SDTGPU_EINVAL, "bad bins");
 	CK (h, cudaSetDevice (h->device));
 	ReadBatch rb;
-	int rc = make_batch (h, rb, d_packed, d_lens, d_nmask, n_reads, uniform_len, stride_bytes, first_read_ordinal);
+	int rc = make_push_batch (h, rb, d_packed, d_lens, d_nmask, n_reads, uniform_len, stride_bytes, first_read_ordinal);
 	if (rc || n_reads == 0)
 		return rc;
 	Bins b;
@@ -2112,6 +2192,59 @@ int sdtgpu_table_checksum (sdtgpu_t *h, uint64_t out[4])
 	cudaFree (d);
 	CK (h, e);
 	return SDTGPU_OK;
+}
+
+int sdtgpu_lookup_kmers_device (sdtgpu_t *h, const uint64_t *d_keys, uint64_t n, sdtgpu_hit *d_out)
+{
+	if (!h)
+		return SDTGPU_EINVAL;
+	if (n && (!d_keys || !d_out))
+		return fail (h, SDTGPU_EINVAL, "sdtgpu_lookup_kmers_device: NULL buffer");
+	int rc = lookup_prologue (h, d_out);
+	if (rc)
+		return rc;
+	if ((uintptr_t) d_keys & 15)
+		return fail (h, SDTGPU_EINVAL, "the key buffer must be 16-byte aligned");
+	if (n == 0)
+		return SDTGPU_OK;
+	if ((rc = ensure_index (h)))
+		return rc;
+	const Lookup lk = make_lookup (h, d_out);
+	const unsigned grid = (unsigned) std::min<u64> ((n + BLOCK - 1) / BLOCK, (u64) h->sm_count * 16);
+	{
+		TimedLaunch tl (h, 7);
+		switch (h->W)
+		{
+		case 1: lookup_kmers_kernel<1><<<grid, BLOCK, 0, h->stream>>> (static_cast<const Slot1 *> (h->table), lk, reinterpret_cast<const u64 *> (d_keys), n, h->K); break;
+		case 2: lookup_kmers_kernel<2><<<grid, BLOCK, 0, h->stream>>> (static_cast<const Slot2 *> (h->table), lk, reinterpret_cast<const u64 *> (d_keys), n, h->K); break;
+		default: lookup_kmers_kernel<4><<<grid, BLOCK, 0, h->stream>>> (static_cast<const Slot4 *> (h->table), lk, reinterpret_cast<const u64 *> (d_keys), n, h->K); break;
+		}
+	}
+	CK (h, cudaGetLastError ());
+	return SDTGPU_OK;
+}
+
+int sdtgpu_lookup_reads_device (sdtgpu_t *h, const uint8_t *d_packed, const uint32_t *d_lens, const uint8_t *d_nmask,
+				uint64_t n_reads, uint32_t uniform_len, uint32_t stride_bytes, sdtgpu_hit *d_out)
+{
+	if (!h)
+		return SDTGPU_EINVAL;
+	if (n_reads && (!d_packed || !d_out))
+		return fail (h, SDTGPU_EINVAL, "sdtgpu_lookup_reads_device: NULL buffer");
+	int rc = lookup_prologue (h, d_out);
+	if (rc)
+		return rc;
+	ReadBatch rb;
+	if ((rc = make_batch (h, rb, d_packed, d_lens, d_nmask, n_reads, uniform_len, stride_bytes, 0)))
+		return rc;
+	if (n_reads == 0)
+		return SDTGPU_OK;
+	if ((rc = ensure_index (h)))
+		return rc;
+	// windows a read does not have are never written by the kernel: zero them first, unless every read has them all
+	if (d_lens || std::min (uniform_len, (u32) h->max_read_len) != (u32) h->max_read_len)
+		CK (h, cudaMemsetAsync (d_out, 0, n_reads * h->maxwin * sizeof (sdtgpu_hit), h->stream));
+	return launch_insert<6> (h, rb, Bins (), make_lookup (h, d_out));
 }
 
 int sdtgpu_host_alloc (void **out, size_t bytes)

@@ -18,6 +18,10 @@ LIB_PATH = os.path.join(PKG_DIR, "libsdtgpu.so")
 NODE_DTYPE = np.dtype([("key", "<u8", (4,)), ("l_links", "<u4"), ("rword", "<u4"), ("count", "<u4"),
                        ("set", "<u4"), ("ordinal", "<u8")])
 assert NODE_DTYPE.itemsize == 56
+# sdtgpu_hit: one lookup result (include/sdtgpu.h); status holds the HIT_* bits
+HIT_DTYPE = np.dtype([("count", "<u4"), ("l_links", "<u4"), ("rword", "<u4"), ("status", "<u4")])
+assert HIT_DTYPE.itemsize == 16
+HIT_WINDOW, HIT_FOUND, HIT_RC = 1, 2, 4
 
 F_NKMER = 1
 F_SLICED = 4
@@ -46,7 +50,7 @@ class KmerSet(C.Structure):
 def build_library(force: bool = False) -> str:
     """Compiles csrc/ + host/ for sm_100a into libsdtgpu.so (in-tree, so it travels to the GPU box)."""
     srcs = [os.path.join(PKG_DIR, p) for p in ("csrc/sdtgpu.cu", "csrc/sdt_synth.cu", "csrc/sdt_device.cuh",
-                                               "csrc/sdt_kernels.cuh", "csrc/sdt_sliced.cuh", "csrc/sdt_skm.cuh", "csrc/sdt_build.cuh", "host/kmerset_builder.cpp", "host/sdt_readpack.c", "../include/sdtpack.h",
+                                               "csrc/sdt_kernels.cuh", "csrc/sdt_sliced.cuh", "csrc/sdt_skm.cuh", "csrc/sdt_build.cuh", "csrc/sdt_lookup.cuh", "host/kmerset_builder.cpp", "host/sdt_readpack.c", "../include/sdtpack.h",
                                                "../include/sdtgpu.h")]
     stale = (not os.path.exists(LIB_PATH)) or any(os.path.getmtime(s) > os.path.getmtime(LIB_PATH) for s in srcs)
     if force or stale:
@@ -107,6 +111,8 @@ def library() -> C.CDLL:
     L.sdtgpu_aux_stream.argtypes = [vp]
     L.sdtgpu_kernel_time.argtypes = [vp, i32, C.POINTER(C.c_double), C.POINTER(u64), C.POINTER(u64)]
     L.sdtgpu_table_checksum.argtypes = [vp, vp]
+    L.sdtgpu_lookup_kmers_device.argtypes = [vp, vp, u64, vp]
+    L.sdtgpu_lookup_reads_device.argtypes = [vp, vp, vp, vp, u64, u32, u32, vp]
     L.sdtgpu_last_ordinals.argtypes = [vp, i32, vp]
     L.sdtgpu_kernel_times.argtypes = [vp, i32, C.POINTER(C.c_double), C.POINTER(u64)]
     L.sdtgpu_phase_times.argtypes = [vp, i32, C.POINTER(C.c_double), C.POINTER(u64)]
@@ -146,6 +152,12 @@ def _ptr(x) -> int | None:
         assert x.flags["C_CONTIGUOUS"]
         return x.ctypes.data
     return x.data_ptr()
+
+
+def hits_numpy(hits) -> np.ndarray:
+    """Hits as returned by PregraphGPU.lookup_* on the device (int32 [..., 4]) -> a HIT_DTYPE array of shape [...]."""
+    a = np.ascontiguousarray(hits.cpu().numpy() if hasattr(hits, "cpu") else hits).view(np.uint32)
+    return a.view(HIT_DTYPE)[..., 0]
 
 
 def node_bytes(key_words: int) -> int:
@@ -321,6 +333,45 @@ class PregraphGPU:
             return read_kmersets(sets, thrd_num, self.key_words)
         finally:
             self.L.sdtgpu_free_kmersets(sets, thrd_num)
+
+    # ---- lookups in the finalized table (include/sdtgpu.h sdtgpu_lookup_*)
+    def _torch_device(self):
+        import torch
+        return torch.device("cuda", self.device)
+
+    def lookup_kmers(self, keys):
+        """keys: uint64 [n, 4] in the sdtgpu_node layout, a numpy array or a CUDA tensor (int64 or uint64).
+        numpy in -> HIT_DTYPE numpy array [n] out; CUDA tensor in -> CUDA int32 tensor [n, 4] (count, l_links, rword,
+        status; hits_numpy() decodes it).  Synchronises the handle's stream."""
+        import torch
+        dev = self._torch_device()
+        host = isinstance(keys, np.ndarray)
+        if host:
+            keys = torch.from_numpy(np.ascontiguousarray(keys, dtype=np.uint64).view(np.int64)).to(dev)
+        keys = keys.contiguous()
+        assert keys.ndim == 2 and keys.shape[1] == 4 and keys.element_size() == 8, "keys must be [n, 4] 64-bit words"
+        n = keys.shape[0]
+        out = torch.empty((n, 4), dtype=torch.int32, device=dev)
+        torch.cuda.current_stream(dev).synchronize()          # the keys are written on torch's stream, read on the handle's
+        self._ck(self.L.sdtgpu_lookup_kmers_device(self.h, _ptr(keys), n, _ptr(out)))
+        self.sync()
+        return hits_numpy(out) if host else out
+
+    def lookup_reads(self, packed, lens=None, nmask=None, n_reads=None, uniform_len=0, stride_bytes=None):
+        """Every window of a batch of reads in CUDA tensors (the conventions of push_reads(..., device=True)) ->
+        CUDA int32 tensor [n_reads, max_read_len - K + 1, 4] of hits: window j of read r at [r, j]; windows a read
+        does not have are all zero.  Synchronises the handle's stream."""
+        import torch
+        if n_reads is None:
+            n_reads = packed.shape[0]
+        if stride_bytes is None:
+            stride_bytes = packed.shape[1]
+        out = torch.empty((n_reads, self.max_read_len - self.K + 1, 4), dtype=torch.int32, device=self._torch_device())
+        torch.cuda.current_stream(self._torch_device()).synchronize()
+        self._ck(self.L.sdtgpu_lookup_reads_device(self.h, _ptr(packed), _ptr(lens), _ptr(nmask), n_reads, uniform_len,
+                                                   stride_bytes, _ptr(out)))
+        self.sync()
+        return out
 
     def kernel_time(self, reset: bool = True):
         ms, nl, al = C.c_double(), C.c_uint64(), C.c_uint64()
