@@ -177,8 +177,9 @@ void sdtgpu_free_kmersets (sdtgpu_kmerset **sets, int thrd_num);
  * node; SDTGPU_ENOMEM if it does not fit, SDTGPU_ERANGE for a table of 2^32 - 1 slots or more), which is kept until
  * sdtgpu_reset or sdtgpu_destroy; a lookup after reset, push and finalize sees the new table.
  * Both calls only enqueue work on sdtgpu_stream(h): the hits are valid once that stream has been synchronised.
- * Several GPUs: a handle answers for its own share of the table only, so a key is FOUND on exactly one rank (the
- * one that owns it) and the others report it as absent; lookups are not routed between ranks.
+ * Several GPUs: these two calls answer for the handle's own share of the table only, so a key is FOUND on exactly
+ * one rank (the one that owns it) and the others report it as absent.  The routed lookups below send every query to
+ * its owner and answer like one table.
  *
  * A hit reports count, l_links and rword exactly as sdtgpu_export_nodes would for the node: links after the -d
  * cutoff of finalize, rword with the linear, deleted and single flags.  A window or key that is not in the table
@@ -207,6 +208,62 @@ int sdtgpu_lookup_kmers_device (sdtgpu_t *h, const uint64_t *d_keys, uint64_t n,
 int sdtgpu_lookup_reads_device (sdtgpu_t *h, const uint8_t *d_packed, const uint32_t *d_lens, const uint8_t *d_nmask,
 				uint64_t n_reads, uint32_t uniform_len, uint32_t stride_bytes,
 				sdtgpu_hit *d_out /* n_reads x (max_read_len - K + 1) */);
+
+/* ---- routed lookups: several GPUs, each rank with a disjoint share of the table, answer like ONE table.  Each rank
+ * passes its own queries; every query travels to the rank that owns its canonical key, is answered there, and the
+ * hit comes back into the caller's output in the layout of the two calls above.  The hits are bit-identical to
+ * sdtgpu_lookup_kmers_device / sdtgpu_lookup_reads_device on one handle built from all ranks' reads with the same -d
+ * (every field of a hit depends only on its own node, and the union of the shares is that table).
+ *
+ * The owner of a canonical key k is the rank whose share holds it, under the sharding the handle was built with:
+ *   sliced build, sdtgpu_skm_set_world (rank, world), world > 1     slice_of_min (minval (k)) / n_local  (the slices
+ *        (SDTGPU_ROUTE_SKM)                                         are dealt to the ranks in contiguous ranges)
+ *   sliced build, sdtgpu_set_owner (rank, n), n > 1                 slice_of_min (minval (k)) % n
+ *        (SDTGPU_ROUTE_SLICED)
+ *   single-pass insert, sdtgpu_set_owner (rank, n), n > 1            owner_of (key_hash (k), n), the owner function of
+ *        (SDTGPU_ROUTE_HASHED)                                      the replicated-reads sharding and of the record
+ *                                                                   exchange (sdtgpu_bucket_reads_device)
+ *   neither (SDTGPU_ROUTE_ONE)                                      0: the world is 1
+ * minval (k) is the minimizer value the sliced build gives a window: the smallest hashed canonical m-mer among the
+ * central m-mers of the k-mer (sdtgpu_lookup_route: m, lo, w), computed from the key alone.  A handle filled by the
+ * record exchange must declare its share with sdtgpu_set_owner (rank, world) before it finalizes: bucket_reads_device
+ * takes the number of ranks per call, and the handle does not otherwise know it.
+ *
+ * Three halves, so that any transport can move the buffers (sdtgpu_lookup_*_exchange below drives them over NCCL):
+ *   stage     sdtgpu_lookup_stage_kmers / _reads take the arguments and conventions of the two calls above, without
+ *             the output.  Each well-formed key or window is canonicalised and goes, as device_key_words u64 words
+ *             (most significant first), into the region of its owner: owner r's queries are counts[r] queries from
+ *             query starts[r] of *d_queries on, with no gaps (starts, counts: [world]).  Malformed keys and windows a
+ *             read does not have stay home.  The handle keeps each staged query's output position and RC bit.
+ *   answer    the owner: sdtgpu_lookup_answer_buffer (h, n, &q, &r) gives room for n received queries (q) and their
+ *             hits (r); the caller puts the queries there in any order; sdtgpu_lookup_answer (h, n) writes hit i for
+ *             query i.
+ *   unstage   sdtgpu_lookup_unstage_buffer (h, &back) gives room for the hits of this rank's staged queries, which
+ *             the caller puts there in staged order (same starts and counts); sdtgpu_lookup_unstage (h, d_out) writes
+ *             them to d_out (n hits for keys, n_reads x maxwin for reads, 16-byte aligned), RC put back, and what
+ *             did not travel as the single-GPU call writes it (all zero).
+ * All of it only after sdtgpu_finalize (SDTGPU_ESTATE before it and after sdtgpu_reset), at most 64 ranks.  A stage
+ * builds the lookup index of this rank's share if it is missing.  Unstage needs a stage (else SDTGPU_ESTATE); a new
+ * stage replaces the last one.  n = 0 is legal everywhere.  NULL buffers are SDTGPU_EINVAL before any CUDA call.
+ * The buffers belong to the handle, grow only and are kept across calls (each call may move them: take the
+ * addresses again); sdtgpu_reset and sdtgpu_destroy free them.  The kernels run on sdtgpu_stream(h) and are timed in
+ * class 7 of sdtgpu_phase_times; a stage synchronises that stream once (the counts), the other calls only enqueue. */
+#define SDTGPU_ROUTE_ONE    0
+#define SDTGPU_ROUTE_SKM    1
+#define SDTGPU_ROUTE_SLICED 2
+#define SDTGPU_ROUTE_HASHED 3
+/* out = { SDTGPU_ROUTE_*, rank, world, K, device_key_words, n_slices, n_local, m, lo, w, deLowKmer of finalize,
+ * finalized }; the slice fields are 0 where the sharding does not use them */
+int sdtgpu_lookup_route (const sdtgpu_t *h, uint64_t out[12]);
+int sdtgpu_lookup_stage_kmers (sdtgpu_t *h, const uint64_t *d_keys, uint64_t n,
+			       void **d_queries, uint64_t *starts /* world */, uint64_t *counts /* world */);
+int sdtgpu_lookup_stage_reads (sdtgpu_t *h, const uint8_t *d_packed, const uint32_t *d_lens, const uint8_t *d_nmask,
+			       uint64_t n_reads, uint32_t uniform_len, uint32_t stride_bytes,
+			       void **d_queries, uint64_t *starts /* world */, uint64_t *counts /* world */);
+int sdtgpu_lookup_answer_buffer (sdtgpu_t *h, uint64_t n, void **d_queries, sdtgpu_hit **d_replies);
+int sdtgpu_lookup_answer (sdtgpu_t *h, uint64_t n);
+int sdtgpu_lookup_unstage_buffer (sdtgpu_t *h, sdtgpu_hit **d_back);
+int sdtgpu_lookup_unstage (sdtgpu_t *h, sdtgpu_hit *d_out);
 
 /* pinned host memory for the caller's batch buffers (the reference's seqBuffer/lenBuffer role,
  * prlHashReads.c:387-395); plain pageable memory also works with push_reads, only slower */
@@ -277,6 +334,22 @@ int sdtgpu_comm_create (sdtgpu_comm_t **out, int device, const uint8_t id[SDTGPU
 int sdtgpu_comm_destroy (sdtgpu_comm_t *c);
 const char *sdtgpu_comm_last_error (const sdtgpu_comm_t *c);	/* c may be NULL: last failure without a communicator */
 int sdtgpu_skm_exchange (sdtgpu_t *h, sdtgpu_comm_t *c, uint64_t reads_end_this_rank, uint64_t *n_received, double *collective_ms);
+/* Routed lookups in ONE collective call each (every rank of the communicator makes it, after finalize; a rank with
+ * nothing to ask passes n = 0).  The comm's rank and world must equal the handle's sharding (sdtgpu_lookup_route),
+ * else SDTGPU_EINVAL before any collective.  Then the ranks all-gather their sharding descriptors (case, world, K,
+ * device key words, n_slices, n_local, m, lo, w, -d of finalize, finalized) and all return SDTGPU_EINVAL if they
+ * differ; stage, all-gather of the counts (and of every rank's stage status: if one failed, all return), one grouped
+ * ncclSend / ncclRecv of the queries into the owners' answer buffers (the own share is a device-local copy), answer,
+ * one grouped send / recv of the hits back, unstage into d_out.  Same inputs and outputs as
+ * sdtgpu_lookup_kmers_device / sdtgpu_lookup_reads_device; returns when the hits are in d_out.
+ * collective_ms (may be NULL): device time of the collectives that move the lookup's data, i.e. the counts
+ * all-gather and the two grouped send / recv (CUDA events); stage, answer and unstage are in class 7 of
+ * sdtgpu_phase_times. */
+int sdtgpu_lookup_kmers_exchange (sdtgpu_t *h, sdtgpu_comm_t *c, const uint64_t *d_keys, uint64_t n, sdtgpu_hit *d_out,
+				  double *collective_ms);
+int sdtgpu_lookup_reads_exchange (sdtgpu_t *h, sdtgpu_comm_t *c, const uint8_t *d_packed, const uint32_t *d_lens,
+				  const uint8_t *d_nmask, uint64_t n_reads, uint32_t uniform_len, uint32_t stride_bytes,
+				  sdtgpu_hit *d_out, double *collective_ms);
 
 /* ---- synthetic reads on the device (bench/test utility; bit-identical to synth.py).
  * d_tr_bases: uint8 codes of all transcripts; d_starts u64[T]; d_lengths u32[T]; d_cum u64[T]. */

@@ -1,7 +1,9 @@
 // sdt_nccl.cu — the super-k-mer exchange of the sliced build behind the C ABI: one call per epoch does what a
 // host would otherwise script around sdtgpu_skm_stage / sdtgpu_skm_import (include/sdtgpu.h): the ordinal
 // bound (an all-reduce), the merge and pack by owner, the counts (an all-gather), the records (ONE grouped
-// ncclSend / ncclRecv straight into the import buffer) and the build of this rank's slices.
+// ncclSend / ncclRecv straight into the import buffer) and the build of this rank's slices.  The routed lookups
+// (sdtgpu_lookup_kmers_exchange, sdtgpu_lookup_reads_exchange) drive sdtgpu_lookup_stage / _answer / _unstage the
+// same way: the queries travel to their owners and the hits come back, one grouped send / recv each way.
 //
 // Host code only, layered on the public C ABI of the handle.  NCCL is bound at run time (dlopen of
 // libnccl.so.2: in a process that already holds an NCCL — torch's — that one is used; a plain C host gets the
@@ -79,11 +81,14 @@ struct sdtgpu_comm
 	ncclComm_t comm = nullptr;
 	int device = 0, rank = 0, world = 1;
 	unsigned long long *d_buf = nullptr, *h_pin = nullptr;	// [0] mine, [1] reduced, [8 ..) my counts, [8 + world ..) everybody's
-	cudaEvent_t e0 = nullptr, e1 = nullptr;
+	unsigned long long *d_lk = nullptr, *h_lk = nullptr;	// routed lookups: [0, LK_WORDS) mine, then LK_WORDS per rank
+	cudaEvent_t e0 = nullptr, e1 = nullptr, e2 = nullptr, e3 = nullptr;
 	std::string err;
 };
 
 namespace {
+
+constexpr size_t LK_WORDS = 80;	// a routed lookup's messages: the 12-word descriptor, or world counts + a status
 
 int comm_fail (sdtgpu_comm *c, int code, const std::string &what)
 {
@@ -139,8 +144,11 @@ int sdtgpu_comm_create (sdtgpu_comm_t **out, int device, const uint8_t id[SDTGPU
 		return bail (comm_fail (c, SDTGPU_ECUDA, std::string ("ncclCommInitRank: ") + g_nccl.GetErrorString (r)));
 	}
 	const size_t words = 8 + (size_t) world + (size_t) world * world;
+	const size_t lk_words = LK_WORDS * (1 + (size_t) world);
 	if (cudaMalloc (&c->d_buf, words * 8) != cudaSuccess || cudaMallocHost (&c->h_pin, words * 8) != cudaSuccess
-	    || cudaEventCreate (&c->e0) != cudaSuccess || cudaEventCreate (&c->e1) != cudaSuccess)
+	    || cudaMalloc (&c->d_lk, lk_words * 8) != cudaSuccess || cudaMallocHost (&c->h_lk, lk_words * 8) != cudaSuccess
+	    || cudaEventCreate (&c->e0) != cudaSuccess || cudaEventCreate (&c->e1) != cudaSuccess
+	    || cudaEventCreate (&c->e2) != cudaSuccess || cudaEventCreate (&c->e3) != cudaSuccess)
 		return bail (comm_fail (c, SDTGPU_ENOMEM, "sdtgpu_comm_create: allocation failed"));
 	*out = c;
 	return SDTGPU_OK;
@@ -157,10 +165,13 @@ int sdtgpu_comm_destroy (sdtgpu_comm_t *c)
 		cudaFree (c->d_buf);
 	if (c->h_pin)
 		cudaFreeHost (c->h_pin);
-	if (c->e0)
-		cudaEventDestroy (c->e0);
-	if (c->e1)
-		cudaEventDestroy (c->e1);
+	if (c->d_lk)
+		cudaFree (c->d_lk);
+	if (c->h_lk)
+		cudaFreeHost (c->h_lk);
+	for (cudaEvent_t e : { c->e0, c->e1, c->e2, c->e3 })
+		if (e)
+			cudaEventDestroy (e);
 	delete c;
 	return SDTGPU_OK;
 }
@@ -240,6 +251,168 @@ int sdtgpu_skm_exchange (sdtgpu_t *h, sdtgpu_comm_t *c, uint64_t reads_end_this_
 		*collective_ms = ms;
 	}
 	return SDTGPU_OK;
+}
+
+}	// extern "C"
+
+namespace {
+
+// one all-gather of n words per rank (n <= LK_WORDS): this rank's in h_lk[0, n), everybody's to h_lk + LK_WORDS
+// (rank r's at r * n); synchronises the stream
+int lk_allgather (sdtgpu_comm *c, cudaStream_t s, size_t n)
+{
+	CU (c, cudaMemcpyAsync (c->d_lk, c->h_lk, n * 8, cudaMemcpyHostToDevice, s));
+	NC (c, g_nccl.AllGather (c->d_lk, c->d_lk + LK_WORDS, n, ncclUint64, c->comm, s));
+	CU (c, cudaMemcpyAsync (c->h_lk + LK_WORDS, c->d_lk + LK_WORDS, (size_t) c->world * n * 8, cudaMemcpyDeviceToHost, s));
+	CU (c, cudaStreamSynchronize (s));
+	return SDTGPU_OK;
+}
+
+// a routed lookup over NCCL, built from the public halves (include/sdtgpu.h): stage (void **, starts, counts) is
+// sdtgpu_lookup_stage_kmers or _reads with the caller's queries bound
+template <class Stage>
+int lookup_exchange (sdtgpu_t *h, sdtgpu_comm *c, Stage stage, sdtgpu_hit *d_out, double *collective_ms)
+{
+	const int world = c->world, rank = c->rank;
+	int rc;
+	// 1. this rank's handle must be sharded as the communicator is (no collective yet)
+	uint64_t desc[12];
+	if ((rc = sdtgpu_lookup_route (h, desc)))
+		return comm_fail (c, rc, "sdtgpu_lookup_route failed");
+	if (desc[1] != (uint64_t) rank || desc[2] != (uint64_t) world)
+	{
+		char b[200];
+		snprintf (b, sizeof b, "routed lookup: the handle is rank %llu of %llu, the communicator rank %d of %d",
+			  (unsigned long long) desc[1], (unsigned long long) desc[2], rank, world);
+		return comm_fail (c, SDTGPU_EINVAL, b);
+	}
+	cudaStream_t s = static_cast<cudaStream_t> (sdtgpu_stream (h));
+	CU (c, cudaSetDevice (c->device));
+	// 2. every rank's sharding: all equal but the rank, or nobody goes on
+	const size_t nd = 12;
+	for (size_t i = 0; i < nd; i++)
+		c->h_lk[i] = desc[i];
+	if ((rc = lk_allgather (c, s, nd)))
+		return rc;
+	for (int r = 0; r < world; r++)
+		for (size_t i = 0; i < nd; i++)
+			if (i != 1 && c->h_lk[LK_WORDS + r * nd + i] != desc[i])
+			{
+				char b[200];
+				snprintf (b, sizeof b, "routed lookup: rank %d's sharding differs from rank %d's in word %zu of sdtgpu_lookup_route (%llu vs %llu)",
+					  r, rank, i, c->h_lk[LK_WORDS + r * nd + i], (unsigned long long) desc[i]);
+				return comm_fail (c, SDTGPU_EINVAL, b);
+			}
+	if (!desc[11])
+		return comm_fail (c, SDTGPU_ESTATE, "routed lookup before sdtgpu_finalize");
+	// 3. this rank's queries by owner
+	void *d_q = nullptr;
+	std::vector<uint64_t> starts (world, 0), counts (world, 0), recv (world), roff (world);
+	const int st = stage (&d_q, starts.data (), counts.data ());
+	const std::string why = st ? sdtgpu_last_error (h) : "";
+	// 4. who sends how much to whom, and whether every stage worked
+	CU (c, cudaEventRecord (c->e0, s));
+	const size_t nc = (size_t) world + 1;
+	for (int r = 0; r < world; r++)
+		c->h_lk[r] = st ? 0 : counts[r];
+	c->h_lk[world] = (unsigned long long) st;
+	if ((rc = lk_allgather (c, s, nc)))
+		return rc;
+	const unsigned long long *all = c->h_lk + LK_WORDS;	// all[src * nc + dst]: queries src sends to dst; all[src * nc + world]: src's stage status
+	if (st)
+		return comm_fail (c, st, "sdtgpu_lookup_stage: " + why);
+	for (int r = 0; r < world; r++)
+		if (all[r * nc + world])
+			return comm_fail (c, SDTGPU_ESTATE, "routed lookup: the stage of rank " + std::to_string (r) + " failed");
+	uint64_t total = 0;
+	for (int src = 0; src < world; src++)
+	{
+		roff[src] = total;
+		total += (recv[src] = all[src * nc + rank]);
+	}
+	// 5. the queries, in place: sender's region -> owner's answer buffer (runs in source-rank order)
+	void *d_aq = nullptr;
+	sdtgpu_hit *d_ar = nullptr;
+	if ((rc = sdtgpu_lookup_answer_buffer (h, total, &d_aq, &d_ar)))
+		return comm_fail (c, rc, std::string ("sdtgpu_lookup_answer_buffer: ") + sdtgpu_last_error (h));
+	const size_t qw = (size_t) desc[4], qb = 8 * qw, hw = sizeof (sdtgpu_hit) / 8;
+	const char *q_out = static_cast<const char *> (d_q);
+	char *q_in = static_cast<char *> (d_aq);
+	NC (c, g_nccl.GroupStart ());
+	for (int src = 0; src < world; src++)
+	{
+		if (!recv[src])
+			continue;
+		if (src == rank)
+			CU (c, cudaMemcpyAsync (q_in + roff[src] * qb, q_out + starts[rank] * qb, recv[src] * qb, cudaMemcpyDeviceToDevice, s));
+		else
+			NC (c, g_nccl.Recv (q_in + roff[src] * qb, recv[src] * qw, ncclUint64, src, c->comm, s));
+	}
+	for (int dst = 0; dst < world; dst++)
+		if (dst != rank && counts[dst])
+			NC (c, g_nccl.Send (q_out + starts[dst] * qb, counts[dst] * qw, ncclUint64, dst, c->comm, s));
+	NC (c, g_nccl.GroupEnd ());
+	CU (c, cudaEventRecord (c->e1, s));
+	// 6. this rank answers what it owns
+	if ((rc = sdtgpu_lookup_answer (h, total)))
+		return comm_fail (c, rc, std::string ("sdtgpu_lookup_answer: ") + sdtgpu_last_error (h));
+	// 7. the hits back to the askers, into their unstage buffers in staged order
+	sdtgpu_hit *d_back = nullptr;
+	if ((rc = sdtgpu_lookup_unstage_buffer (h, &d_back)))
+		return comm_fail (c, rc, std::string ("sdtgpu_lookup_unstage_buffer: ") + sdtgpu_last_error (h));
+	CU (c, cudaEventRecord (c->e2, s));
+	NC (c, g_nccl.GroupStart ());
+	for (int dst = 0; dst < world; dst++)
+	{
+		if (!counts[dst])
+			continue;
+		if (dst == rank)
+			CU (c, cudaMemcpyAsync (d_back + starts[dst], d_ar + roff[rank], counts[dst] * sizeof (sdtgpu_hit), cudaMemcpyDeviceToDevice, s));
+		else
+			NC (c, g_nccl.Recv (d_back + starts[dst], counts[dst] * hw, ncclUint64, dst, c->comm, s));
+	}
+	for (int src = 0; src < world; src++)
+		if (src != rank && recv[src])
+			NC (c, g_nccl.Send (d_ar + roff[src], recv[src] * hw, ncclUint64, src, c->comm, s));
+	NC (c, g_nccl.GroupEnd ());
+	CU (c, cudaEventRecord (c->e3, s));
+	// 8. into the caller's output
+	if ((rc = sdtgpu_lookup_unstage (h, d_out)))
+		return comm_fail (c, rc, std::string ("sdtgpu_lookup_unstage: ") + sdtgpu_last_error (h));
+	CU (c, cudaStreamSynchronize (s));
+	if (collective_ms)
+	{
+		float a = 0, b = 0;
+		CU (c, cudaEventElapsedTime (&a, c->e0, c->e1));
+		CU (c, cudaEventElapsedTime (&b, c->e2, c->e3));
+		*collective_ms = (double) a + b;
+	}
+	return SDTGPU_OK;
+}
+
+}	// namespace
+
+extern "C" {
+
+int sdtgpu_lookup_kmers_exchange (sdtgpu_t *h, sdtgpu_comm_t *c, const uint64_t *d_keys, uint64_t n, sdtgpu_hit *d_out,
+				  double *collective_ms)
+{
+	if (!h || !c || (n && (!d_keys || !d_out)))
+		return comm_fail (nullptr, SDTGPU_EINVAL, "sdtgpu_lookup_kmers_exchange: NULL handle, communicator or buffer");
+	return lookup_exchange (h, c, [&](void **q, uint64_t *starts, uint64_t *counts) {
+		return sdtgpu_lookup_stage_kmers (h, d_keys, n, q, starts, counts);
+	}, d_out, collective_ms);
+}
+
+int sdtgpu_lookup_reads_exchange (sdtgpu_t *h, sdtgpu_comm_t *c, const uint8_t *d_packed, const uint32_t *d_lens,
+				  const uint8_t *d_nmask, uint64_t n_reads, uint32_t uniform_len, uint32_t stride_bytes,
+				  sdtgpu_hit *d_out, double *collective_ms)
+{
+	if (!h || !c || (n_reads && (!d_packed || !d_out)))
+		return comm_fail (nullptr, SDTGPU_EINVAL, "sdtgpu_lookup_reads_exchange: NULL handle, communicator or buffer");
+	return lookup_exchange (h, c, [&](void **q, uint64_t *starts, uint64_t *counts) {
+		return sdtgpu_lookup_stage_reads (h, d_packed, d_lens, d_nmask, n_reads, uniform_len, stride_bytes, q, starts, counts);
+	}, d_out, collective_ms);
 }
 
 }	// extern "C"

@@ -7,6 +7,7 @@
 #include "sdt_merge.cuh"
 #include "sdt_build.cuh"
 #include "sdt_lookup.cuh"
+#include "sdt_route.cuh"
 
 #include <algorithm>
 #include <cstdio>
@@ -93,6 +94,13 @@ struct sdtgpu
 	int deLowKmer = 0;
 	u64 *index = nullptr;	// lookup index over the finalized table (sdt_lookup.cuh): made by the first lookup, freed by reset
 	u64 idx_cap = 0;
+	// routed lookups (sdt_route.cuh): the buffers grow only and are kept across calls; reset and destroy free them
+	u64 *rt_q = nullptr, *rt_tag = nullptr, *rt_aq = nullptr;	// staged queries and their tags, received queries
+	Hit *rt_ar = nullptr, *rt_back = nullptr;	// replies of this rank as owner, replies to this rank's staged queries
+	size_t rt_cap_q = 0, rt_cap_tag = 0, rt_cap_aq = 0, rt_cap_ar = 0, rt_cap_back = 0;	// bytes
+	u64 *rt_cur = nullptr, *rt_hcur = nullptr;	// per-owner counts / cursors of the stage; pinned mirror
+	bool rt_staged = false;	// a stage awaits its unstage
+	u64 rt_n = 0, rt_out = 0;	// queries staged, entries of the caller's output
 	u32 owner_rank = 0, owner_ranks = 1;	// sdtgpu_set_owner
 	// sliced build (SDTGPU_F_SLICED): reads of the open epoch are kept in a log and turned into super-k-mer
 	// records in the chains of their slices as they arrive; sliced_flush merges copies and builds the slices
@@ -1460,6 +1468,129 @@ Lookup make_lookup (const sdtgpu *h, sdtgpu_hit *d_out)
 	return lk;
 }
 
+// ---- routed lookups (sdt_route.cuh): how this handle's keys are sharded, as the insert side does it
+Route make_route (const sdtgpu *h)
+{
+	Route rt = {};
+	rt.kind = ROUTE_ONE;
+	rt.world = 1;
+	rt.K = h->K;
+	if (h->sliced && h->skm_world > 1)
+	{
+		rt.kind = ROUTE_SKM;
+		rt.world = h->skm_world;
+		rt.n_local = h->n_local;
+	}
+	else if (h->owner_ranks > 1)
+	{
+		rt.kind = h->sliced ? ROUTE_SLICED : ROUTE_HASHED;
+		rt.world = h->owner_ranks;
+	}
+	if (rt.kind == ROUTE_SKM || rt.kind == ROUTE_SLICED)
+	{
+		rt.n_slices = h->geom.n_slices;
+		rt.m = h->geom.m;
+		rt.lo = h->geom.lo;
+		rt.w = h->geom.w;
+	}
+	return rt;
+}
+
+void free_route (sdtgpu *h)
+{
+	cudaFree (h->rt_q); cudaFree (h->rt_tag); cudaFree (h->rt_aq); cudaFree (h->rt_ar); cudaFree (h->rt_back);
+	h->rt_q = h->rt_tag = h->rt_aq = nullptr;
+	h->rt_ar = h->rt_back = nullptr;
+	h->rt_cap_q = h->rt_cap_tag = h->rt_cap_aq = h->rt_cap_ar = h->rt_cap_back = 0;
+	h->rt_staged = false;
+}
+
+// a finalized table, at most ROUTE_MAX_WORLD ranks, the small count buffers, and the index: a rank that stages
+// also answers, and building the index here lets a routed lookup fail before any query travels
+int route_prologue (sdtgpu *h)
+{
+	int rc = lookup_prologue (h, nullptr);
+	if (rc)
+		return rc;
+	if (make_route (h).world > ROUTE_MAX_WORLD)
+		return fail (h, SDTGPU_EINVAL, "routed lookups: at most 64 ranks");
+	if (!h->rt_cur)
+	{
+		CK (h, cudaMalloc (&h->rt_cur, ROUTE_MAX_WORLD * sizeof (u64)));
+		CK (h, cudaMallocHost (&h->rt_hcur, ROUTE_MAX_WORLD * sizeof (u64)));
+	}
+	return ensure_index (h);
+}
+
+// The two passes of a stage around the host's scan of `world` counts.  launch (scatter, stage) enqueues one pass
+// on the handle's stream.  n_out: entries of the caller's output (what unstage writes).
+template <class F> int route_stage (sdtgpu *h, u64 n_out, F launch, void **d_queries, uint64_t *starts, uint64_t *counts)
+{
+	int rc;
+	const u32 world = make_route (h).world;
+	h->rt_staged = false;
+	Stage st = { nullptr, nullptr, reinterpret_cast<unsigned long long *> (h->rt_cur) };
+	CK (h, cudaMemsetAsync (h->rt_cur, 0, world * sizeof (u64), h->stream));
+	if ((rc = launch (false, st)))
+		return rc;
+	CK (h, cudaMemcpyAsync (h->rt_hcur, h->rt_cur, world * sizeof (u64), cudaMemcpyDeviceToHost, h->stream));
+	CK (h, cudaStreamSynchronize (h->stream));
+	u64 total = 0;
+	for (u32 r = 0; r < world; r++)
+	{
+		starts[r] = total;
+		counts[r] = h->rt_hcur[r];
+		h->rt_hcur[r] = total;
+		total += counts[r];
+	}
+	const size_t qb = 8 * (size_t) h->W;
+	if ((rc = grow_device (h, (void **) &h->rt_q, &h->rt_cap_q, 0, std::max<u64> (total, 1) * qb, "staged lookups"))
+	    || (rc = grow_device (h, (void **) &h->rt_tag, &h->rt_cap_tag, 0, std::max<u64> (total, 1) * sizeof (u64), "staged lookups")))
+		return rc;
+	if (total)
+	{
+		CK (h, cudaMemcpyAsync (h->rt_cur, h->rt_hcur, world * sizeof (u64), cudaMemcpyHostToDevice, h->stream));
+		st.q = h->rt_q;
+		st.tag = h->rt_tag;
+		if ((rc = launch (true, st)))
+			return rc;
+	}
+	h->rt_staged = true;
+	h->rt_n = total;
+	h->rt_out = n_out;
+	*d_queries = h->rt_q;
+	return SDTGPU_OK;
+}
+
+template <int W, bool SCATTER> void launch_route_kmers_t (sdtgpu *h, const u64 *keys, u64 n, const Route &rt, const Stage &st)
+{
+	const unsigned grid = (unsigned) std::min<u64> ((n + BLOCK - 1) / BLOCK, (u64) h->sm_count * 16);
+	TimedLaunch tl (h, 7);
+	route_kmers_kernel<W, SCATTER><<<grid, BLOCK, 0, h->stream>>> (keys, n, rt, st);
+}
+
+template <int W, bool NMODE, bool SCATTER> int launch_route_reads_t (sdtgpu *h, const ReadBatch &rb, const Route &rt, const Stage &st)
+{
+	auto kern = route_reads_kernel<W, NMODE, SCATTER>;
+	const size_t smem = 4 * tile_words (rb, NMODE);
+	if (smem > 48 * 1024)
+		CK (h, cudaFuncSetAttribute (kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem));
+	int occ = 0;
+	CK (h, cudaOccupancyMaxActiveBlocksPerMultiprocessor (&occ, kern, BLOCK, smem));
+	if (occ < 1)
+		return fail (h, SDTGPU_EINVAL, "read stride too large for one shared-memory tile");
+	const u64 n_tiles = (rb.n_reads + rb.tile_reads - 1) / rb.tile_reads;
+	const unsigned grid = (unsigned) std::min<u64> (n_tiles, (u64) h->sm_count * occ);
+	TimedLaunch tl (h, 7);
+	kern<<<grid, BLOCK, smem, h->stream>>> (rb, rt, st);
+	return SDTGPU_OK;
+}
+
+template <int W, bool NMODE> int launch_route_reads_w (sdtgpu *h, const ReadBatch &rb, const Route &rt, bool scatter, const Stage &st)
+{
+	return scatter ? launch_route_reads_t<W, NMODE, true> (h, rb, rt, st) : launch_route_reads_t<W, NMODE, false> (h, rb, rt, st);
+}
+
 }	// namespace
 
 // =================================================================================================
@@ -1587,6 +1718,9 @@ void sdtgpu_destroy (sdtgpu_t *h)
 	if (h->h_failed) cudaFreeHost (h->h_failed);
 	cudaFree (h->table);
 	cudaFree (h->index);
+	free_route (h);
+	cudaFree (h->rt_cur);
+	if (h->rt_hcur) cudaFreeHost (h->rt_hcur);
 	cudaFree (h->d_ctr);
 	if (h->h_ctr) cudaFreeHost (h->h_ctr);
 	if (h->h_nodes_snap) cudaFreeHost (h->h_nodes_snap);
@@ -1602,11 +1736,13 @@ int sdtgpu_reset (sdtgpu_t *h)
 		return SDTGPU_EINVAL;
 	CK (h, cudaSetDevice (h->device));
 	Trace tr (h);
-	if (h->index)
+	if (h->index || h->rt_q || h->rt_aq || h->rt_back)
 	{
-		CK (h, cudaStreamSynchronize (h->stream));	// (a lookup may still be reading it)
+		CK (h, cudaStreamSynchronize (h->stream));	// (a lookup may still be reading them)
 		free_index (h);
+		free_route (h);
 	}
+	h->rt_staged = false;
 	CK (h, cudaMemsetAsync (h->d_ctr, 0, sizeof (Counters), h->stream));
 	tr.mark ("reset: counters");
 	if (h->sliced)
@@ -2245,6 +2381,168 @@ int sdtgpu_lookup_reads_device (sdtgpu_t *h, const uint8_t *d_packed, const uint
 	if (d_lens || std::min (uniform_len, (u32) h->max_read_len) != (u32) h->max_read_len)
 		CK (h, cudaMemsetAsync (d_out, 0, n_reads * h->maxwin * sizeof (sdtgpu_hit), h->stream));
 	return launch_insert<6> (h, rb, Bins (), make_lookup (h, d_out));
+}
+
+int sdtgpu_lookup_route (const sdtgpu_t *h, uint64_t out[12])
+{
+	if (!h || !out)
+		return SDTGPU_EINVAL;
+	const Route rt = make_route (h);
+	const u32 rank = rt.kind == ROUTE_SKM ? h->skm_rank : (rt.kind == ROUTE_ONE ? 0 : h->owner_rank);
+	const uint64_t v[12] = { rt.kind, rank, rt.world, (u64) h->K, (u64) h->W, rt.n_slices, rt.n_local, rt.m, rt.lo, rt.w,
+				 (u64) h->deLowKmer, h->finalized ? 1u : 0u };
+	memcpy (out, v, sizeof v);
+	return SDTGPU_OK;
+}
+
+int sdtgpu_lookup_stage_kmers (sdtgpu_t *h, const uint64_t *d_keys, uint64_t n, void **d_queries, uint64_t *starts, uint64_t *counts)
+{
+	if (!h)
+		return SDTGPU_EINVAL;
+	if ((n && !d_keys) || !d_queries || !starts || !counts)
+		return fail (h, SDTGPU_EINVAL, "sdtgpu_lookup_stage_kmers: NULL buffer");
+	int rc = route_prologue (h);
+	if (rc)
+		return rc;
+	if ((uintptr_t) d_keys & 15)
+		return fail (h, SDTGPU_EINVAL, "the key buffer must be 16-byte aligned");
+	const Route rt = make_route (h);
+	const u64 *keys = reinterpret_cast<const u64 *> (d_keys);
+	auto launch = [&](bool scatter, const Stage &st) -> int {
+		if (n == 0)
+			return SDTGPU_OK;
+		switch (h->W)
+		{
+		case 1: scatter ? launch_route_kmers_t<1, true> (h, keys, n, rt, st) : launch_route_kmers_t<1, false> (h, keys, n, rt, st); break;
+		case 2: scatter ? launch_route_kmers_t<2, true> (h, keys, n, rt, st) : launch_route_kmers_t<2, false> (h, keys, n, rt, st); break;
+		default: scatter ? launch_route_kmers_t<4, true> (h, keys, n, rt, st) : launch_route_kmers_t<4, false> (h, keys, n, rt, st); break;
+		}
+		CK (h, cudaGetLastError ());
+		return SDTGPU_OK;
+	};
+	return route_stage (h, n, launch, d_queries, starts, counts);
+}
+
+int sdtgpu_lookup_stage_reads (sdtgpu_t *h, const uint8_t *d_packed, const uint32_t *d_lens, const uint8_t *d_nmask,
+			       uint64_t n_reads, uint32_t uniform_len, uint32_t stride_bytes,
+			       void **d_queries, uint64_t *starts, uint64_t *counts)
+{
+	if (!h)
+		return SDTGPU_EINVAL;
+	if ((n_reads && !d_packed) || !d_queries || !starts || !counts)
+		return fail (h, SDTGPU_EINVAL, "sdtgpu_lookup_stage_reads: NULL buffer");
+	int rc = route_prologue (h);
+	if (rc)
+		return rc;
+	ReadBatch rb;
+	if ((rc = make_batch (h, rb, d_packed, d_lens, d_nmask, n_reads, uniform_len, stride_bytes, 0)))
+		return rc;
+	const Route rt = make_route (h);
+	const bool nmode = (h->flags & SDTGPU_F_NKMER) && rb.nmask;
+	auto launch = [&](bool scatter, const Stage &st) -> int {
+		if (n_reads == 0)
+			return SDTGPU_OK;
+		int r;
+		switch (h->W)
+		{
+		case 1: r = nmode ? launch_route_reads_w<1, true> (h, rb, rt, scatter, st) : launch_route_reads_w<1, false> (h, rb, rt, scatter, st); break;
+		case 2: r = nmode ? launch_route_reads_w<2, true> (h, rb, rt, scatter, st) : launch_route_reads_w<2, false> (h, rb, rt, scatter, st); break;
+		default: r = nmode ? launch_route_reads_w<4, true> (h, rb, rt, scatter, st) : launch_route_reads_w<4, false> (h, rb, rt, scatter, st); break;
+		}
+		if (r)
+			return r;
+		CK (h, cudaGetLastError ());
+		return SDTGPU_OK;
+	};
+	return route_stage (h, n_reads * h->maxwin, launch, d_queries, starts, counts);
+}
+
+int sdtgpu_lookup_answer_buffer (sdtgpu_t *h, uint64_t n, void **d_queries, sdtgpu_hit **d_replies)
+{
+	if (!h)
+		return SDTGPU_EINVAL;
+	if (!d_queries || !d_replies)
+		return fail (h, SDTGPU_EINVAL, "sdtgpu_lookup_answer_buffer: NULL buffer");
+	int rc = lookup_prologue (h, nullptr);
+	if (rc)
+		return rc;
+	if ((rc = grow_device (h, (void **) &h->rt_aq, &h->rt_cap_aq, 0, std::max<u64> (n, 1) * 8 * h->W, "received lookups"))
+	    || (rc = grow_device (h, (void **) &h->rt_ar, &h->rt_cap_ar, 0, std::max<u64> (n, 1) * sizeof (Hit), "lookup replies")))
+		return rc;
+	*d_queries = h->rt_aq;
+	*d_replies = reinterpret_cast<sdtgpu_hit *> (h->rt_ar);
+	return SDTGPU_OK;
+}
+
+int sdtgpu_lookup_answer (sdtgpu_t *h, uint64_t n)
+{
+	if (!h)
+		return SDTGPU_EINVAL;
+	int rc = lookup_prologue (h, nullptr);
+	if (rc)
+		return rc;
+	if (n > h->rt_cap_aq / (8 * h->W) || n > h->rt_cap_ar / sizeof (Hit))
+		return fail (h, SDTGPU_EINVAL, "sdtgpu_lookup_answer: more queries than sdtgpu_lookup_answer_buffer made room for");
+	if (n == 0)
+		return SDTGPU_OK;
+	if ((rc = ensure_index (h)))
+		return rc;
+	const Lookup lk = make_lookup (h, reinterpret_cast<sdtgpu_hit *> (h->rt_ar));
+	const unsigned grid = (unsigned) std::min<u64> ((n + BLOCK - 1) / BLOCK, (u64) h->sm_count * 16);
+	{
+		TimedLaunch tl (h, 7);
+		switch (h->W)
+		{
+		case 1: route_answer_kernel<1><<<grid, BLOCK, 0, h->stream>>> (static_cast<const Slot1 *> (h->table), lk, h->rt_aq, n); break;
+		case 2: route_answer_kernel<2><<<grid, BLOCK, 0, h->stream>>> (static_cast<const Slot2 *> (h->table), lk, h->rt_aq, n); break;
+		default: route_answer_kernel<4><<<grid, BLOCK, 0, h->stream>>> (static_cast<const Slot4 *> (h->table), lk, h->rt_aq, n); break;
+		}
+	}
+	CK (h, cudaGetLastError ());
+	return SDTGPU_OK;
+}
+
+int sdtgpu_lookup_unstage_buffer (sdtgpu_t *h, sdtgpu_hit **d_back)
+{
+	if (!h)
+		return SDTGPU_EINVAL;
+	if (!d_back)
+		return fail (h, SDTGPU_EINVAL, "sdtgpu_lookup_unstage_buffer: NULL buffer");
+	int rc = lookup_prologue (h, nullptr);
+	if (rc)
+		return rc;
+	if (!h->rt_staged)
+		return fail (h, SDTGPU_ESTATE, "sdtgpu_lookup_unstage_buffer without a stage");
+	if ((rc = grow_device (h, (void **) &h->rt_back, &h->rt_cap_back, 0, std::max<u64> (h->rt_n, 1) * sizeof (Hit), "lookup replies")))
+		return rc;
+	*d_back = reinterpret_cast<sdtgpu_hit *> (h->rt_back);
+	return SDTGPU_OK;
+}
+
+int sdtgpu_lookup_unstage (sdtgpu_t *h, sdtgpu_hit *d_out)
+{
+	if (!h)
+		return SDTGPU_EINVAL;
+	if (!d_out && (!h->rt_staged || h->rt_out))
+		return fail (h, SDTGPU_EINVAL, "sdtgpu_lookup_unstage: NULL buffer");
+	int rc = lookup_prologue (h, d_out);
+	if (rc)
+		return rc;
+	if (!h->rt_staged)
+		return fail (h, SDTGPU_ESTATE, "sdtgpu_lookup_unstage without a stage");
+	if (h->rt_n > h->rt_cap_back / sizeof (Hit))
+		return fail (h, SDTGPU_ESTATE, "sdtgpu_lookup_unstage: the replies need sdtgpu_lookup_unstage_buffer first");
+	h->rt_staged = false;
+	if (h->rt_n < h->rt_out)	// malformed keys, windows a read does not have: all zero, as the single-GPU lookup writes them
+		CK (h, cudaMemsetAsync (d_out, 0, h->rt_out * sizeof (sdtgpu_hit), h->stream));
+	if (h->rt_n)
+	{
+		const unsigned grid = (unsigned) std::min<u64> ((h->rt_n + BLOCK - 1) / BLOCK, (u64) h->sm_count * 16);
+		TimedLaunch tl (h, 7);
+		route_unstage_kernel<<<grid, BLOCK, 0, h->stream>>> (h->rt_back, h->rt_tag, h->rt_n, reinterpret_cast<Hit *> (d_out));
+	}
+	CK (h, cudaGetLastError ());
+	return SDTGPU_OK;
 }
 
 int sdtgpu_host_alloc (void **out, size_t bytes)

@@ -50,7 +50,7 @@ class KmerSet(C.Structure):
 def build_library(force: bool = False) -> str:
     """Compiles csrc/ + host/ for sm_100a into libsdtgpu.so (in-tree, so it travels to the GPU box)."""
     srcs = [os.path.join(PKG_DIR, p) for p in ("csrc/sdtgpu.cu", "csrc/sdt_synth.cu", "csrc/sdt_device.cuh",
-                                               "csrc/sdt_kernels.cuh", "csrc/sdt_sliced.cuh", "csrc/sdt_skm.cuh", "csrc/sdt_build.cuh", "csrc/sdt_lookup.cuh", "host/kmerset_builder.cpp", "host/sdt_readpack.c", "../include/sdtpack.h",
+                                               "csrc/sdt_kernels.cuh", "csrc/sdt_sliced.cuh", "csrc/sdt_skm.cuh", "csrc/sdt_build.cuh", "csrc/sdt_lookup.cuh", "csrc/sdt_route.cuh", "csrc/sdt_nccl.cu", "host/kmerset_builder.cpp", "host/sdt_readpack.c", "../include/sdtpack.h",
                                                "../include/sdtgpu.h")]
     stale = (not os.path.exists(LIB_PATH)) or any(os.path.getmtime(s) > os.path.getmtime(LIB_PATH) for s in srcs)
     if force or stale:
@@ -113,6 +113,15 @@ def library() -> C.CDLL:
     L.sdtgpu_table_checksum.argtypes = [vp, vp]
     L.sdtgpu_lookup_kmers_device.argtypes = [vp, vp, u64, vp]
     L.sdtgpu_lookup_reads_device.argtypes = [vp, vp, vp, vp, u64, u32, u32, vp]
+    L.sdtgpu_lookup_route.argtypes = [vp, vp]
+    L.sdtgpu_lookup_stage_kmers.argtypes = [vp, vp, u64, C.POINTER(vp), vp, vp]
+    L.sdtgpu_lookup_stage_reads.argtypes = [vp, vp, vp, vp, u64, u32, u32, C.POINTER(vp), vp, vp]
+    L.sdtgpu_lookup_answer_buffer.argtypes = [vp, u64, C.POINTER(vp), C.POINTER(vp)]
+    L.sdtgpu_lookup_answer.argtypes = [vp, u64]
+    L.sdtgpu_lookup_unstage_buffer.argtypes = [vp, C.POINTER(vp)]
+    L.sdtgpu_lookup_unstage.argtypes = [vp, vp]
+    L.sdtgpu_lookup_kmers_exchange.argtypes = [vp, vp, vp, u64, vp, C.POINTER(C.c_double)]
+    L.sdtgpu_lookup_reads_exchange.argtypes = [vp, vp, vp, vp, vp, u64, u32, u32, vp, C.POINTER(C.c_double)]
     L.sdtgpu_last_ordinals.argtypes = [vp, i32, vp]
     L.sdtgpu_kernel_times.argtypes = [vp, i32, C.POINTER(C.c_double), C.POINTER(u64)]
     L.sdtgpu_phase_times.argtypes = [vp, i32, C.POINTER(C.c_double), C.POINTER(u64)]
@@ -371,6 +380,102 @@ class PregraphGPU:
         self._ck(self.L.sdtgpu_lookup_reads_device(self.h, _ptr(packed), _ptr(lens), _ptr(nmask), n_reads, uniform_len,
                                                    stride_bytes, _ptr(out)))
         self.sync()
+        return out
+
+    # ---- lookups routed to the rank that owns each k-mer (include/sdtgpu.h sdtgpu_lookup_stage_* ... _exchange)
+    def lookup_route(self) -> dict:
+        """How this handle's keys are sharded (sdtgpu_lookup_route)."""
+        out = (C.c_uint64 * 12)()
+        self._ck(self.L.sdtgpu_lookup_route(self.h, out))
+        names = ("kind", "rank", "world", "K", "key_words", "n_slices", "n_local", "m", "lo", "w", "deLowKmer", "finalized")
+        return {k: int(v) for k, v in zip(names, out)}
+
+    def _stage(self, fn, *args):
+        world = self.lookup_route()["world"]
+        ptr, starts, counts = C.c_void_p(), (C.c_uint64 * world)(), (C.c_uint64 * world)()
+        self._ck(fn(self.h, *args, C.byref(ptr), starts, counts))
+        self.sync()
+        return int(ptr.value or 0), [int(x) for x in starts], [int(x) for x in counts]
+
+    def lookup_stage_kmers(self, keys):
+        """keys: CUDA tensor [n, 4] of 64-bit words (the layout of lookup_kmers) -> (device address of the staged
+        queries, starts[world], counts[world] in queries of key_words u64 each).  Synchronises the handle's stream."""
+        import torch
+        torch.cuda.current_stream(self._torch_device()).synchronize()
+        return self._stage(self.L.sdtgpu_lookup_stage_kmers, _ptr(keys), keys.shape[0])
+
+    def lookup_stage_reads(self, packed, lens=None, nmask=None, n_reads=None, uniform_len=0, stride_bytes=None):
+        """Every window of a batch of reads (the conventions of lookup_reads) staged by owner; as lookup_stage_kmers."""
+        import torch
+        n_reads = packed.shape[0] if n_reads is None else n_reads
+        stride_bytes = packed.shape[1] if stride_bytes is None else stride_bytes
+        torch.cuda.current_stream(self._torch_device()).synchronize()
+        return self._stage(self.L.sdtgpu_lookup_stage_reads, _ptr(packed), _ptr(lens), _ptr(nmask), n_reads, uniform_len, stride_bytes)
+
+    def lookup_answer_buffer(self, n: int):
+        """-> (device address for n received queries, device address of their n hits)."""
+        q, r = C.c_void_p(), C.c_void_p()
+        self._ck(self.L.sdtgpu_lookup_answer_buffer(self.h, n, C.byref(q), C.byref(r)))
+        return int(q.value or 0), int(r.value or 0)
+
+    def lookup_answer(self, n: int):
+        """Answers the n queries in the answer buffer.  Synchronises the handle's stream."""
+        self._ck(self.L.sdtgpu_lookup_answer(self.h, n))
+        self.sync()
+
+    def lookup_unstage_buffer(self) -> int:
+        """-> device address for the hits of this rank's staged queries, in staged order."""
+        p = C.c_void_p()
+        self._ck(self.L.sdtgpu_lookup_unstage_buffer(self.h, C.byref(p)))
+        return int(p.value or 0)
+
+    def lookup_unstage(self, out):
+        """Writes the hits to out (a CUDA int32 tensor shaped as lookup_kmers' or lookup_reads' output).  Synchronises
+        the handle's stream."""
+        import torch
+        torch.cuda.current_stream(self._torch_device()).synchronize()
+        self._ck(self.L.sdtgpu_lookup_unstage(self.h, _ptr(out)))
+        self.sync()
+        return out
+
+    def _exchange(self, fn, comm: "SkmComm", *args):
+        ms = C.c_double()
+        rc = fn(self.h, comm.c, *args, C.byref(ms))
+        if rc:     # (argument errors are reported without the communicator)
+            raise SdtGpuError(rc, (self.L.sdtgpu_comm_last_error(comm.c) or self.L.sdtgpu_comm_last_error(None) or b"").decode())
+        self.last_collective_ms = float(ms.value)
+
+    def lookup_kmers_exchange(self, comm: "SkmComm", keys):
+        """lookup_kmers over all ranks of comm (every rank calls it with its own keys, possibly none): each key is
+        answered by the rank that owns it.  Same inputs and outputs as lookup_kmers; the device time of the collectives
+        is left in self.last_collective_ms."""
+        import torch
+        dev = self._torch_device()
+        host = isinstance(keys, np.ndarray)
+        if host:
+            keys = torch.from_numpy(np.ascontiguousarray(keys, dtype=np.uint64).view(np.int64)).to(dev)
+        keys = keys.contiguous()
+        assert keys.ndim == 2 and keys.shape[1] == 4 and keys.element_size() == 8, "keys must be [n, 4] 64-bit words"
+        out = torch.empty((keys.shape[0], 4), dtype=torch.int32, device=dev)
+        torch.cuda.current_stream(dev).synchronize()
+        self._exchange(self.L.sdtgpu_lookup_kmers_exchange, comm, _ptr(keys), keys.shape[0], _ptr(out))
+        return hits_numpy(out) if host else out
+
+    def lookup_reads_exchange(self, comm: "SkmComm", packed, lens=None, nmask=None, n_reads=None, uniform_len=0,
+                              stride_bytes=None, out=None):
+        """lookup_reads over all ranks of comm, every window answered by the rank that owns it.  Same inputs and outputs
+        as lookup_reads; out (optional): a CUDA int32 tensor [>= n_reads, max_read_len - K + 1, 4] to reuse."""
+        import torch
+        dev = self._torch_device()
+        n_reads = packed.shape[0] if n_reads is None else n_reads
+        stride_bytes = packed.shape[1] if stride_bytes is None else stride_bytes
+        if out is None:
+            out = torch.empty((n_reads, self.max_read_len - self.K + 1, 4), dtype=torch.int32, device=dev)
+        else:
+            out = out[:n_reads]
+        torch.cuda.current_stream(dev).synchronize()
+        self._exchange(self.L.sdtgpu_lookup_reads_exchange, comm, _ptr(packed), _ptr(lens), _ptr(nmask), n_reads,
+                       uniform_len, stride_bytes, _ptr(out))
         return out
 
     def kernel_time(self, reset: bool = True):
