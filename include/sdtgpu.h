@@ -358,6 +358,30 @@ int sdtgpu_synth_reads_device (int device, void *stream, const uint8_t *d_tr_bas
 			       uint64_t seed, uint64_t first_pair, uint64_t n_pairs, uint32_t read_len,
 			       uint32_t stride_bytes, uint8_t *d_packed_out);
 
+/* ---- FASTA/FASTQ files parsed and packed on the GPU (csrc/sdt_parse.cu).  The records, their order and every output
+ * byte equal what sdtpack_next (include/sdtpack.h) produces for the same files and options; the batches are in the
+ * layout sdtgpu_push_reads_device and sdtgpu_lookup_reads_device take.  The text goes to the device in chunks (pinned
+ * staging, parallel pread, cudaMemcpyAsync); every chunk starts at a record boundary, a record longer than a chunk
+ * makes the chunk grow, junk lines never do.  Device buffers grow only and are freed by close.
+ * path2 == NULL: single-ended.  fastq: 0 FASTA, 1 FASTQ.  chunk_bytes: size of one text upload (0 = 64 MiB;
+ * small values are for tests).  SDTGPU_EINVAL if a file cannot be opened (sdtgpu_reader_last_error names it).
+ * open touches no CUDA state; the first sdtgpu_reader_next sets the reader up on `device`. */
+typedef struct sdtgpu_reader sdtgpu_reader_t;
+int sdtgpu_reader_open (sdtgpu_reader_t **out, int device, const char *path1, const char *path2, int fastq,
+			uint64_t chunk_bytes);
+/* The next min (M, remaining) records of the stream, M = max_reads (pairs: max_reads rounded down to even),
+ * written to d_packed / d_lens / d_nmask (16-byte aligned device buffers, nmask only with n_kmer) with the
+ * conventions and argument checks of sdtpack_next.  *n_out = 0 at end of input.  The pack kernels are enqueued
+ * on `stream` (NULL: the legacy default stream); the call returns once *n_out is known, and the outputs are
+ * valid once that stream has reached them.  stride_bytes is at most 6144 (4096 with n_kmer). */
+int sdtgpu_reader_next (sdtgpu_reader_t *r, void *stream, int max_read_len, int n_kmer, int reverse,
+			uint8_t *d_packed, uint32_t *d_lens, uint8_t *d_nmask, uint64_t max_reads,
+			uint32_t stride_bytes, uint64_t *n_out);
+/* out = { text bytes copied host to device, records returned, chunks uploaded, device buffer (re)allocations } */
+int sdtgpu_reader_stats (const sdtgpu_reader_t *r, uint64_t out[4]);
+const char *sdtgpu_reader_last_error (const sdtgpu_reader_t *r);	/* r may be NULL: last open() failure */
+void sdtgpu_reader_close (sdtgpu_reader_t *r);
+
 /* reference helpers restated for host callers (tests bind them) */
 uint64_t sdtgpu_hash_kmer (const uint64_t key[4], int key_words);	/* hashFunction.c:108 */
 int sdtgpu_version (void);

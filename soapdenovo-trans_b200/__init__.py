@@ -11,6 +11,6 @@ The directory name contains a hyphen, so import it through `load()` in the repo-
 """
 from . import synth  # noqa: F401
 from .pregraph import (  # noqa: F401
-    HIT_DTYPE, HIT_FOUND, HIT_RC, HIT_WINDOW, LIB_PATH, NODE_DTYPE, PregraphGPU, ReadPacker, SdtGpuError, build_library,
+    DeviceReadPacker, HIT_DTYPE, HIT_FOUND, HIT_RC, HIT_WINDOW, LIB_PATH, NODE_DTYPE, PregraphGPU, ReadPacker, SdtGpuError, build_library,
     hash_kmer, hits_numpy, library, nodes_to_records, read_kmersets,
 )

@@ -50,7 +50,7 @@ class KmerSet(C.Structure):
 def build_library(force: bool = False) -> str:
     """Compiles csrc/ + host/ for sm_100a into libsdtgpu.so (in-tree, so it travels to the GPU box)."""
     srcs = [os.path.join(PKG_DIR, p) for p in ("csrc/sdtgpu.cu", "csrc/sdt_synth.cu", "csrc/sdt_device.cuh",
-                                               "csrc/sdt_kernels.cuh", "csrc/sdt_sliced.cuh", "csrc/sdt_skm.cuh", "csrc/sdt_build.cuh", "csrc/sdt_lookup.cuh", "csrc/sdt_route.cuh", "csrc/sdt_nccl.cu", "host/kmerset_builder.cpp", "host/sdt_readpack.c", "../include/sdtpack.h",
+                                               "csrc/sdt_kernels.cuh", "csrc/sdt_sliced.cuh", "csrc/sdt_skm.cuh", "csrc/sdt_build.cuh", "csrc/sdt_lookup.cuh", "csrc/sdt_route.cuh", "csrc/sdt_nccl.cu", "csrc/sdt_parse.cu", "host/kmerset_builder.cpp", "host/sdt_readpack.c", "../include/sdtpack.h",
                                                "../include/sdtgpu.h")]
     stale = (not os.path.exists(LIB_PATH)) or any(os.path.getmtime(s) > os.path.getmtime(LIB_PATH) for s in srcs)
     if force or stale:
@@ -133,6 +133,13 @@ def library() -> C.CDLL:
     L.sdtpack_close.argtypes = [vp]
     L.sdtpack_close.restype = None
     L.sdtgpu_synth_reads_device.argtypes = [i32, vp, vp, vp, vp, vp, u32, u64, u64, u64, u32, u32, vp]
+    L.sdtgpu_reader_open.argtypes = [C.POINTER(vp), i32, C.c_char_p, C.c_char_p, i32, u64]
+    L.sdtgpu_reader_next.argtypes = [vp, vp, i32, i32, i32, vp, vp, vp, u64, u32, C.POINTER(u64)]
+    L.sdtgpu_reader_stats.argtypes = [vp, C.POINTER(u64)]
+    L.sdtgpu_reader_last_error.restype = C.c_char_p
+    L.sdtgpu_reader_last_error.argtypes = [vp]
+    L.sdtgpu_reader_close.argtypes = [vp]
+    L.sdtgpu_reader_close.restype = None
     _lib = L
     return L
 
@@ -570,3 +577,56 @@ class ReadPacker:
             self.h = None
 
     __del__ = close
+
+
+class DeviceReadPacker:
+    """include/sdtgpu.h sdtgpu_reader_*: FASTA/FASTQ parsed and packed on the GPU.  Same records, order and bytes as
+    ReadPacker, delivered as CUDA tensors in the layout of PregraphGPU.push_reads(..., device=True)."""
+
+    def __init__(self, path1: str, path2: str | None = None, fastq: bool = False, device: int = 0, chunk_bytes: int = 0):
+        self.L = library()
+        self.h = C.c_void_p()
+        self.device = device
+        rc = self.L.sdtgpu_reader_open(C.byref(self.h), device, path1.encode(), path2.encode() if path2 else None,
+                                       int(fastq), chunk_bytes)
+        if rc:
+            raise SdtGpuError(rc, self.L.sdtgpu_reader_last_error(None).decode())
+
+    def next(self, max_read_len: int, max_reads: int, n_kmer: bool = False, reverse: bool = False,
+             stride_bytes: int | None = None):
+        """Returns (packed[n, stride], lens[n], nmask[n, stride/2] or None) as CUDA uint8 / int32 (lens: uint32 bits)
+        tensors; n == 0 at end of input.  Written on torch's current stream of the device."""
+        import torch
+        from .synth import stride_bytes as _sb
+        stride = stride_bytes or _sb(max_read_len)
+        dev = torch.device("cuda", self.device)
+        packed = torch.empty((max_reads, stride), dtype=torch.uint8, device=dev)
+        lens = torch.empty(max_reads, dtype=torch.int32, device=dev)
+        nmask = torch.empty((max_reads, stride // 2), dtype=torch.uint8, device=dev) if n_kmer else None
+        n = C.c_uint64()
+        rc = self.L.sdtgpu_reader_next(self.h, torch.cuda.current_stream(dev).cuda_stream, max_read_len, int(n_kmer),
+                                       int(reverse), _ptr(packed), _ptr(lens), _ptr(nmask), max_reads, stride, C.byref(n))
+        if rc:
+            raise SdtGpuError(rc, self.L.sdtgpu_reader_last_error(self.h).decode())
+        n = int(n.value)
+        return packed[:n], lens[:n], (nmask[:n] if n_kmer else None)
+
+    def stats(self) -> dict:
+        out = (C.c_uint64 * 4)()
+        rc = self.L.sdtgpu_reader_stats(self.h, out)
+        if rc:
+            raise SdtGpuError(rc, "sdtgpu_reader_stats")
+        return dict(text_bytes=int(out[0]), records=int(out[1]), chunks=int(out[2]), allocations=int(out[3]))
+
+    def close(self):
+        if getattr(self, "h", None):
+            self.L.sdtgpu_reader_close(self.h)
+            self.h = None
+
+    __del__ = close
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *a):
+        self.close()
