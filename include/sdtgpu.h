@@ -382,6 +382,42 @@ int sdtgpu_reader_stats (const sdtgpu_reader_t *r, uint64_t out[4]);
 const char *sdtgpu_reader_last_error (const sdtgpu_reader_t *r);	/* r may be NULL: last open() failure */
 void sdtgpu_reader_close (sdtgpu_reader_t *r);
 
+/* One library read by `world` ranks together, each parsing only its own byte range (DESIGN §9.1 "One library, several
+ * readers").  The stream is the records sdtpack_next returns; a record's ordinal is its place in it (a pair of n1 and n2
+ * records, m = min (n1, n2): record i < m of file 1 is 2i, of file 2 is 2i + 1, record j >= m of the longer file is
+ * m + j).  Rank r's range of a file of S bytes is [r S / world, (r + 1) S / world); a line belongs to the range that
+ * holds its first byte, a record to the range that holds its header line.  Rank r returns the records of its range of
+ * file 1 (single-ended), or (pairs) the pairs i in [min (m, c1_r), min (m, c1_r+1)), c1_r = file-1 records before range
+ * r, then the records j >= m of the longer file in its range of that file.  Put in ordinal order, every rank's batches
+ * are byte for byte the output of sdtpack_next, and every ordinal comes back once.
+ *   open_shard  like open (no CUDA state), plus rank and world; SDTGPU_EINVAL unless 0 <= rank < world <= 1024.
+ *   summary     scans this rank's range of each file on the device (sets the reader up on `device`) into 256 opaque
+ *               bytes: rank, world, fastq, files, sizes, a fingerprint of each file's first and last 4 KiB, and per
+ *               file the first line start of the range, its line starts, the FASTA header rule over them and the
+ *               first FASTQ header candidate.  Computed once; later calls return the same bytes.
+ *   plan        host arithmetic only, the same on every rank: from every rank's summary (world x 256 bytes, in rank
+ *               order) where each range starts and how many records come before it.  SDTGPU_EINVAL if a summary is of
+ *               other files, sizes, FASTQ-ness or world, or out of order.  out = { records this rank returns,
+ *               records of the library, n1, n2 (0 single-ended) }.
+ *   next        as for a plain reader, SDTGPU_ESTATE before plan; one call never returns records across a jump in
+ *               ordinals (a rank's pairs, then its records of the longer file).
+ *   tell        the ordinal of the next record (nothing left: one past the last one returned); on a plain reader
+ *               the records returned so far.  SDTGPU_ESTATE on a shard reader before plan.
+ *   plan_exchange (csrc/sdt_nccl.cu)  summary, all-gather of the summaries over the library's communicator (a device
+ *               buffer of world x 256 bytes), plan.  Collective; SDTGPU_EINVAL before any collective if the
+ *               communicator's rank or world is not the reader's.
+ * summary and plan on a plain reader are SDTGPU_ESTATE.  The text bytes of sdtgpu_reader_stats count the summary pass
+ * and the seeks too: a rank reads its range twice (summary, parse), at most a chunk past its end, and for the file-2
+ * half of its pairs (and its records of the longer file) the text from the start of the range that holds the first of
+ * them: a few records when both files lay their records out alike, up to one range otherwise. */
+#define SDTGPU_READER_SUMMARY_BYTES 256
+int sdtgpu_reader_open_shard (sdtgpu_reader_t **out, int device, const char *path1, const char *path2, int fastq,
+			      uint64_t chunk_bytes, int rank, int world);
+int sdtgpu_reader_summary (sdtgpu_reader_t *r, uint8_t out[SDTGPU_READER_SUMMARY_BYTES]);
+int sdtgpu_reader_plan (sdtgpu_reader_t *r, const uint8_t *summaries, uint64_t out[4]);
+int sdtgpu_reader_tell (const sdtgpu_reader_t *r, uint64_t *ordinal);
+int sdtgpu_reader_plan_exchange (sdtgpu_reader_t *r, sdtgpu_comm_t *c, uint64_t out[4]);
+
 /* reference helpers restated for host callers (tests bind them) */
 uint64_t sdtgpu_hash_kmer (const uint64_t key[4], int key_words);	/* hashFunction.c:108 */
 int sdtgpu_version (void);

@@ -416,3 +416,71 @@ int sdtgpu_lookup_reads_exchange (sdtgpu_t *h, sdtgpu_comm_t *c, const uint8_t *
 }
 
 }	// extern "C"
+
+int sdt_reader_shard (const sdtgpu_reader_t *r, int *rank, int *world);	// csrc/sdt_parse.cu
+
+namespace {
+
+// the all-gather of plan_exchange: this rank's 256 bytes in, everybody's out (rank order)
+int gather_summaries (sdtgpu_comm *c, const uint8_t *mine, std::vector<uint8_t> &all)
+{
+	const size_t B = SDTGPU_READER_SUMMARY_BYTES;
+	cudaStream_t s = nullptr;
+	uint8_t *d = nullptr;
+	int rc = SDTGPU_OK;
+	auto step = [&] (int code, const std::string &what) { if (!rc && code) rc = comm_fail (c, code, what); };
+	auto cu = [&] (cudaError_t e, const char *what) { step (e == cudaSuccess ? SDTGPU_OK : SDTGPU_ECUDA, std::string (what) + ": " + cudaGetErrorString (e)); };
+	cu (cudaSetDevice (c->device), "cudaSetDevice");
+	if (!rc)
+		cu (cudaStreamCreateWithFlags (&s, cudaStreamNonBlocking), "cudaStreamCreateWithFlags");
+	if (!rc)
+		cu (cudaMalloc (&d, B * (size_t) c->world), "cudaMalloc");
+	if (!rc)	// in place: this rank's block is already where the all-gather puts it
+		cu (cudaMemcpyAsync (d + B * (size_t) c->rank, mine, B, cudaMemcpyHostToDevice, s), "cudaMemcpyAsync");
+	if (!rc)
+	{
+		const ncclResult_t r = g_nccl.AllGather (d + B * (size_t) c->rank, d, B, ncclUint8, c->comm, s);
+		step (r == ncclSuccess ? SDTGPU_OK : SDTGPU_ECUDA, std::string ("ncclAllGather: ") + (r == ncclSuccess ? "" : g_nccl.GetErrorString (r)));
+	}
+	if (!rc)
+		cu (cudaMemcpyAsync (all.data (), d, B * (size_t) c->world, cudaMemcpyDeviceToHost, s), "cudaMemcpyAsync");
+	if (s)
+		cu (cudaStreamSynchronize (s), "cudaStreamSynchronize");
+	if (d)
+		cudaFree (d);
+	if (s)
+		cudaStreamDestroy (s);
+	return rc;
+}
+
+}	// namespace
+
+extern "C" int sdtgpu_reader_plan_exchange (sdtgpu_reader_t *r, sdtgpu_comm_t *c, uint64_t out[4])
+{
+	if (!r || !c || !out)
+		return comm_fail (nullptr, SDTGPU_EINVAL, "sdtgpu_reader_plan_exchange: NULL reader, communicator or output");
+	int rank = 0, world = 0;
+	sdt_reader_shard (r, &rank, &world);
+	if (!world)
+		return comm_fail (c, SDTGPU_ESTATE, "sdtgpu_reader_plan_exchange needs a reader made by sdtgpu_reader_open_shard");
+	if (rank != c->rank || world != c->world)
+	{
+		char b[200];
+		snprintf (b, sizeof b, "sdtgpu_reader_plan_exchange: the reader is rank %d of %d, the communicator rank %d of %d", rank, world, c->rank, c->world);
+		return comm_fail (c, SDTGPU_EINVAL, b);
+	}
+	// a rank whose summary fails still takes part: its all-zero block makes every rank's plan refuse
+	uint8_t mine[SDTGPU_READER_SUMMARY_BYTES];
+	const int src = sdtgpu_reader_summary (r, mine);
+	if (src)
+		memset (mine, 0, sizeof mine);
+	std::vector<uint8_t> all ((size_t) world * SDTGPU_READER_SUMMARY_BYTES);
+	int rc = gather_summaries (c, mine, all);
+	if (rc)
+		return rc;
+	if (src)
+		return comm_fail (c, src, std::string ("sdtgpu_reader_summary: ") + sdtgpu_reader_last_error (r));
+	if ((rc = sdtgpu_reader_plan (r, all.data (), out)))
+		return comm_fail (c, rc, std::string ("sdtgpu_reader_plan: ") + sdtgpu_reader_last_error (r));
+	return SDTGPU_OK;
+}

@@ -380,6 +380,63 @@ __global__ void parse_finalize_kernel (int fastq, int first, int eof, u32 len, c
 	*res = r;
 }
 
+// ---- a shard's summary (sdtgpu_reader_summary): per piece of the rank's byte range, the lines j_lo .. n_lines - 1
+// of the piece (line 0 is not a line start of the file when the byte before the piece is not '\n')
+struct SumRes
+{
+	Tr tr;			// FASTA: the lines as one transfer function
+	u32 first;		// start of line j_lo (NONE: the piece holds no line start)
+	u32 open[2];		// FASTQ: start of the '@' line n_lines - 2 + k if its line two further down is not in the piece
+	u64 cand;		// FASTQ: (line << 32 | start) of the first '@' line whose line two further down starts with '+'
+};
+
+__global__ void __launch_bounds__ (LINE_THREADS)
+shard_fa_tile_kernel (const char *text, const u32 *nl, u32 j_lo, u32 n_lines, Tr *agg)
+{
+	__shared__ Tr sh[17];
+	const u32 j0 = blockIdx.x * TILE_LINES + threadIdx.x * LINES_PER_THREAD;
+	Tr t = tr_id ();
+#pragma unroll
+	for (int k = 0; k < LINES_PER_THREAD; k++)
+		if (j0 + k >= j_lo && j0 + k < n_lines)
+			t = tr_then (t, tr_line (text[line_start (nl, j0 + k)] == '>'));
+	Tr total;
+	tr_block_excl (t, sh, &total);
+	if (threadIdx.x == 0)
+		agg[blockIdx.x] = total;
+}
+
+// one warp: the tiles composed into res->tr, and the piece's first line start
+__global__ void shard_piece_kernel (const Tr *agg, u32 nt, const u32 *nl, u32 j_lo, u32 n_lines, SumRes *res)
+{
+	const int lane = threadIdx.x;
+	Tr carry = tr_id ();
+	for (u32 i0 = 0; i0 < nt; i0 += 32)
+	{
+		const Tr inc = tr_warp_incl (i0 + lane < nt ? agg[i0 + lane] : tr_id ());
+		carry = tr_then (carry, Tr{__shfl_sync (0xFFFFFFFFu, inc.f, 31), __shfl_sync (0xFFFFFFFFu, inc.c0, 31), __shfl_sync (0xFFFFFFFFu, inc.c1, 31)});
+	}
+	if (lane == 0)
+	{
+		res->tr = carry;
+		res->first = j_lo < n_lines ? line_start (nl, j_lo) : NONE;
+	}
+}
+
+// the parse_fq_find_kernel rule from line j_lo on; lines whose line two further down lies past the piece are left to
+// the host, which reads on in the file
+__global__ void __launch_bounds__ (256)
+shard_fq_find_kernel (const char *text, const u32 *nl, u32 j_lo, u32 n_lines, SumRes *res)
+{
+	const u32 i = j_lo + blockIdx.x * 256 + threadIdx.x;
+	if (i >= n_lines || text[line_start (nl, i)] != '@')
+		return;
+	if (i + 2 >= n_lines)
+		res->open[i + 2 - n_lines] = line_start (nl, i);
+	else if (text[line_start (nl, i + 2)] == '+')
+		atomicMin (&res->cand, (u64) i << 32 | line_start (nl, i));
+}
+
 // ---- pack: one warp per record, straight to its output row
 
 __device__ __forceinline__ u32 base_code (u32 c, int n_kmer)
@@ -485,7 +542,59 @@ struct File
 	u32 len = 0, cursor = 0;
 	ChunkRes res{};
 	bool eof = false, first = true;
-	bool exhausted () const { return cur >= 0 && eof && cursor == res.n_rec; }
+	// a shard reader's position: the first chunk starts at `origin`, the next record is record `rec` of the file,
+	// and `left` more records may be taken (ALL: no budget, a plain reader)
+	u64 origin = 0, rec = 0, left = ~0ull;
+	bool placed = false;
+	u64 fingerprint = 0;
+	bool exhausted () const { return left == 0 || (cur >= 0 && eof && cursor == res.n_rec); }
+};
+
+constexpr u64 ALL = ~0ull;
+constexpr u64 SUM_MAGIC = 0x31304d5553544453ull;	// "SDTSUM01"
+
+// a run of FASTA lines as a function of the state before it, with 64-bit header counts (host side of Tr)
+struct Tr64
+{
+	u32 f = 2;
+	u64 c0 = 0, c1 = 0;
+	u32 state (u32 P) const { return (f >> P) & 1u; }
+	u64 count (u32 P) const { return P ? c1 : c0; }
+	Tr64 then (const Tr64 &b) const
+	{
+		const u32 a0 = f & 1u, a1 = (f >> 1) & 1u;
+		Tr64 t;
+		t.f = b.state (a0) | b.state (a1) << 1;
+		t.c0 = c0 + b.count (a0);
+		t.c1 = c1 + b.count (a1);
+		return t;
+	}
+};
+
+// what a summary holds per file (sdtgpu_reader_summary), for this rank's range of it
+struct FileSum
+{
+	u64 first = ALL;	// offset of the range's first line start (ALL: none)
+	u64 n_lines = 0;	// line starts in the range
+	Tr64 tr;		// FASTA: those lines
+	u64 cand = ALL;		// FASTQ: offset of the first header candidate (ALL: none) ...
+	u64 cand_line = 0;	// ... and its line number in the range
+};
+
+// where a shard reader enters the ranges of a file: the record numbers before every range (c[q], q = 0 .. world)
+// and the start of range q's first record, `skip` lines after its first line start `off`
+struct FilePlan
+{
+	std::vector<u64> c, off;
+	std::vector<uint8_t> skip;
+};
+
+// records k0 .. k1 - 1 of one file (file 0 or 1), or of both alternately (file -1, a pair segment); ordinals from ord0
+struct Seg
+{
+	int file = 0;
+	u64 k0 = 0, k1 = 0, ord0 = 0;
+	u64 size () const { return (file < 0 ? 2 : 1) * (k1 - k0); }
 };
 
 }	// namespace
@@ -499,6 +608,16 @@ struct sdtgpu_reader
 	cudaStream_t stream = nullptr;
 	u64 stats[4] = {0, 0, 0, 0};
 	std::string err;
+	// shard readers (sdtgpu_reader_open_shard): world = 0 is a plain reader
+	int rank = 0, world = 0;
+	bool summarized = false, planned = false;
+	uint8_t summary[SDTGPU_READER_SUMMARY_BYTES] = {};
+	FilePlan plan[2];
+	Seg seg[3];			// pairs (or the one file's records), drain, and an empty one past the end
+	int seg_i = 0;			// the current segment
+	u64 seg_done = 0;		// records of it returned
+	bool seg_ready = false;		// the files are placed for it
+	SumRes *d_sum = nullptr, *h_sum = nullptr;
 };
 
 namespace {
@@ -638,7 +757,7 @@ int grow_scratch (sdtgpu_reader *r, File &f, u64 text_cap)
 int load_chunk (sdtgpu_reader *r, File &f)
 {
 	const bool have = f.cur >= 0;
-	u64 start = 0, tail = 0;
+	u64 start = f.origin, tail = 0;
 	if (have)
 	{
 		start = f.chunk_start + f.res.next;
@@ -733,6 +852,8 @@ int fill (sdtgpu_reader *r, File &f)
 {
 	while (!(f.cur >= 0 && f.cursor < f.res.n_rec) && !f.exhausted ())
 		RET (load_chunk (r, f));
+	if (f.left != ALL && f.left && f.exhausted ())
+		return reader_fail (r, SDTGPU_ESTATE, f.path + " holds fewer records than the summaries counted (did it change?)");
 	return SDTGPU_OK;
 }
 
@@ -771,7 +892,11 @@ int pack (sdtgpu_reader *r, File &f, u32 n, u64 out0, u64 step, const Out &o)
 	RCK (r, cudaGetLastError ());
 	RCK (r, cudaEventRecord (S.packed, o.stream));
 	f.cursor += n;
+	f.rec += n;
+	if (f.left != ALL)
+		f.left -= n;
 	r->stats[1] += n;
+	r->seg_done += n;
 	return SDTGPU_OK;
 }
 
@@ -794,11 +919,325 @@ int init_cuda (sdtgpu_reader *r)
 		RCK (r, cudaHostAlloc ((void **) &f.h_res, sizeof (ChunkRes), cudaHostAllocDefault));
 		RCK (r, cudaMalloc ((void **) &f.d_res, sizeof (ChunkRes)));
 	}
+	if (r->world)
+	{
+		RCK (r, cudaHostAlloc ((void **) &r->h_sum, sizeof (SumRes), cudaHostAllocDefault));
+		RCK (r, cudaMalloc ((void **) &r->d_sum, sizeof (SumRes)));
+	}
 	r->cuda_ready = true;
 	return SDTGPU_OK;
 }
 
+// ---- shard readers: a summary of this rank's byte range of each file, a plan from every rank's summary, and the
+// segments of records this rank returns
+
+// rank q's range of a file of `size` bytes starts here
+u64 range_lo (u64 size, int q, int world) { return (u64) ((unsigned __int128) size * (u64) q / (u64) world); }
+
+// FNV-1a of the first and last 4 KiB: tells two files of the same size apart in nearly every case
+int fingerprint (sdtgpu_reader *r, File &f)
+{
+	const u64 n = std::min<u64> (4096, f.size);
+	std::vector<char> b (2 * n);
+	if (n)
+	{
+		RET (read_range (r, f, b.data (), 0, n));
+		RET (read_range (r, f, b.data () + n, f.size - n, n));
+	}
+	u64 h = 0xcbf29ce484222325ull;
+	for (char c : b)
+		h = (h ^ (unsigned char) c) * 0x100000001b3ull;
+	f.fingerprint = h;
+	return SDTGPU_OK;
+}
+
+// FASTQ header rule for the '@' line at p, on the host: the line two further down starts with '+' or is past the end
+int fq_rule_on_host (sdtgpu_reader *r, File &f, u64 p, bool *yes)
+{
+	u64 q;
+	RET (skip_line (r, f, p, &q));
+	RET (skip_line (r, f, q, &q));
+	char c = 0;
+	if (q < f.size)
+		RET (read_range (r, f, &c, q, 1));
+	*yes = q >= f.size || c == '+';
+	return SDTGPU_OK;
+}
+
+// this rank's range of f, streamed through the device in pieces of at most stage_bytes: line starts, the FASTA
+// transfer function of those lines and the first FASTQ header candidate
+int summarize_file (sdtgpu_reader *r, File &f, FileSum &s)
+{
+	s = FileSum{};
+	const u64 a = range_lo (f.size, r->rank, r->world), b = range_lo (f.size, r->rank + 1, r->world);
+	if (a >= b)
+		return SDTGPU_OK;
+	char prev = '\n';	// the byte before the piece; offset 0 starts a line
+	if (a)
+		RET (read_range (r, f, &prev, a - 1, 1));
+	Slot &S = f.slot[0];
+	for (u64 x = a; x < b;)
+	{
+		const u64 n = std::min (r->stage_bytes, b - x);
+		const int si = f.stage_next;
+		if (f.stage_off[si] != x || f.stage_len[si] < n)
+			RET (fill_stage (r, f, si, x));
+		RET (grow (r, S, (void **) &S.text, &S.text_cap, n + 64));
+		RET (grow_scratch (r, f, S.text_cap));
+		RCK (r, cudaMemcpyAsync (S.text, f.stage[si], n, cudaMemcpyHostToDevice, r->stream));
+		r->stats[0] += n;
+		r->stats[2]++;
+		f.stage_next ^= 1;
+		const u32 L = (u32) n, nb = (u32) ((n + NL_BLOCK_BYTES - 1) / NL_BLOCK_BYTES);
+		u32 *blk_cnt = f.scratch, *blk_off = f.scratch + nb;
+		parse_nl_count_kernel<<<nb, NL_THREADS, 0, r->stream>>> (S.text, L, blk_cnt);
+		parse_nl_scan_kernel<<<1, 1024, 0, r->stream>>> (blk_cnt, nb, blk_off, S.text, L, f.d_res);
+		RCK (r, cudaGetLastError ());
+		RCK (r, cudaMemcpyAsync (f.h_res, f.d_res, sizeof (ChunkRes), cudaMemcpyDeviceToHost, r->stream));
+		const char last = f.stage[si][n - 1];
+		if (x + n < b)	// while that runs: the next piece
+			RET (fill_stage (r, f, f.stage_next, x + n));
+		RCK (r, cudaStreamSynchronize (r->stream));
+		const u32 T = f.h_res->T, n_lines = f.h_res->n_lines, j_lo = prev == '\n' ? 0 : 1;
+		RET (grow (r, S, (void **) &S.nl, &S.nl_cap, ((u64) T + 1) * sizeof (u32)));
+		parse_nl_write_kernel<<<nb, NL_THREADS, 0, r->stream>>> (S.text, L, blk_off, S.nl);
+		RCK (r, cudaMemsetAsync (r->d_sum, 0xFF, sizeof (SumRes), r->stream));
+		const bool find = r->fastq && s.cand == ALL && n_lines > j_lo;
+		if (find)
+			shard_fq_find_kernel<<<(n_lines - j_lo + 255) / 256, 256, 0, r->stream>>> (S.text, S.nl, j_lo, n_lines, r->d_sum);
+		const u32 nt = r->fastq ? 0 : (n_lines + TILE_LINES - 1) / TILE_LINES;
+		Tr *agg = reinterpret_cast<Tr *> (blk_off + nb);
+		if (nt)
+			shard_fa_tile_kernel<<<nt, LINE_THREADS, 0, r->stream>>> (S.text, S.nl, j_lo, n_lines, agg);
+		shard_piece_kernel<<<1, 32, 0, r->stream>>> (agg, nt, S.nl, j_lo, n_lines, r->d_sum);
+		RCK (r, cudaGetLastError ());
+		RCK (r, cudaMemcpyAsync (r->h_sum, r->d_sum, sizeof (SumRes), cudaMemcpyDeviceToHost, r->stream));
+		RCK (r, cudaStreamSynchronize (r->stream));
+		const SumRes h = *r->h_sum;
+		if (s.first == ALL && h.first != NONE)
+			s.first = x + h.first;
+		if (find && h.cand != ~0ull)
+		{
+			s.cand = x + (u32) h.cand;
+			s.cand_line = s.n_lines + (h.cand >> 32) - j_lo;
+		}
+		for (int k = 0; find && k < 2 && s.cand == ALL; k++)
+			if (h.open[k] != NONE)
+			{	// line n_lines - 2 + k: the line two further down is in a later piece, or past the range
+				bool yes;
+				RET (fq_rule_on_host (r, f, x + h.open[k], &yes));
+				if (yes)
+				{
+					s.cand = x + h.open[k];
+					s.cand_line = s.n_lines + (n_lines - 2 + k) - j_lo;
+				}
+			}
+		s.tr = s.tr.then (Tr64{h.tr.f, h.tr.c0, h.tr.c1});
+		s.n_lines += n_lines > j_lo ? n_lines - j_lo : 0;
+		prev = last;
+		x += n;
+	}
+	return SDTGPU_OK;
+}
+
+void encode_summary (sdtgpu_reader *r, const FileSum *fs)
+{
+	u64 w[SDTGPU_READER_SUMMARY_BYTES / 8] = {};
+	w[0] = SUM_MAGIC;
+	w[1] = (u64) r->rank;
+	w[2] = (u64) r->world;
+	w[3] = (u64) r->fastq;
+	w[4] = (u64) r->n_files;
+	w[5] = r->f[0].size;
+	w[6] = r->n_files == 2 ? r->f[1].size : 0;
+	for (int i = 0; i < r->n_files; i++)
+	{
+		u64 *p = w + 8 + 8 * i;
+		p[0] = fs[i].first;
+		p[1] = fs[i].n_lines;
+		p[2] = fs[i].tr.f;
+		p[3] = fs[i].tr.c0;
+		p[4] = fs[i].tr.c1;
+		p[5] = fs[i].cand;
+		p[6] = fs[i].cand_line;
+		p[7] = r->f[i].fingerprint;
+	}
+	memcpy (r->summary, w, sizeof w);
+}
+
+// host arithmetic only: every rank runs it on the same summaries and gets the same c[] and entries
+int make_plan (sdtgpu_reader *r, const uint8_t *all, uint64_t out[4])
+{
+	r->planned = false;
+	const int W = r->world;
+	constexpr int WORDS = SDTGPU_READER_SUMMARY_BYTES / 8;
+	std::vector<u64> w ((size_t) W * WORDS);
+	memcpy (w.data (), all, (size_t) W * SDTGPU_READER_SUMMARY_BYTES);
+	for (int q = 0; q < W; q++)
+	{
+		const u64 *s = &w[(size_t) q * WORDS];
+		bool ok = s[0] == SUM_MAGIC && s[1] == (u64) q && s[2] == (u64) W && s[3] == (u64) r->fastq && s[4] == (u64) r->n_files
+			  && s[5] == r->f[0].size && s[6] == (r->n_files == 2 ? r->f[1].size : 0);
+		for (int i = 0; ok && i < r->n_files; i++)
+		{
+			const u64 *p = s + 8 + 8 * i;
+			ok = p[7] == r->f[i].fingerprint && p[2] < 4 && (p[5] == ALL || p[6] < p[1]);
+		}
+		if (!ok)
+			return reader_fail (r, SDTGPU_EINVAL, "summary " + std::to_string (q) + " is not rank " + std::to_string (q) + " of " +
+					    std::to_string (W) + " over the same files (sizes, contents, FASTA/FASTQ) as this reader");
+		if (q == r->rank && r->summarized && memcmp (s, r->summary, SDTGPU_READER_SUMMARY_BYTES))
+			return reader_fail (r, SDTGPU_EINVAL, "summary " + std::to_string (q) + " is not the one this reader made");
+	}
+	for (int i = 0; i < r->n_files; i++)
+	{
+		FilePlan &P = r->plan[i];
+		P.c.assign (W + 1, 0);
+		P.off.assign (W, ALL);
+		P.skip.assign (W, 0);
+		auto sum = [&] (int q) { return &w[(size_t) q * WORDS + 8 + 8 * i]; };
+		if (!r->fastq)
+		{	// the state before range q is the ranks before it composed from state 0
+			u32 P_state = 0;
+			for (int q = 0; q < W; q++)
+			{
+				const u64 *p = sum (q);
+				const Tr64 t{(u32) p[2], p[3], p[4]};
+				P.off[q] = p[0];
+				P.skip[q] = (uint8_t) P_state;	// P = 1: the first line is the sequence line of a header before it
+				P.c[q + 1] = P.c[q] + t.count (P_state);
+				P_state = t.state (P_state);
+			}
+			continue;
+		}
+		// FASTQ: headers are lines h0, h0 + 4, ... of the file, h0 the first candidate of any range
+		std::vector<u64> L (W + 1, 0);
+		int qs = -1;
+		for (int q = 0; q < W; q++)
+		{
+			L[q + 1] = L[q] + sum (q)[1];
+			if (qs < 0 && sum (q)[5] != ALL)
+				qs = q;
+		}
+		if (qs < 0)
+			continue;
+		const u64 h0 = L[qs] + sum (qs)[6];
+		for (int q = 0; q <= W; q++)
+			P.c[q] = L[q] > h0 ? (L[q] - h0 + 3) / 4 : 0;
+		for (int q = qs; q < W; q++)
+		{
+			P.off[q] = q == qs ? sum (q)[5] : sum (q)[0];
+			P.skip[q] = q == qs ? 0 : (uint8_t) ((4 - (L[q] - h0) % 4) % 4);
+		}
+	}
+	const int k = r->rank;
+	const std::vector<u64> &c1 = r->plan[0].c;
+	const u64 n1 = c1[W], n2 = r->n_files == 2 ? r->plan[1].c[W] : 0;
+	if (r->n_files == 1)
+	{
+		r->seg[0] = Seg{0, c1[k], c1[k + 1], c1[k]};
+		r->seg[1] = Seg{};
+	}
+	else
+	{	// pairs of this rank's file-1 records, then this rank's records of the longer file past the pairs
+		const u64 m = std::min (n1, n2);
+		const u64 p0 = std::min (m, c1[k]), p1 = std::min (m, c1[k + 1]);
+		r->seg[0] = Seg{-1, p0, p1, 2 * p0};
+		const int lf = n1 >= n2 ? 0 : 1;
+		const std::vector<u64> &cl = r->plan[lf].c;
+		const u64 d0 = std::max (m, cl[k]), d1 = std::max (m, cl[k + 1]);
+		r->seg[1] = Seg{lf, d0, d1, m + d0};
+	}
+	r->seg[2] = Seg{};
+	r->seg_i = 0;
+	r->seg_done = 0;
+	r->seg_ready = false;
+	for (File &f : r->f)
+	{
+		f.placed = false;
+		f.left = 0;
+	}
+	r->planned = true;
+	out[0] = r->seg[0].size () + r->seg[1].size ();
+	out[1] = n1 + n2;
+	out[2] = n1;
+	out[3] = n2;
+	return SDTGPU_OK;
+}
+
+// file fi at record k (k < its record count): enter the range that holds record k, then consume records without
+// packing them up to k.  Entering a range starts a chunk `skip` lines after its first line start (FASTA: past the
+// sequence line of a header before the range; FASTQ: on the next line that is 0 mod 4 from the first header)
+int seek (sdtgpu_reader *r, int fi, u64 k)
+{
+	File &f = r->f[fi];
+	if (f.placed && f.rec == k)
+		return SDTGPU_OK;
+	const FilePlan &P = r->plan[fi];
+	const int q = (int) (std::upper_bound (P.c.begin (), P.c.end (), k) - P.c.begin ()) - 1;	// c[q] <= k < c[q + 1]
+	u64 off = P.off[q];
+	for (int i = 0; i < P.skip[q]; i++)
+		RET (skip_line (r, f, off, &off));
+	f.cur = -1;
+	f.origin = off;
+	f.eof = false;
+	f.first = false;	// FASTQ: the first header is known
+	f.res = ChunkRes{};
+	f.cursor = 0;
+	f.rec = P.c[q];
+	f.placed = true;
+	for (f.left = k - f.rec; f.left;)
+	{
+		RET (fill (r, f));
+		const u32 n = (u32) std::min<u64> (f.res.n_rec - f.cursor, f.left);
+		f.cursor += n;
+		f.rec += n;
+		f.left -= n;
+	}
+	return SDTGPU_OK;
+}
+
+// places the files for the current segment and gives each its budget
+int seg_enter (sdtgpu_reader *r)
+{
+	if (r->seg_ready)
+		return SDTGPU_OK;
+	const Seg &s = r->seg[r->seg_i];
+	for (int i = 0; i < r->n_files; i++)
+		r->f[i].left = 0;
+	for (int i = 0; i < r->n_files && s.size (); i++)
+		if (s.file < 0 || s.file == i)
+		{
+			RET (seek (r, i, s.k0));
+			r->f[i].left = s.k1 - s.k0;
+		}
+	r->seg_ready = true;
+	return SDTGPU_OK;
+}
+
+// the current segment is done: moves to the next one; true if the same call may go on with it (it has records and
+// its ordinals follow on, or the call has returned nothing yet)
+bool seg_advance (sdtgpu_reader *r, u64 got)
+{
+	if (r->seg_i >= 2)
+		return false;
+	const u64 end = r->seg[r->seg_i].ord0 + r->seg[r->seg_i].size ();
+	r->seg_i++;
+	r->seg_done = 0;
+	r->seg_ready = false;
+	const Seg &s = r->seg[r->seg_i];
+	return s.size () && (got == 0 || s.ord0 == end);
+}
+
 }	// namespace
+
+// rank and world of a reader (world 0: a plain reader), for csrc/sdt_nccl.cu
+int sdt_reader_shard (const sdtgpu_reader *r, int *rank, int *world)
+{
+	*rank = r->rank;
+	*world = r->world;
+	return SDTGPU_OK;
+}
 
 extern "C" {
 
@@ -832,6 +1271,8 @@ void sdtgpu_reader_close (sdtgpu_reader_t *r)
 			cudaFreeHost (f.stage[0]);
 			cudaFreeHost (f.stage[1]);
 		}
+		cudaFree (r->d_sum);
+		cudaFreeHost (r->h_sum);
 		if (r->stream)
 			cudaStreamDestroy (r->stream);
 	}
@@ -888,36 +1329,126 @@ int sdtgpu_reader_next (sdtgpu_reader_t *r, void *stream, int max_read_len, int 
 	const size_t smem = (size_t) words * 4 * PACK_WARPS;
 	if (smem > 48 * 1024)
 		return reader_fail (r, SDTGPU_EINVAL, "stride_bytes too large for the pack kernel (at most 4096 with n_kmer, 6144 without)");
+	if (r->world && !r->planned)
+		return reader_fail (r, SDTGPU_ESTATE, "a shard reader needs sdtgpu_reader_plan before sdtgpu_reader_next");
 	RCK (r, cudaSetDevice (r->device));
 	if (!r->cuda_ready)
 		RET (init_cuda (r));
 	const Out o{d_packed, d_nmask, d_lens, max_read_len, n_kmer, reverse, stride_bytes, (cudaStream_t) stream, smem};
 	const u64 M = r->n_files == 2 ? max_reads & ~1ull : max_reads;
 	u64 got = 0;
-	while (got < M)
-	{
-		File &a = r->f[0], &b = r->f[1];
-		if (r->n_files == 2 && !a.exhausted () && !b.exhausted ())
-		{	// alternate file 1 / file 2 while both have records
-			RET (fill (r, a));
-			RET (fill (r, b));
-			if (a.exhausted () || b.exhausted ())
+	for (;;)
+	{	// a plain reader runs this once; a shard reader once per segment, as long as the ordinals follow on
+		if (r->world)
+			RET (seg_enter (r));
+		while (got < M)
+		{
+			File &a = r->f[0], &b = r->f[1];
+			if (r->n_files == 2 && !a.exhausted () && !b.exhausted ())
+			{	// alternate file 1 / file 2 while both have records
+				RET (fill (r, a));
+				RET (fill (r, b));
+				if (a.exhausted () || b.exhausted ())
+					continue;
+				const u32 n = (u32) std::min<u64> ({a.res.n_rec - a.cursor, b.res.n_rec - b.cursor, a.left, b.left, (M - got) / 2});
+				RET (pack (r, a, n, got, 2, o));
+				RET (pack (r, b, n, got + 1, 2, o));
+				got += 2 * (u64) n;
 				continue;
-			const u32 n = (u32) std::min<u64> ({a.res.n_rec - a.cursor, b.res.n_rec - b.cursor, (M - got) / 2});
-			RET (pack (r, a, n, got, 2, o));
-			RET (pack (r, b, n, got + 1, 2, o));
-			got += 2 * (u64) n;
-			continue;
+			}
+			File &f = r->n_files == 1 || !a.exhausted () ? a : b;	// then the rest of the longer one
+			RET (fill (r, f));
+			if (f.exhausted ())
+				break;
+			const u32 n = (u32) std::min<u64> ({f.res.n_rec - f.cursor, f.left, M - got});
+			RET (pack (r, f, n, got, 1, o));
+			got += n;
 		}
-		File &f = r->n_files == 1 || !a.exhausted () ? a : b;	// then the rest of the longer one
-		RET (fill (r, f));
-		if (f.exhausted ())
+		if (!r->world || got == M || !seg_advance (r, got))
 			break;
-		const u32 n = (u32) std::min<u64> (f.res.n_rec - f.cursor, M - got);
-		RET (pack (r, f, n, got, 1, o));
-		got += n;
 	}
 	*n_out = got;
+	return SDTGPU_OK;
+}
+
+int sdtgpu_reader_open_shard (sdtgpu_reader_t **out, int device, const char *path1, const char *path2, int fastq,
+			      uint64_t chunk_bytes, int rank, int world)
+{
+	if (!out || !path1 || world < 1 || world > 1024 || rank < 0 || rank >= world)
+	{
+		g_reader_open_error = "sdtgpu_reader_open_shard: need out and path1, and 0 <= rank < world <= 1024";
+		return SDTGPU_EINVAL;
+	}
+	RET (sdtgpu_reader_open (out, device, path1, path2, fastq, chunk_bytes));
+	sdtgpu_reader *r = *out;
+	r->rank = rank;
+	r->world = world;
+	for (int i = 0; i < r->n_files; i++)
+		if (fingerprint (r, r->f[i]))
+		{
+			g_reader_open_error = r->err;
+			sdtgpu_reader_close (r);
+			*out = nullptr;
+			return SDTGPU_EINVAL;
+		}
+	return SDTGPU_OK;
+}
+
+int sdtgpu_reader_summary (sdtgpu_reader_t *r, uint8_t out[SDTGPU_READER_SUMMARY_BYTES])
+{
+	if (!r || !out)
+		return SDTGPU_EINVAL;
+	if (!r->world)
+		return reader_fail (r, SDTGPU_ESTATE, "sdtgpu_reader_summary needs a reader made by sdtgpu_reader_open_shard");
+	if (!r->summarized)
+	{
+		if (r->planned)
+			return reader_fail (r, SDTGPU_ESTATE, "sdtgpu_reader_summary comes before sdtgpu_reader_plan");
+		RCK (r, cudaSetDevice (r->device));
+		if (!r->cuda_ready)
+			RET (init_cuda (r));
+		FileSum fs[2];
+		for (int i = 0; i < r->n_files; i++)
+			RET (summarize_file (r, r->f[i], fs[i]));
+		encode_summary (r, fs);
+		r->summarized = true;
+	}
+	memcpy (out, r->summary, SDTGPU_READER_SUMMARY_BYTES);
+	return SDTGPU_OK;
+}
+
+int sdtgpu_reader_plan (sdtgpu_reader_t *r, const uint8_t *summaries, uint64_t out[4])
+{
+	if (!r || !summaries || !out)
+		return SDTGPU_EINVAL;
+	if (!r->world)
+		return reader_fail (r, SDTGPU_ESTATE, "sdtgpu_reader_plan needs a reader made by sdtgpu_reader_open_shard");
+	return make_plan (r, summaries, out);
+}
+
+int sdtgpu_reader_tell (const sdtgpu_reader_t *r, uint64_t *ordinal)
+{
+	if (!r || !ordinal)
+		return SDTGPU_EINVAL;
+	if (!r->world)
+	{
+		*ordinal = r->stats[1];
+		return SDTGPU_OK;
+	}
+	if (!r->planned)
+		return SDTGPU_ESTATE;
+	for (int i = r->seg_i; i < 2; i++)
+	{
+		const u64 done = i == r->seg_i ? r->seg_done : 0;
+		if (done < r->seg[i].size ())
+		{
+			*ordinal = r->seg[i].ord0 + done;
+			return SDTGPU_OK;
+		}
+	}
+	// nothing left: one past the last record this rank returns (where its share starts if it returns none)
+	const Seg &s = r->seg[1].size () ? r->seg[1] : r->seg[0];
+	*ordinal = s.ord0 + s.size ();
 	return SDTGPU_OK;
 }
 

@@ -309,3 +309,24 @@ class SkmExchange:
         self.host_ms["flushes"] = self.host_ms.get("flushes", 0) + 1
         self.host_log.append([round(1e3 * (b - a), 2) for a, b in ((t0, t1), (t1, t2), (t2, t3), (t3, t4))])   # per flush: bound, stage, exchange, import
         return total
+
+
+def plan_reader(reader, dev, group=None) -> dict:
+    """Plans a shard reader (pregraph.DeviceReadPacker(..., rank=, world=)) over torch.distributed: this rank's summary,
+    an all-gather of every rank's 256 bytes, then the same host-side plan on every rank.  Collective over `group`,
+    whose rank and size must be the reader's.  Returns the plan (records this rank returns, library_records, n1, n2)."""
+    world = dist.get_world_size(group)
+    if world != reader.world:
+        raise ValueError(f"plan_reader: the group has {world} ranks, the reader {reader.world}")
+    err = None
+    try:
+        mine = reader.summary()
+    except Exception as e:      # noqa: BLE001  (the other ranks are in the all-gather: an all-zero block makes every plan refuse)
+        mine, err = bytes(reader.SUMMARY_BYTES), e
+    t = torch.frombuffer(bytearray(mine), dtype=torch.uint8).to(dev)
+    allv = torch.empty((world, reader.SUMMARY_BYTES), dtype=torch.uint8, device=dev)
+    dist.all_gather_into_tensor(allv.view(-1), t, group=group)
+    host = allv.cpu().numpy()
+    if err is not None:
+        raise err
+    return reader.plan([host[r].tobytes() for r in range(world)])

@@ -140,6 +140,11 @@ def library() -> C.CDLL:
     L.sdtgpu_reader_last_error.argtypes = [vp]
     L.sdtgpu_reader_close.argtypes = [vp]
     L.sdtgpu_reader_close.restype = None
+    L.sdtgpu_reader_open_shard.argtypes = [C.POINTER(vp), i32, C.c_char_p, C.c_char_p, i32, u64, i32, i32]
+    L.sdtgpu_reader_summary.argtypes = [vp, vp]
+    L.sdtgpu_reader_plan.argtypes = [vp, vp, vp]
+    L.sdtgpu_reader_tell.argtypes = [vp, C.POINTER(u64)]
+    L.sdtgpu_reader_plan_exchange.argtypes = [vp, vp, vp]
     _lib = L
     return L
 
@@ -581,16 +586,67 @@ class ReadPacker:
 
 class DeviceReadPacker:
     """include/sdtgpu.h sdtgpu_reader_*: FASTA/FASTQ parsed and packed on the GPU.  Same records, order and bytes as
-    ReadPacker, delivered as CUDA tensors in the layout of PregraphGPU.push_reads(..., device=True)."""
+    ReadPacker, delivered as CUDA tensors in the layout of PregraphGPU.push_reads(..., device=True).
 
-    def __init__(self, path1: str, path2: str | None = None, fastq: bool = False, device: int = 0, chunk_bytes: int = 0):
+    world > 0 makes a shard reader (sdtgpu_reader_open_shard): rank `rank` of `world` readers of the same library, each
+    parsing only its own byte range.  Every rank calls summary(), the ranks share the bytes, every rank calls
+    plan(all summaries in rank order) (or plan_exchange(comm) / exchange.plan_reader for both steps), then next();
+    tell() gives the global ordinal of the next record."""
+
+    SUMMARY_BYTES = 256
+
+    def __init__(self, path1: str, path2: str | None = None, fastq: bool = False, device: int = 0, chunk_bytes: int = 0,
+                 rank: int = 0, world: int = 0):
         self.L = library()
         self.h = C.c_void_p()
         self.device = device
-        rc = self.L.sdtgpu_reader_open(C.byref(self.h), device, path1.encode(), path2.encode() if path2 else None,
-                                       int(fastq), chunk_bytes)
+        self.world = world
+        p1, p2 = path1.encode(), path2.encode() if path2 else None
+        if world:
+            rc = self.L.sdtgpu_reader_open_shard(C.byref(self.h), device, p1, p2, int(fastq), chunk_bytes, rank, world)
+        else:
+            rc = self.L.sdtgpu_reader_open(C.byref(self.h), device, p1, p2, int(fastq), chunk_bytes)
         if rc:
             raise SdtGpuError(rc, self.L.sdtgpu_reader_last_error(None).decode())
+
+    def _rck(self, rc: int, what: str):
+        if rc:
+            raise SdtGpuError(rc, f"{what}: " + self.L.sdtgpu_reader_last_error(self.h).decode())
+
+    def summary(self) -> bytes:
+        """This rank's 256-byte summary (a device pass over its byte range the first time)."""
+        buf = (C.c_uint8 * self.SUMMARY_BYTES)()
+        self._rck(self.L.sdtgpu_reader_summary(self.h, buf), "sdtgpu_reader_summary")
+        return bytes(buf)
+
+    @staticmethod
+    def _plan_dict(out) -> dict:
+        return dict(records=int(out[0]), library_records=int(out[1]), n1=int(out[2]), n2=int(out[3]))
+
+    def plan(self, summaries) -> dict:
+        """Plans from every rank's summary, in rank order: {records (this rank returns), library_records, n1, n2}."""
+        summaries = list(summaries)
+        if len(summaries) != self.world or any(len(s) != self.SUMMARY_BYTES for s in summaries):
+            raise SdtGpuError(1, f"plan: need {self.world} summaries of {self.SUMMARY_BYTES} bytes, got {len(summaries)}")
+        blob = b"".join(bytes(s) for s in summaries)
+        buf = (C.c_uint8 * len(blob)).from_buffer_copy(blob)
+        out = (C.c_uint64 * 4)()
+        self._rck(self.L.sdtgpu_reader_plan(self.h, buf, out), "sdtgpu_reader_plan")
+        return self._plan_dict(out)
+
+    def plan_exchange(self, comm: "SkmComm") -> dict:
+        """summary + all-gather over the library's communicator + plan, in one collective call."""
+        out = (C.c_uint64 * 4)()
+        rc = self.L.sdtgpu_reader_plan_exchange(self.h, comm.c, out)
+        if rc:
+            raise SdtGpuError(rc, (self.L.sdtgpu_comm_last_error(comm.c) or self.L.sdtgpu_comm_last_error(None) or b"").decode())
+        return self._plan_dict(out)
+
+    def tell(self) -> int:
+        """The global ordinal of the next record (a plain reader: records returned so far)."""
+        o = C.c_uint64()
+        self._rck(self.L.sdtgpu_reader_tell(self.h, C.byref(o)), "sdtgpu_reader_tell")
+        return int(o.value)
 
     def next(self, max_read_len: int, max_reads: int, n_kmer: bool = False, reverse: bool = False,
              stride_bytes: int | None = None):
