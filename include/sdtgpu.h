@@ -265,6 +265,51 @@ int sdtgpu_lookup_answer (sdtgpu_t *h, uint64_t n);
 int sdtgpu_lookup_unstage_buffer (sdtgpu_t *h, sdtgpu_hit **d_back);
 int sdtgpu_lookup_unstage (sdtgpu_t *h, sdtgpu_hit *d_out);
 
+/* ---- edges between junction k-mers (the graph kmer2edges builds, node2edge.c:46, without its pruning), one GPU.
+ * A node with canonical key k = b0..b(K-1) is read as (v,+) = k and (v,-) = rc(k).  The out-links of (v,+) are the
+ * right counters R[x] > 0 of the finalized table (after -d), successor b1..b(K-1) x canonicalised; those of (v,-) the
+ * left counters L[x] > 0, successor rc(x b0..b(K-2)), base appended comp(x) = x ^ 2.  A node is linear when exactly one
+ * left and one right counter are non-zero (the linear bit of rword), a vertex when it is neither linear nor deleted.
+ *   edge    a walk x0 -> x1 -> ... -> xm (m >= 1) over out-links, x0 and xm vertices, x1 .. x(m-1) linear: one per
+ *           (oriented vertex, out-link).  Its sequence has m + K bases.  Of a walk and its reverse complement (the walk
+ *           from xm in the other orientation) the one kept is the one whose first (K+1)-mer is <= the reverse
+ *           complement of its last (K+1)-mer, as (2K+2)-bit integers; equality means the walk is its own reverse
+ *           complement (SDTGPU_EDGE_PALINDROME: it runs through a hairpin and holds its interior nodes twice).
+ *   cycle   the linear nodes no edge visits form closed walks (poly-A, a circular transcript, a chain closed by two
+ *           hairpins, which is SDTGPU_EDGE_PALINDROME too and holds its nodes twice).  One record each, flag
+ *           SDTGPU_EDGE_CYCLE: m k-mers read circularly from a start and strand of the library's choice, m + K - 1 bases.
+ *   count_sum  the sum of count over x1 .. x(m-1); for a cycle over all its m k-mers.
+ *   link       x0's counter for the first step.
+ * The records are numbered by start (table position, orientation + before -, counter index), keeping the kept walks
+ * only; the cycles follow the edges.  Two builds of one table give byte-identical buffers.  The sequences are in the
+ * reads' tight-string convention (4 bases per byte, first base in bits 7..6); each starts at a multiple of 32 bases,
+ * its last word zero-padded.
+ *
+ * sdtgpu_edges_build: out = { edges (cycles included), palindromic edges (cycles included), cycles, bases, vertices,
+ * linear nodes on edges, linear nodes on cycles, dangling links } where a palindrome counts its nodes once, and a dangling
+ * link is a non-zero counter whose neighbour is not in the table or a linear node's neighbour without the link back
+ * (there are none in a table built by this library: both ends of a (K+1)-mer count the same instances).  ms: device
+ * time of the build (CUDA events).  Valid after sdtgpu_finalize (SDTGPU_ESTATE before it and after sdtgpu_reset); a
+ * handle that holds one rank's share of a sharded table (sdtgpu_lookup_route case other than SDTGPU_ROUTE_ONE) is
+ * SDTGPU_EINVAL; NULL arguments are SDTGPU_EINVAL before any CUDA call; SDTGPU_ENOMEM if the buffers do not fit (about
+ * 41 bytes per table slot, 8 per walk start, plus the output).  Builds the lookup index if it is missing; synchronises
+ * the handle's stream.
+ * sdtgpu_edges_buffers: the device addresses of the last build's records (out[0] of them) and sequences, SDTGPU_ESTATE
+ * before a build.  The buffers belong to the handle, grow only and may move at the next build; sdtgpu_reset and
+ * sdtgpu_destroy free them. */
+typedef struct sdtgpu_edge {
+	uint64_t seq;		/* first base in the sequence buffer, counted in bases; a multiple of 32 */
+	uint32_t length;	/* m: an edge has m+1 k-mers and m+K bases; a cycle has m k-mers and m+K-1 bases */
+	uint32_t flags;		/* SDTGPU_EDGE_PALINDROME, SDTGPU_EDGE_CYCLE */
+	uint64_t count_sum;
+	uint32_t link;
+	uint32_t unused;	/* 0 */
+} sdtgpu_edge;		/* 32 bytes */
+#define SDTGPU_EDGE_PALINDROME 1u
+#define SDTGPU_EDGE_CYCLE      2u
+int sdtgpu_edges_build (sdtgpu_t *h, uint64_t out[8], double *ms);
+int sdtgpu_edges_buffers (sdtgpu_t *h, const sdtgpu_edge **d_edges, const uint8_t **d_seq);
+
 /* pinned host memory for the caller's batch buffers (the reference's seqBuffer/lenBuffer role,
  * prlHashReads.c:387-395); plain pageable memory also works with push_reads, only slower */
 int sdtgpu_host_alloc (void **out, size_t bytes);

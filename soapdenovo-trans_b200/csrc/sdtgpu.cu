@@ -8,6 +8,7 @@
 #include "sdt_build.cuh"
 #include "sdt_lookup.cuh"
 #include "sdt_route.cuh"
+#include "sdt_edges.cuh"
 
 #include <algorithm>
 #include <cstdio>
@@ -40,6 +41,8 @@ struct LogSeg
 	ReadBatch rb;	// pointers are resolved when the segment is used (the arenas may move)
 	u64 upper;	// windows of the batch at most
 };
+
+enum { ED_STEP, ED_MARK, ED_A, ED_B, ED_OFF_A, ED_OFF_B, ED_STARTS, ED_SEG, ED_CTR, ED_EDGES, ED_SEQ, ED_N };	// sdtgpu::ed
 
 static constexpr int N_CAT = 8;	// timing classes: 0 insert, 1 count / emit, 2 scatter, 3 dedupe, 4 build, 5 scan, 6 build retries, 7 lookups
 
@@ -102,6 +105,10 @@ struct sdtgpu
 	bool rt_staged = false;	// a stage awaits its unstage
 	u64 rt_n = 0, rt_out = 0;	// queries staged, entries of the caller's output
 	u32 owner_rank = 0, owner_ranks = 1;	// sdtgpu_set_owner
+	// edges (sdt_edges.cuh): the buffers grow only and are kept across builds; reset and destroy free them
+	void *ed[ED_N] = {};
+	size_t ed_cap[ED_N] = {};	// bytes
+	bool ed_built = false;
 	// sliced build (SDTGPU_F_SLICED): reads of the open epoch are kept in a log and turned into super-k-mer
 	// records in the chains of their slices as they arrive; sliced_flush merges copies and builds the slices
 	bool sliced = false, table_built = false, epoch_open = false, emitted = false, ord_bound_set = false, chains_dropped = false;
@@ -1505,6 +1512,17 @@ void free_route (sdtgpu *h)
 	h->rt_staged = false;
 }
 
+void free_edges (sdtgpu *h)
+{
+	for (int i = 0; i < ED_N; i++)
+	{
+		cudaFree (h->ed[i]);
+		h->ed[i] = nullptr;
+		h->ed_cap[i] = 0;
+	}
+	h->ed_built = false;
+}
+
 // a finalized table, at most ROUTE_MAX_WORLD ranks, the small count buffers, and the index: a rank that stages
 // also answers, and building the index here lets a routed lookup fail before any query travels
 int route_prologue (sdtgpu *h)
@@ -1589,6 +1607,158 @@ template <int W, bool NMODE, bool SCATTER> int launch_route_reads_t (sdtgpu *h, 
 template <int W, bool NMODE> int launch_route_reads_w (sdtgpu *h, const ReadBatch &rb, const Route &rt, bool scatter, const Stage &st)
 {
 	return scatter ? launch_route_reads_t<W, NMODE, true> (h, rb, rt, st) : launch_route_reads_t<W, NMODE, false> (h, rb, rt, st);
+}
+
+// ---- edges (sdt_edges.cuh)
+static_assert (sizeof (EdgeRec) == sizeof (sdtgpu_edge) && sizeof (EdgeRec) == 32 && SDTGPU_EDGE_PALINDROME == EDGE_PALINDROME
+	       && SDTGPU_EDGE_CYCLE == EDGE_CYCLE, "sdtgpu_edge");
+
+int edge_grow (sdtgpu *h, int i, size_t need, size_t keep = 0)
+{
+	return grow_device (h, &h->ed[i], &h->ed_cap[i], keep, std::max<size_t> (need, 64), "edge graph");
+}
+
+// CUDA events around the groups of launches between two host reads of a size: the device time of a build
+struct EdgeSpans
+{
+	sdtgpu *h;
+	std::vector<cudaEvent_t> ev;
+	explicit EdgeSpans (sdtgpu *h_) : h (h_) { }
+	void mark () { ev.push_back (get_event (h)); cudaEventRecord (ev.back (), h->stream); }
+	double ms () const
+	{
+		double t = 0;
+		for (size_t i = 0; i + 1 < ev.size (); i += 2)
+		{
+			float f = 0;
+			cudaEventElapsedTime (&f, ev[i], ev[i + 1]);
+			t += f;
+		}
+		return t;
+	}
+	~EdgeSpans () { for (auto e : ev) h->ev_pool.push_back (e); }
+};
+
+template <int W> int edges_build_t (sdtgpu *h, uint64_t out[8], double *ms)
+{
+	typedef typename SlotOf<W>::type S;
+	const S *tab = static_cast<const S *> (h->table);
+	const u64 slots = iter_slots (h);
+	int rc = read_counters (h);
+	if (rc)
+		return rc;
+	EdgeGraph g = {};
+	g.index = h->index;
+	g.idx_cap = h->idx_cap;
+	g.slots = slots;
+	g.K = h->K;
+	g.deLowKmer = h->deLowKmer;
+	g.max_m = 2 * h->h_ctr->n_linear + 2;	// a palindromic edge holds its nodes twice
+	auto bind = [&] () {
+		g.step = static_cast<Step *> (h->ed[ED_STEP]);
+		g.mark = static_cast<unsigned char *> (h->ed[ED_MARK]);
+		g.a = static_cast<u32 *> (h->ed[ED_A]);
+		g.b = static_cast<u32 *> (h->ed[ED_B]);
+		g.off_a = static_cast<const u64 *> (h->ed[ED_OFF_A]);
+		g.off_b = static_cast<const u64 *> (h->ed[ED_OFF_B]);
+		g.starts = static_cast<u64 *> (h->ed[ED_STARTS]);
+		g.edges = static_cast<EdgeRec *> (h->ed[ED_EDGES]);
+		g.seq = static_cast<u64 *> (h->ed[ED_SEQ]);
+		g.ctr = static_cast<u64 *> (h->ed[ED_CTR]);
+	};
+	auto grid = [&] (u64 n) { return (unsigned) std::min<u64> ((n + BLOCK - 1) / BLOCK, (u64) h->sm_count * 16); };
+	auto nseg = [] (u64 n) { return (u32) std::max<u64> (1, (n + SCAN_SEG - 1) / SCAN_SEG); };
+	auto scan = [&] (const u32 *in, u64 n, int off) {
+		u64 *seg = static_cast<u64 *> (h->ed[ED_SEG]), *o = static_cast<u64 *> (h->ed[off]);
+		slice_scan_sums_kernel<<<nseg (n), SCAN_NT, 0, h->stream>>> (in, (u32) n, seg);
+		slice_scan_kernel<<<nseg (n), SCAN_NT, 0, h->stream>>> (in, (u32) n, seg, o, nullptr);
+	};
+	auto total = [&] (int off, u64 n, u64 &v) -> int {
+		CK (h, cudaGetLastError ());
+		CK (h, cudaMemcpyAsync (&v, static_cast<u64 *> (h->ed[off]) + n, sizeof v, cudaMemcpyDeviceToHost, h->stream));
+		CK (h, cudaStreamSynchronize (h->stream));
+		return SDTGPU_OK;
+	};
+	h->ed_built = false;
+	if ((rc = edge_grow (h, ED_STEP, slots * sizeof (Step))) || (rc = edge_grow (h, ED_MARK, slots))
+	    || (rc = edge_grow (h, ED_A, slots * 4)) || (rc = edge_grow (h, ED_OFF_A, (slots + 1) * 8))
+	    || (rc = edge_grow (h, ED_SEG, nseg (slots) * 8)) || (rc = edge_grow (h, ED_CTR, 8 * sizeof (u64))))
+		return rc;
+	bind ();
+	EdgeSpans sp (h);
+	// 1. steps of the linear nodes, walk starts of the vertices
+	sp.mark ();
+	CK (h, cudaMemsetAsync (g.ctr, 0, 8 * sizeof (u64), h->stream));
+	if (slots)
+		edge_links_kernel<W><<<grid (slots), BLOCK, 0, h->stream>>> (tab, g);
+	scan (g.a, slots, ED_OFF_A);
+	sp.mark ();
+	u64 n_starts = 0;
+	if ((rc = total (ED_OFF_A, slots, n_starts)))
+		return rc;
+	if (n_starts >= NO_POS)
+		return fail (h, SDTGPU_ERANGE, "edges: 2^32 - 1 walk starts or more");
+	if ((rc = edge_grow (h, ED_STARTS, n_starts * 8)))
+		return rc;
+	bind ();
+	sp.mark ();
+	if (n_starts)
+		edge_starts_kernel<W><<<grid (slots), BLOCK, 0, h->stream>>> (tab, g);
+	sp.mark ();
+	CK (h, cudaGetLastError ());
+	// 2. every walk to its end: which strand is kept, and its length
+	const u64 n2 = std::max (slots, n_starts);
+	if ((rc = edge_grow (h, ED_A, n2 * 4)) || (rc = edge_grow (h, ED_B, n2 * 4)) || (rc = edge_grow (h, ED_OFF_A, (n2 + 1) * 8))
+	    || (rc = edge_grow (h, ED_OFF_B, (n2 + 1) * 8)) || (rc = edge_grow (h, ED_SEG, nseg (n2) * 8)))
+		return rc;
+	bind ();
+	g.n_starts = n_starts;
+	sp.mark ();
+	if (n_starts)
+		edge_walk_kernel<W, 0><<<grid (n_starts), BLOCK, 0, h->stream>>> (tab, g);
+	scan (g.a, n_starts, ED_OFF_A);
+	scan (g.b, n_starts, ED_OFF_B);
+	CK (h, cudaMemsetAsync (g.mark, 0, std::max<u64> (slots, 1), h->stream));
+	sp.mark ();
+	u64 n_edges = 0, n_words = 0;
+	if ((rc = total (ED_OFF_A, n_starts, n_edges)) || (rc = total (ED_OFF_B, n_starts, n_words)))
+		return rc;
+	if ((rc = edge_grow (h, ED_EDGES, n_edges * sizeof (EdgeRec))) || (rc = edge_grow (h, ED_SEQ, n_words * 8)))
+		return rc;
+	bind ();
+	// 3. the kept walks write their edges and mark their nodes; the linear nodes left elect one leader per cycle
+	sp.mark ();
+	if (n_starts)
+		edge_walk_kernel<W, 1><<<grid (n_starts), BLOCK, 0, h->stream>>> (tab, g);
+	if (slots)
+		edge_cycle_kernel<W, 0><<<grid (slots), BLOCK, 0, h->stream>>> (tab, g);
+	scan (g.a, slots, ED_OFF_A);
+	scan (g.b, slots, ED_OFF_B);
+	sp.mark ();
+	u64 n_cycles = 0, n_cwords = 0;
+	if ((rc = total (ED_OFF_A, slots, n_cycles)) || (rc = total (ED_OFF_B, slots, n_cwords)))
+		return rc;
+	if ((rc = edge_grow (h, ED_EDGES, (n_edges + n_cycles) * sizeof (EdgeRec), n_edges * sizeof (EdgeRec)))
+	    || (rc = edge_grow (h, ED_SEQ, (n_words + n_cwords) * 8, n_words * 8)))
+		return rc;
+	bind ();
+	g.edge0 = n_edges;
+	g.unit0 = n_words;
+	// 4. the leaders write their cycles after the edges
+	sp.mark ();
+	if (slots)
+		edge_cycle_kernel<W, 1><<<grid (slots), BLOCK, 0, h->stream>>> (tab, g);
+	sp.mark ();
+	CK (h, cudaGetLastError ());
+	u64 c[8];
+	CK (h, cudaMemcpyAsync (c, g.ctr, sizeof c, cudaMemcpyDeviceToHost, h->stream));
+	CK (h, cudaStreamSynchronize (h->stream));
+	out[0] = n_edges + n_cycles;
+	for (int i = 1; i < 8; i++)
+		out[i] = c[i];
+	*ms = sp.ms ();
+	h->ed_built = true;
+	return SDTGPU_OK;
 }
 
 }	// namespace
@@ -1719,6 +1889,7 @@ void sdtgpu_destroy (sdtgpu_t *h)
 	cudaFree (h->table);
 	cudaFree (h->index);
 	free_route (h);
+	free_edges (h);
 	cudaFree (h->rt_cur);
 	if (h->rt_hcur) cudaFreeHost (h->rt_hcur);
 	cudaFree (h->d_ctr);
@@ -1736,11 +1907,12 @@ int sdtgpu_reset (sdtgpu_t *h)
 		return SDTGPU_EINVAL;
 	CK (h, cudaSetDevice (h->device));
 	Trace tr (h);
-	if (h->index || h->rt_q || h->rt_aq || h->rt_back)
+	if (h->index || h->rt_q || h->rt_aq || h->rt_back || h->ed[ED_STEP])
 	{
 		CK (h, cudaStreamSynchronize (h->stream));	// (a lookup may still be reading them)
 		free_index (h);
 		free_route (h);
+		free_edges (h);
 	}
 	h->rt_staged = false;
 	CK (h, cudaMemsetAsync (h->d_ctr, 0, sizeof (Counters), h->stream));
@@ -2542,6 +2714,40 @@ int sdtgpu_lookup_unstage (sdtgpu_t *h, sdtgpu_hit *d_out)
 		route_unstage_kernel<<<grid, BLOCK, 0, h->stream>>> (h->rt_back, h->rt_tag, h->rt_n, reinterpret_cast<Hit *> (d_out));
 	}
 	CK (h, cudaGetLastError ());
+	return SDTGPU_OK;
+}
+
+int sdtgpu_edges_build (sdtgpu_t *h, uint64_t out[8], double *ms)
+{
+	if (!h)
+		return SDTGPU_EINVAL;
+	if (!out || !ms)
+		return fail (h, SDTGPU_EINVAL, "sdtgpu_edges_build: NULL output");
+	if (make_route (h).kind != ROUTE_ONE)
+		return fail (h, SDTGPU_EINVAL, "sdtgpu_edges_build: the handle holds one rank's share of a sharded table");
+	int rc = lookup_prologue (h, nullptr);
+	if (rc)
+		return rc;
+	if ((rc = ensure_index (h)))
+		return rc;
+	switch (h->W)
+	{
+	case 1: return edges_build_t<1> (h, out, ms);
+	case 2: return edges_build_t<2> (h, out, ms);
+	default: return edges_build_t<4> (h, out, ms);
+	}
+}
+
+int sdtgpu_edges_buffers (sdtgpu_t *h, const sdtgpu_edge **d_edges, const uint8_t **d_seq)
+{
+	if (!h)
+		return SDTGPU_EINVAL;
+	if (!d_edges || !d_seq)
+		return fail (h, SDTGPU_EINVAL, "sdtgpu_edges_buffers: NULL output");
+	if (!h->ed_built)
+		return fail (h, SDTGPU_ESTATE, "sdtgpu_edges_buffers before sdtgpu_edges_build");
+	*d_edges = static_cast<const sdtgpu_edge *> (h->ed[ED_EDGES]);
+	*d_seq = static_cast<const uint8_t *> (h->ed[ED_SEQ]);
 	return SDTGPU_OK;
 }
 

@@ -22,6 +22,12 @@ assert NODE_DTYPE.itemsize == 56
 HIT_DTYPE = np.dtype([("count", "<u4"), ("l_links", "<u4"), ("rword", "<u4"), ("status", "<u4")])
 assert HIT_DTYPE.itemsize == 16
 HIT_WINDOW, HIT_FOUND, HIT_RC = 1, 2, 4
+# sdtgpu_edge: one edge or cycle of PregraphGPU.edges() (include/sdtgpu.h); seq counts bases into the sequence buffer
+EDGE_DTYPE = np.dtype([("seq", "<u8"), ("length", "<u4"), ("flags", "<u4"), ("count_sum", "<u8"), ("link", "<u4"),
+                       ("unused", "<u4")])
+assert EDGE_DTYPE.itemsize == 32
+EDGE_PALINDROME, EDGE_CYCLE = 1, 2
+EDGE_COUNTS = ("edges", "palindromes", "cycles", "bases", "vertices", "linear_on_edges", "linear_on_cycles", "dangling")
 
 F_NKMER = 1
 F_SLICED = 4
@@ -50,7 +56,7 @@ class KmerSet(C.Structure):
 def build_library(force: bool = False) -> str:
     """Compiles csrc/ + host/ for sm_100a into libsdtgpu.so (in-tree, so it travels to the GPU box)."""
     srcs = [os.path.join(PKG_DIR, p) for p in ("csrc/sdtgpu.cu", "csrc/sdt_synth.cu", "csrc/sdt_device.cuh",
-                                               "csrc/sdt_kernels.cuh", "csrc/sdt_sliced.cuh", "csrc/sdt_skm.cuh", "csrc/sdt_build.cuh", "csrc/sdt_lookup.cuh", "csrc/sdt_route.cuh", "csrc/sdt_nccl.cu", "csrc/sdt_parse.cu", "host/kmerset_builder.cpp", "host/sdt_readpack.c", "../include/sdtpack.h",
+                                               "csrc/sdt_kernels.cuh", "csrc/sdt_sliced.cuh", "csrc/sdt_skm.cuh", "csrc/sdt_build.cuh", "csrc/sdt_lookup.cuh", "csrc/sdt_route.cuh", "csrc/sdt_edges.cuh", "csrc/sdt_nccl.cu", "csrc/sdt_parse.cu", "host/kmerset_builder.cpp", "host/sdt_readpack.c", "../include/sdtpack.h",
                                                "../include/sdtgpu.h")]
     stale = (not os.path.exists(LIB_PATH)) or any(os.path.getmtime(s) > os.path.getmtime(LIB_PATH) for s in srcs)
     if force or stale:
@@ -122,6 +128,8 @@ def library() -> C.CDLL:
     L.sdtgpu_lookup_unstage.argtypes = [vp, vp]
     L.sdtgpu_lookup_kmers_exchange.argtypes = [vp, vp, vp, u64, vp, C.POINTER(C.c_double)]
     L.sdtgpu_lookup_reads_exchange.argtypes = [vp, vp, vp, vp, vp, u64, u32, u32, vp, C.POINTER(C.c_double)]
+    L.sdtgpu_edges_build.argtypes = [vp, vp, C.POINTER(C.c_double)]
+    L.sdtgpu_edges_buffers.argtypes = [vp, C.POINTER(vp), C.POINTER(vp)]
     L.sdtgpu_last_ordinals.argtypes = [vp, i32, vp]
     L.sdtgpu_kernel_times.argtypes = [vp, i32, C.POINTER(C.c_double), C.POINTER(u64)]
     L.sdtgpu_phase_times.argtypes = [vp, i32, C.POINTER(C.c_double), C.POINTER(u64)]
@@ -179,6 +187,27 @@ def hits_numpy(hits) -> np.ndarray:
     """Hits as returned by PregraphGPU.lookup_* on the device (int32 [..., 4]) -> a HIT_DTYPE array of shape [...]."""
     a = np.ascontiguousarray(hits.cpu().numpy() if hasattr(hits, "cpu") else hits).view(np.uint32)
     return a.view(HIT_DTYPE)[..., 0]
+
+
+def edge_codes(edges: np.ndarray, seq: np.ndarray, i: int, K: int) -> np.ndarray:
+    """Base codes (uint8, A=0 C=1 T=2 G=3) of edge i of PregraphGPU.edges(): m + K bases, m + K - 1 for a cycle."""
+    e = edges[i]
+    n = int(e["length"]) + K - (1 if int(e["flags"]) & EDGE_CYCLE else 0)
+    a = int(e["seq"]) // 4
+    raw = seq[a: a + (n + 3) // 4]
+    return (raw[:, None] >> np.array([6, 4, 2, 0], dtype=np.uint8) & 3).reshape(-1)[:n]
+
+
+class _DeviceBytes:
+    """A device buffer owned by the library, seen by torch through __cuda_array_interface__ (no copy)."""
+
+    def __init__(self, ptr: int, nbytes: int):
+        self.__cuda_array_interface__ = {"shape": (nbytes,), "typestr": "|u1", "data": (ptr, False), "version": 2}
+
+
+def _device_bytes(ptr: int, nbytes: int, dev):
+    import torch
+    return torch.as_tensor(_DeviceBytes(ptr, nbytes), device=dev)
 
 
 def node_bytes(key_words: int) -> int:
@@ -393,6 +422,33 @@ class PregraphGPU:
                                                    stride_bytes, _ptr(out)))
         self.sync()
         return out
+
+    # ---- edges between junction k-mers (include/sdtgpu.h sdtgpu_edges_*)
+    def edges_build(self) -> dict:
+        """Compacts the finalized table into edges and cycles on the device -> the eight counts of sdtgpu_edges_build
+        (EDGE_COUNTS) and ms, the device time of the build."""
+        out, ms = (C.c_uint64 * 8)(), C.c_double()
+        self._ck(self.L.sdtgpu_edges_build(self.h, out, C.byref(ms)))
+        self._n_edges = int(out[0])
+        res = {k: int(v) for k, v in zip(EDGE_COUNTS, out)}
+        res["ms"] = float(ms.value)
+        return res
+
+    def edges(self):
+        """The last edges_build's records and sequences, copied to the host -> (EDGE_DTYPE array, uint8 sequence
+        buffer in the tight-string convention; edge_codes() decodes one edge)."""
+        import torch
+        e, q = C.c_void_p(), C.c_void_p()
+        self._ck(self.L.sdtgpu_edges_buffers(self.h, C.byref(e), C.byref(q)))
+        n = self._n_edges
+        if n == 0:
+            return np.zeros(0, dtype=EDGE_DTYPE), np.zeros(0, dtype=np.uint8)
+        dev = self._torch_device()
+        edges = _device_bytes(int(e.value), n * EDGE_DTYPE.itemsize, dev).cpu().numpy().view(EDGE_DTYPE)
+        last = edges[-1]      # the records are in sequence order
+        bases = int(last["length"]) + self.K - (1 if int(last["flags"]) & EDGE_CYCLE else 0)
+        words = (int(last["seq"]) + bases + 31) // 32
+        return edges, _device_bytes(int(q.value), words * 8, dev).cpu().numpy()
 
     # ---- lookups routed to the rank that owns each k-mer (include/sdtgpu.h sdtgpu_lookup_stage_* ... _exchange)
     def lookup_route(self) -> dict:
