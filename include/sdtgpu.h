@@ -310,6 +310,55 @@ typedef struct sdtgpu_edge {
 int sdtgpu_edges_build (sdtgpu_t *h, uint64_t out[8], double *ms);
 int sdtgpu_edges_buffers (sdtgpu_t *h, const sdtgpu_edge **d_edges, const uint8_t **d_seq);
 
+/* ---- reads mapped onto the edges of the last sdtgpu_edges_build (the .preArc half of prlRead2edge), one GPU.
+ * The records are walks, numbered as that build numbers them (edges, then cycles).  An edge x0 -> ... -> xm has the
+ * steps s_i = x_i -> x_(i+1), i in [0, m); a cycle of m k-mers has s_i = x_i -> x_((i+1) mod m), x_0 the record's first
+ * k-mer in the record's strand.  A (K+1)-mer of a read is a step of the graph when its first k-mer is a node that is
+ * not deleted, the counter for the read's next base on the read's side (R when the window is stored forward, L when it
+ * is stored as its reverse complement: the out-links above) is non-zero after -d, and (SDTGPU_F_NKMER) neither the
+ * window nor the next base holds an N.  Every step of the graph is some s_i of exactly one record (strand 0) or
+ * rc (s_i) (strand 1), reported as (record, i, strand); in a record flagged SDTGPU_EDGE_PALINDROME rc (s_i) is itself
+ * some s_k (k = m - 1 - i on an edge), and such a step is always reported as strand 0 with that k.
+ * An arc is a crossing of a vertex v by a read: windows j and j+1 with window j+1 = v and steps j and j+1 both steps of
+ * the graph.  It is read in v's + orientation, with the link bases (left, right) of the window as it is stored:
+ * to = the record (and strand) of the walk start (v, +, right), from = the record of the walk start (v, -, left) with
+ * its strand reversed; a palindromic record is strand 0 on both sides.  Each crossing counts once.  Cycles have no
+ * vertices, so no arcs.  This is this library's definition: the reference's .preArc is keyed by its own edge ids,
+ * which this library does not produce, so the two are not byte-compatible.
+ *
+ * sdtgpu_edges_map_reads: the read arguments as sdtgpu_lookup_reads_device.  The step of the (K+1)-mer that starts at
+ * window j of read r goes to d_out[r * maxwin + j] (8-byte aligned device memory, or NULL with count_arcs); the last
+ * window of a read, windows a read does not have and (K+1)-mers that are not steps of the graph are "none" (both fields
+ * all ones).  count_arcs != 0 adds the batch's crossings to the handle's arc counters: a library is counted by mapping
+ * each batch once.  Only enqueues work on sdtgpu_stream(h), timed in class 7 of sdtgpu_phase_times, except that the
+ * first call after a build stamps the graph (8 bytes per table slot, 20 per walk start, 4 per cycle; arc counters
+ * zeroed) and synchronises once.  n_reads = 0 only stamps.
+ * sdtgpu_arcs_build: the non-zero counters as sdtgpu_arc records in (vertex position, left base, right base) order, so
+ * two builds give byte-identical buffers; out = { arcs, sum of their counts }, ms: device time (CUDA events).
+ * Synchronises the handle's stream.
+ * sdtgpu_arcs_buffers: the device address of the last arcs_build's records (out[0] of them); SDTGPU_ESTATE before one.
+ * sdtgpu_arcs_clear: zeroes the arc counters.
+ * All four need an edge build of the current table: SDTGPU_ESTATE before sdtgpu_edges_build and after sdtgpu_reset (a
+ * sharded handle never gets there: the edge build refuses it).  A new edge build drops the stamps, the counters and
+ * the arcs.  NULL buffers are SDTGPU_EINVAL before any CUDA call; SDTGPU_ERANGE if there are 2^31 records or more or
+ * a record's length reaches 2^31.  The buffers belong to the handle, grow only and may move at the next call;
+ * sdtgpu_reset and sdtgpu_destroy free them. */
+typedef struct sdtgpu_step {
+	uint32_t record;	/* none: all ones */
+	uint32_t pos;		/* i << 1 | strand; none: all ones */
+} sdtgpu_step;			/* 8 bytes */
+typedef struct sdtgpu_arc {
+	uint32_t from, to;	/* record << 1 | strand */
+	uint32_t count;		/* crossings */
+	uint32_t unused;	/* 0 */
+} sdtgpu_arc;			/* 16 bytes */
+int sdtgpu_edges_map_reads (sdtgpu_t *h, const uint8_t *d_packed, const uint32_t *d_lens, const uint8_t *d_nmask,
+			    uint64_t n_reads, uint32_t uniform_len, uint32_t stride_bytes,
+			    sdtgpu_step *d_out /* n_reads x (max_read_len - K + 1), or NULL */, int count_arcs);
+int sdtgpu_arcs_build (sdtgpu_t *h, uint64_t out[2] /* arcs, crossings */, double *ms);
+int sdtgpu_arcs_buffers (sdtgpu_t *h, const sdtgpu_arc **d_arcs);
+int sdtgpu_arcs_clear (sdtgpu_t *h);
+
 /* pinned host memory for the caller's batch buffers (the reference's seqBuffer/lenBuffer role,
  * prlHashReads.c:387-395); plain pageable memory also works with push_reads, only slower */
 int sdtgpu_host_alloc (void **out, size_t bytes);

@@ -9,6 +9,7 @@
 #include "sdt_lookup.cuh"
 #include "sdt_route.cuh"
 #include "sdt_edges.cuh"
+#include "sdt_paths.cuh"
 
 #include <algorithm>
 #include <cstdio>
@@ -43,6 +44,7 @@ struct LogSeg
 };
 
 enum { ED_STEP, ED_MARK, ED_A, ED_B, ED_OFF_A, ED_OFF_B, ED_STARTS, ED_SEG, ED_CTR, ED_EDGES, ED_SEQ, ED_N };	// sdtgpu::ed
+enum { PA_STAMP, PA_SREC, PA_AUX, PA_CTR, PA_SMALL, PA_ARCS, PA_N };	// sdtgpu::pa
 
 static constexpr int N_CAT = 8;	// timing classes: 0 insert, 1 count / emit, 2 scatter, 3 dedupe, 4 build, 5 scan, 6 build retries, 7 lookups
 
@@ -109,6 +111,12 @@ struct sdtgpu
 	void *ed[ED_N] = {};
 	size_t ed_cap[ED_N] = {};	// bytes
 	bool ed_built = false;
+	u64 ed_n_starts = 0, ed_n_edges = 0, ed_n_records = 0;	// of the last build
+	// reads mapped onto the edges (sdt_paths.cuh): stamps made by the first map after a build, arc counters, arcs
+	void *pa[PA_N] = {};
+	size_t pa_cap[PA_N] = {};	// bytes
+	bool pa_ready = false, pa_arcs = false;	// stamps of the last build (counters zeroed with them); arcs built since
+	u64 pa_n_arcs = 0;
 	// sliced build (SDTGPU_F_SLICED): reads of the open epoch are kept in a log and turned into super-k-mer
 	// records in the chains of their slices as they arrive; sliced_flush merges copies and builds the slices
 	bool sliced = false, table_built = false, epoch_open = false, emitted = false, ord_bound_set = false, chains_dropped = false;
@@ -1521,6 +1529,13 @@ void free_edges (sdtgpu *h)
 		h->ed_cap[i] = 0;
 	}
 	h->ed_built = false;
+	for (int i = 0; i < PA_N; i++)
+	{
+		cudaFree (h->pa[i]);
+		h->pa[i] = nullptr;
+		h->pa_cap[i] = 0;
+	}
+	h->pa_ready = h->pa_arcs = false;
 }
 
 // a finalized table, at most ROUTE_MAX_WORLD ranks, the small count buffers, and the index: a rank that stages
@@ -1680,6 +1695,7 @@ template <int W> int edges_build_t (sdtgpu *h, uint64_t out[8], double *ms)
 		return SDTGPU_OK;
 	};
 	h->ed_built = false;
+	h->pa_ready = h->pa_arcs = false;	// the stamps and arc counters of the last build go with it
 	if ((rc = edge_grow (h, ED_STEP, slots * sizeof (Step))) || (rc = edge_grow (h, ED_MARK, slots))
 	    || (rc = edge_grow (h, ED_A, slots * 4)) || (rc = edge_grow (h, ED_OFF_A, (slots + 1) * 8))
 	    || (rc = edge_grow (h, ED_SEG, nseg (slots) * 8)) || (rc = edge_grow (h, ED_CTR, 8 * sizeof (u64))))
@@ -1757,7 +1773,160 @@ template <int W> int edges_build_t (sdtgpu *h, uint64_t out[8], double *ms)
 	for (int i = 1; i < 8; i++)
 		out[i] = c[i];
 	*ms = sp.ms ();
+	h->ed_n_starts = n_starts;
+	h->ed_n_edges = n_edges;
+	h->ed_n_records = n_edges + n_cycles;
 	h->ed_built = true;
+	return SDTGPU_OK;
+}
+
+// ---- reads mapped onto the edges (sdt_paths.cuh)
+static_assert (sizeof (ArcRec) == sizeof (sdtgpu_arc) && sizeof (sdtgpu_step) == 8, "sdtgpu_arc, sdtgpu_step");
+
+int path_grow (sdtgpu *h, int i, size_t need)
+{
+	return grow_device (h, &h->pa[i], &h->pa_cap[i], 0, std::max<size_t> (need, 64), "read paths");
+}
+
+PathMap make_path_map (sdtgpu *h)
+{
+	PathMap g = {};
+	g.index = h->index;
+	g.idx_cap = h->idx_cap;
+	g.step = static_cast<const Step *> (h->ed[ED_STEP]);
+	g.starts = static_cast<const u64 *> (h->ed[ED_STARTS]);
+	g.edges = static_cast<const EdgeRec *> (h->ed[ED_EDGES]);
+	g.seq = static_cast<const u64 *> (h->ed[ED_SEQ]);
+	g.stamp = static_cast<uint2 *> (h->pa[PA_STAMP]);
+	g.srec = static_cast<u32 *> (h->pa[PA_SREC]);
+	g.aux = static_cast<u32 *> (h->pa[PA_AUX]);
+	g.ctr = static_cast<u32 *> (h->pa[PA_CTR]);
+	g.cnt = static_cast<u32 *> (h->ed[ED_A]);	// the edge build's scratch: n_starts entries at least
+	g.off = static_cast<const u64 *> (h->ed[ED_OFF_A]);
+	g.arcs = static_cast<ArcRec *> (h->pa[PA_ARCS]);
+	g.small = static_cast<u64 *> (h->pa[PA_SMALL]);
+	g.n_starts = h->ed_n_starts;
+	g.n_edges = h->ed_n_edges;
+	g.n_records = h->ed_n_records;
+	g.K = h->K;
+	return g;
+}
+
+// The stamps of the last edge build, made by the first call that needs them (like the lookup index): per slot 8
+// bytes, per walk start 4 + 16 (arc counters, zeroed), per cycle 4.  Synchronises once, to check the longest record.
+template <int W> int ensure_paths_t (sdtgpu *h)
+{
+	if (h->pa_ready)
+		return SDTGPU_OK;
+	typedef typename SlotOf<W>::type S;
+	const u64 slots = iter_slots (h);
+	if (h->ed_n_records >= (1ull << 31))
+		return fail (h, SDTGPU_ERANGE, "read paths: 2^31 records or more");
+	int rc;
+	if ((rc = path_grow (h, PA_STAMP, slots * 8)) || (rc = path_grow (h, PA_SREC, h->ed_n_starts * 4))
+	    || (rc = path_grow (h, PA_AUX, (h->ed_n_records - h->ed_n_edges) * 4)) || (rc = path_grow (h, PA_CTR, h->ed_n_starts * 16))
+	    || (rc = path_grow (h, PA_SMALL, 2 * sizeof (u64))))
+		return rc;
+	PathMap g = make_path_map (h);
+	auto grid = [&] (u64 n) { return (unsigned) std::min<u64> ((n + BLOCK - 1) / BLOCK, (u64) h->sm_count * 16); };
+	CK (h, cudaMemsetAsync (g.stamp, 0xFF, std::max<u64> (slots, 1) * 8, h->stream));
+	CK (h, cudaMemsetAsync (g.srec, 0xFF, std::max<u64> (g.n_starts, 1) * 4, h->stream));
+	CK (h, cudaMemsetAsync (g.ctr, 0, std::max<u64> (g.n_starts, 1) * 16, h->stream));
+	CK (h, cudaMemsetAsync (g.small, 0, 2 * sizeof (u64), h->stream));
+	{
+		TimedLaunch tl (h, 7);
+		if (g.n_starts)
+			path_starts_kernel<<<grid (g.n_starts), BLOCK, 0, h->stream>>> (g);
+		if (g.n_records)
+			path_records_kernel<W><<<grid (g.n_records), BLOCK, 0, h->stream>>> (static_cast<const S *> (h->table), g);
+	}
+	CK (h, cudaGetLastError ());
+	u64 longest = 0;
+	CK (h, cudaMemcpyAsync (&longest, g.small, sizeof longest, cudaMemcpyDeviceToHost, h->stream));
+	CK (h, cudaStreamSynchronize (h->stream));
+	if (longest >= (1ull << 31))
+		return fail (h, SDTGPU_ERANGE, "read paths: a record of length 2^31 or more");
+	h->pa_ready = true;
+	return SDTGPU_OK;
+}
+
+// what every call on the read paths checks first: an edge build of the current table, and its stamps
+int path_prologue (sdtgpu *h)
+{
+	CK (h, cudaSetDevice (h->device));
+	if (!h->ed_built)
+		return fail (h, SDTGPU_ESTATE, "read paths need sdtgpu_edges_build of the current table");
+	switch (h->W)
+	{
+	case 1: return ensure_paths_t<1> (h);
+	case 2: return ensure_paths_t<2> (h);
+	default: return ensure_paths_t<4> (h);
+	}
+}
+
+template <int W, bool NMODE> int launch_path_map_t (sdtgpu *h, const ReadBatch &rb, const PathMap &g)
+{
+	auto kern = path_map_kernel<W, NMODE>;
+	const size_t smem = 4 * tile_words (rb, NMODE);
+	if (smem > 48 * 1024)
+		CK (h, cudaFuncSetAttribute (kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem));
+	int occ = 0;
+	CK (h, cudaOccupancyMaxActiveBlocksPerMultiprocessor (&occ, kern, BLOCK, smem));
+	if (occ < 1)
+		return fail (h, SDTGPU_EINVAL, "read stride too large for one shared-memory tile");
+	const u64 n_tiles = (rb.n_reads + rb.tile_reads - 1) / rb.tile_reads;
+	const unsigned grid = (unsigned) std::min<u64> (n_tiles, (u64) h->sm_count * occ);
+	{
+		TimedLaunch tl (h, 7);
+		kern<<<grid, BLOCK, smem, h->stream>>> (static_cast<const typename SlotOf<W>::type *> (h->table), rb, g);
+	}
+	CK (h, cudaGetLastError ());
+	return SDTGPU_OK;
+}
+
+template <int W> int arcs_build_t (sdtgpu *h, uint64_t out[2], double *ms)
+{
+	typedef typename SlotOf<W>::type S;
+	const S *tab = static_cast<const S *> (h->table);
+	PathMap g = make_path_map (h);
+	const u64 n = g.n_starts;
+	auto grid = [&] (u64 k) { return (unsigned) std::min<u64> ((k + BLOCK - 1) / BLOCK, (u64) h->sm_count * 16); };
+	const u32 nseg = (u32) std::max<u64> (1, (n + SCAN_SEG - 1) / SCAN_SEG);
+	EdgeSpans sp (h);
+	sp.mark ();
+	CK (h, cudaMemsetAsync (g.small + 1, 0, sizeof (u64), h->stream));
+	if (n)
+	{
+		path_arcs_kernel<W, 0><<<grid (n), BLOCK, 0, h->stream>>> (tab, g);
+		slice_scan_sums_kernel<<<nseg, SCAN_NT, 0, h->stream>>> (g.cnt, (u32) n, static_cast<u64 *> (h->ed[ED_SEG]));
+		slice_scan_kernel<<<nseg, SCAN_NT, 0, h->stream>>> (g.cnt, (u32) n, static_cast<const u64 *> (h->ed[ED_SEG]), static_cast<u64 *> (h->ed[ED_OFF_A]), nullptr);
+	}
+	sp.mark ();
+	CK (h, cudaGetLastError ());
+	u64 n_arcs = 0;
+	if (n)
+	{
+		CK (h, cudaMemcpyAsync (&n_arcs, g.off + n, sizeof n_arcs, cudaMemcpyDeviceToHost, h->stream));
+		CK (h, cudaStreamSynchronize (h->stream));
+	}
+	h->pa_arcs = false;
+	int rc = path_grow (h, PA_ARCS, n_arcs * sizeof (ArcRec));
+	if (rc)
+		return rc;
+	g.arcs = static_cast<ArcRec *> (h->pa[PA_ARCS]);
+	sp.mark ();
+	if (n_arcs)
+		path_arcs_kernel<W, 1><<<grid (n), BLOCK, 0, h->stream>>> (tab, g);
+	sp.mark ();
+	CK (h, cudaGetLastError ());
+	u64 crossings = 0;
+	CK (h, cudaMemcpyAsync (&crossings, g.small + 1, sizeof crossings, cudaMemcpyDeviceToHost, h->stream));
+	CK (h, cudaStreamSynchronize (h->stream));
+	out[0] = n_arcs;
+	out[1] = crossings;
+	*ms = sp.ms ();
+	h->pa_n_arcs = n_arcs;
+	h->pa_arcs = true;
 	return SDTGPU_OK;
 }
 
@@ -2748,6 +2917,81 @@ int sdtgpu_edges_buffers (sdtgpu_t *h, const sdtgpu_edge **d_edges, const uint8_
 		return fail (h, SDTGPU_ESTATE, "sdtgpu_edges_buffers before sdtgpu_edges_build");
 	*d_edges = static_cast<const sdtgpu_edge *> (h->ed[ED_EDGES]);
 	*d_seq = static_cast<const uint8_t *> (h->ed[ED_SEQ]);
+	return SDTGPU_OK;
+}
+
+int sdtgpu_edges_map_reads (sdtgpu_t *h, const uint8_t *d_packed, const uint32_t *d_lens, const uint8_t *d_nmask,
+			    uint64_t n_reads, uint32_t uniform_len, uint32_t stride_bytes, sdtgpu_step *d_out, int count_arcs)
+{
+	if (!h)
+		return SDTGPU_EINVAL;
+	if ((n_reads && !d_packed) || (!d_out && !count_arcs))
+		return fail (h, SDTGPU_EINVAL, "sdtgpu_edges_map_reads: NULL buffer");
+	if ((uintptr_t) d_out & 7)
+		return fail (h, SDTGPU_EINVAL, "the step buffer must be 8-byte aligned");
+	int rc = path_prologue (h);
+	if (rc)
+		return rc;
+	ReadBatch rb;
+	if ((rc = make_batch (h, rb, d_packed, d_lens, d_nmask, n_reads, uniform_len, stride_bytes, 0)))
+		return rc;
+	if (n_reads == 0)
+		return SDTGPU_OK;
+	// windows a read does not have are never written by the kernel: "none" first, unless every read has them all
+	if (d_out && (d_lens || std::min (uniform_len, (u32) h->max_read_len) != (u32) h->max_read_len))
+		CK (h, cudaMemsetAsync (d_out, 0xFF, n_reads * h->maxwin * sizeof (sdtgpu_step), h->stream));
+	PathMap g = make_path_map (h);
+	g.out = reinterpret_cast<uint2 *> (d_out);
+	if (!count_arcs)
+		g.ctr = nullptr;
+	const bool nmode = (h->flags & SDTGPU_F_NKMER) && rb.nmask;
+	switch (h->W)
+	{
+	case 1: return nmode ? launch_path_map_t<1, true> (h, rb, g) : launch_path_map_t<1, false> (h, rb, g);
+	case 2: return nmode ? launch_path_map_t<2, true> (h, rb, g) : launch_path_map_t<2, false> (h, rb, g);
+	default: return nmode ? launch_path_map_t<4, true> (h, rb, g) : launch_path_map_t<4, false> (h, rb, g);
+	}
+}
+
+int sdtgpu_arcs_build (sdtgpu_t *h, uint64_t out[2], double *ms)
+{
+	if (!h)
+		return SDTGPU_EINVAL;
+	if (!out || !ms)
+		return fail (h, SDTGPU_EINVAL, "sdtgpu_arcs_build: NULL output");
+	int rc = path_prologue (h);
+	if (rc)
+		return rc;
+	switch (h->W)
+	{
+	case 1: return arcs_build_t<1> (h, out, ms);
+	case 2: return arcs_build_t<2> (h, out, ms);
+	default: return arcs_build_t<4> (h, out, ms);
+	}
+}
+
+int sdtgpu_arcs_buffers (sdtgpu_t *h, const sdtgpu_arc **d_arcs)
+{
+	if (!h)
+		return SDTGPU_EINVAL;
+	if (!d_arcs)
+		return fail (h, SDTGPU_EINVAL, "sdtgpu_arcs_buffers: NULL output");
+	if (!h->ed_built || !h->pa_arcs)
+		return fail (h, SDTGPU_ESTATE, "sdtgpu_arcs_buffers before sdtgpu_arcs_build");
+	*d_arcs = static_cast<const sdtgpu_arc *> (h->pa[PA_ARCS]);
+	return SDTGPU_OK;
+}
+
+int sdtgpu_arcs_clear (sdtgpu_t *h)
+{
+	if (!h)
+		return SDTGPU_EINVAL;
+	const bool fresh = !h->pa_ready;
+	int rc = path_prologue (h);
+	if (rc)
+		return rc;
+	if (!fresh)	// (stamps just made come with zero counters)
+		CK (h, cudaMemsetAsync (h->pa[PA_CTR], 0, std::max<u64> (h->ed_n_starts, 1) * 16, h->stream));
 	return SDTGPU_OK;
 }
 

@@ -27,6 +27,13 @@ EDGE_DTYPE = np.dtype([("seq", "<u8"), ("length", "<u4"), ("flags", "<u4"), ("co
                        ("unused", "<u4")])
 assert EDGE_DTYPE.itemsize == 32
 EDGE_PALINDROME, EDGE_CYCLE = 1, 2
+# sdtgpu_step: the step of one read window on the edges (include/sdtgpu.h); pos = index << 1 | strand, all ones = none
+STEP_DTYPE = np.dtype([("record", "<u4"), ("pos", "<u4")])
+assert STEP_DTYPE.itemsize == 8
+STEP_NONE = 0xFFFFFFFF
+# sdtgpu_arc: reads crossing a vertex from one record to the next; from / to = record << 1 | strand
+ARC_DTYPE = np.dtype([("from", "<u4"), ("to", "<u4"), ("count", "<u4"), ("unused", "<u4")])
+assert ARC_DTYPE.itemsize == 16
 EDGE_COUNTS = ("edges", "palindromes", "cycles", "bases", "vertices", "linear_on_edges", "linear_on_cycles", "dangling")
 
 F_NKMER = 1
@@ -56,7 +63,7 @@ class KmerSet(C.Structure):
 def build_library(force: bool = False) -> str:
     """Compiles csrc/ + host/ for sm_100a into libsdtgpu.so (in-tree, so it travels to the GPU box)."""
     srcs = [os.path.join(PKG_DIR, p) for p in ("csrc/sdtgpu.cu", "csrc/sdt_synth.cu", "csrc/sdt_device.cuh",
-                                               "csrc/sdt_kernels.cuh", "csrc/sdt_sliced.cuh", "csrc/sdt_skm.cuh", "csrc/sdt_build.cuh", "csrc/sdt_lookup.cuh", "csrc/sdt_route.cuh", "csrc/sdt_edges.cuh", "csrc/sdt_nccl.cu", "csrc/sdt_parse.cu", "host/kmerset_builder.cpp", "host/sdt_readpack.c", "../include/sdtpack.h",
+                                               "csrc/sdt_kernels.cuh", "csrc/sdt_sliced.cuh", "csrc/sdt_skm.cuh", "csrc/sdt_build.cuh", "csrc/sdt_lookup.cuh", "csrc/sdt_route.cuh", "csrc/sdt_edges.cuh", "csrc/sdt_paths.cuh", "csrc/sdt_nccl.cu", "csrc/sdt_parse.cu", "host/kmerset_builder.cpp", "host/sdt_readpack.c", "../include/sdtpack.h",
                                                "../include/sdtgpu.h")]
     stale = (not os.path.exists(LIB_PATH)) or any(os.path.getmtime(s) > os.path.getmtime(LIB_PATH) for s in srcs)
     if force or stale:
@@ -130,6 +137,10 @@ def library() -> C.CDLL:
     L.sdtgpu_lookup_reads_exchange.argtypes = [vp, vp, vp, vp, vp, u64, u32, u32, vp, C.POINTER(C.c_double)]
     L.sdtgpu_edges_build.argtypes = [vp, vp, C.POINTER(C.c_double)]
     L.sdtgpu_edges_buffers.argtypes = [vp, C.POINTER(vp), C.POINTER(vp)]
+    L.sdtgpu_edges_map_reads.argtypes = [vp, vp, vp, vp, u64, u32, u32, vp, i32]
+    L.sdtgpu_arcs_build.argtypes = [vp, C.POINTER(u64), C.POINTER(C.c_double)]
+    L.sdtgpu_arcs_buffers.argtypes = [vp, C.POINTER(vp)]
+    L.sdtgpu_arcs_clear.argtypes = [vp]
     L.sdtgpu_last_ordinals.argtypes = [vp, i32, vp]
     L.sdtgpu_kernel_times.argtypes = [vp, i32, C.POINTER(C.c_double), C.POINTER(u64)]
     L.sdtgpu_phase_times.argtypes = [vp, i32, C.POINTER(C.c_double), C.POINTER(u64)]
@@ -187,6 +198,17 @@ def hits_numpy(hits) -> np.ndarray:
     """Hits as returned by PregraphGPU.lookup_* on the device (int32 [..., 4]) -> a HIT_DTYPE array of shape [...]."""
     a = np.ascontiguousarray(hits.cpu().numpy() if hasattr(hits, "cpu") else hits).view(np.uint32)
     return a.view(HIT_DTYPE)[..., 0]
+
+
+def steps_numpy(steps) -> np.ndarray:
+    """Steps as returned by PregraphGPU.map_reads (int32 [..., 2]) -> int64 [..., 3] of (record, index, strand),
+    all three -1 where the window's (K+1)-mer is not a step of the graph."""
+    a = np.ascontiguousarray(steps.cpu().numpy() if hasattr(steps, "cpu") else steps).view(np.uint32)
+    rec, pos = a[..., 0].astype(np.int64), a[..., 1].astype(np.int64)
+    none = rec == STEP_NONE
+    out = np.stack([rec, pos >> 1, pos & 1], axis=-1)
+    out[none] = -1
+    return out
 
 
 def edge_codes(edges: np.ndarray, seq: np.ndarray, i: int, K: int) -> np.ndarray:
@@ -449,6 +471,47 @@ class PregraphGPU:
         bases = int(last["length"]) + self.K - (1 if int(last["flags"]) & EDGE_CYCLE else 0)
         words = (int(last["seq"]) + bases + 31) // 32
         return edges, _device_bytes(int(q.value), words * 8, dev).cpu().numpy()
+
+    # ---- reads mapped onto the edges (include/sdtgpu.h sdtgpu_edges_map_reads, sdtgpu_arcs_*)
+    def map_reads(self, packed, lens=None, nmask=None, n_reads=None, uniform_len=0, stride_bytes=None, count_arcs=True,
+                  out=None):
+        """Every read (K+1)-mer of a batch in CUDA tensors (the conventions of lookup_reads) onto the last edges_build ->
+        CUDA int32 tensor [n_reads, max_read_len - K + 1, 2] of sdtgpu_step (record, index << 1 | strand; all ones =
+        none; steps_numpy() decodes it), window j of read r at [r, j].  count_arcs adds the batch's vertex crossings
+        to the handle's arc counters.  out: a tensor of that shape to write into.  Synchronises the handle's stream."""
+        import torch
+        if n_reads is None:
+            n_reads = packed.shape[0]
+        if stride_bytes is None:
+            stride_bytes = packed.shape[1]
+        if out is None:
+            out = torch.empty((n_reads, self.max_read_len - self.K + 1, 2), dtype=torch.int32, device=self._torch_device())
+        assert out.is_contiguous() and out.numel() >= n_reads * (self.max_read_len - self.K + 1) * 2
+        torch.cuda.current_stream(self._torch_device()).synchronize()
+        self._ck(self.L.sdtgpu_edges_map_reads(self.h, _ptr(packed), _ptr(lens), _ptr(nmask), n_reads, uniform_len,
+                                               stride_bytes, _ptr(out), int(bool(count_arcs))))
+        self.sync()
+        return out
+
+    def arcs_build(self) -> dict:
+        """The non-zero arc counters as records on the device -> arcs, crossings (the sum of their counts) and ms, the
+        device time of the build."""
+        out, ms = (C.c_uint64 * 2)(), C.c_double()
+        self._ck(self.L.sdtgpu_arcs_build(self.h, out, C.byref(ms)))
+        self._n_arcs = int(out[0])
+        return dict(arcs=int(out[0]), crossings=int(out[1]), ms=float(ms.value))
+
+    def arcs(self) -> np.ndarray:
+        """The last arcs_build's records, copied to the host -> ARC_DTYPE array in (vertex position, left base, right
+        base) order."""
+        a = C.c_void_p()
+        self._ck(self.L.sdtgpu_arcs_buffers(self.h, C.byref(a)))
+        if self._n_arcs == 0:
+            return np.zeros(0, dtype=ARC_DTYPE)
+        return _device_bytes(int(a.value), self._n_arcs * ARC_DTYPE.itemsize, self._torch_device()).cpu().numpy().view(ARC_DTYPE)
+
+    def arcs_clear(self):
+        self._ck(self.L.sdtgpu_arcs_clear(self.h))
 
     # ---- lookups routed to the rank that owns each k-mer (include/sdtgpu.h sdtgpu_lookup_stage_* ... _exchange)
     def lookup_route(self) -> dict:
