@@ -359,6 +359,44 @@ int sdtgpu_arcs_build (sdtgpu_t *h, uint64_t out[2] /* arcs, crossings */, doubl
 int sdtgpu_arcs_buffers (sdtgpu_t *h, const sdtgpu_arc **d_arcs);
 int sdtgpu_arcs_clear (sdtgpu_t *h);
 
+/* ---- the finalized table pruned of minor branches and tips (removeMinorOut, removeSingleTips, removeMinorTips of
+ * the reference's call_pregraph), one GPU.  Terms of the edges above; every non-zero counter of a node has a
+ * reciprocal counter in its neighbour (the same (K+1)-mer seen from the other end).
+ *   remove  a node's counters are all set to zero, and in every neighbour the reciprocal of each of them; its count is
+ *           kept.  After a prune a node with no non-zero counter is deleted, whatever -d finalize had, so every
+ *           non-zero counter still links two live nodes both ways; linear stays derived from the counters.
+ *   round   every decision reads the table as it was at the start of the round; all cuts are applied together after.
+ *           A junction may lose several branches in one round.
+ *   dead end  a live node with exactly one non-zero counter, oriented so that this counter is an out-link.  A tip
+ *           walks from it, x0 = the dead end, x1, ... to the first node xm that is not linear (m >= 1); when m <= 2K
+ *           the tip is x0 .. x(m-1).  If xm is a dead end too (a hairpin comes back to x0 itself) the chain x0 .. xm
+ *           is isolated and is removed whole by either tip phase.
+ * Three phases, in this order:
+ *   1. minor branches (minor_pct > 0; the reference's -i, default 5), one round: for every side with two or more
+ *      non-zero counters, each neighbour u on that side with 100 count(u) < minor_pct x the largest count of the
+ *      neighbours on that side is removed (64-bit integers: the reference's double comparison, 5 % included).
+ *   2. single tips (SDTGPU_PRUNE_SINGLE_TIPS), one round: a tip is cut when every k-mer of it has count 1.
+ *   3. minor tips (SDTGPU_PRUNE_MINOR_TIPS), rounds until one cuts nothing: a tip is cut when xm's counter toward
+ *      x(m-1) is below the largest non-zero counter on that side of xm (a branch at the maximum is never minor).
+ * The result is a function of the table alone: the same for both insert paths, any slot order and any batching.  The
+ * reference differs on purpose: its sweeps run in (set, slot) order and mutate their neighbours, so its result
+ * depends on that order and on -p; and it leaves the interior of a cut tip as a floating linear chain, where here the
+ * whole tip is removed.
+ *
+ * sdtgpu_prune: out = { nodes removed as minor branches, as single tips, as minor tips (nodes that were live at the
+ * start of the phase and deleted at its end), tips cut (an isolated chain counts once), minor-tip rounds (the last one
+ * cuts nothing), live nodes left, linear nodes left, vertices left }; ms: device time (CUDA events).  Valid after
+ * sdtgpu_finalize, at most once per table (SDTGPU_ESTATE before finalize, after sdtgpu_reset and for a second prune); a
+ * sharded handle is SDTGPU_EINVAL; NULL outputs, minor_pct outside 0..100 and unknown flags are SDTGPU_EINVAL before
+ * any CUDA call.  Builds the lookup index if it is missing (it stays valid: keys do not move) and uses 2 bytes per
+ * table slot more; synchronises the handle's stream.
+ * After a prune the edge, read-path and arc calls are SDTGPU_ESTATE until the next sdtgpu_edges_build, which builds
+ * the pruned graph.  Lookups, export, sdtgpu_table_checksum and the edge build see the pruned table (rword's deleted bit
+ * as above); sdtgpu_get_stats, kmerFreq and sdtgpu_lookup_route's -d stay those of finalize.  sdtgpu_reset clears it. */
+#define SDTGPU_PRUNE_SINGLE_TIPS 1u
+#define SDTGPU_PRUNE_MINOR_TIPS  2u
+int sdtgpu_prune (sdtgpu_t *h, int minor_pct, unsigned flags, uint64_t out[8], double *ms);
+
 /* pinned host memory for the caller's batch buffers (the reference's seqBuffer/lenBuffer role,
  * prlHashReads.c:387-395); plain pageable memory also works with push_reads, only slower */
 int sdtgpu_host_alloc (void **out, size_t bytes);

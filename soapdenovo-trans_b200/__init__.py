@@ -11,7 +11,7 @@ The directory name contains a hyphen, so import it through `load()` in the repo-
 """
 from . import synth  # noqa: F401
 from .pregraph import (  # noqa: F401
-    ARC_DTYPE, DeviceReadPacker, EDGE_COUNTS, EDGE_CYCLE, EDGE_DTYPE, EDGE_PALINDROME, HIT_DTYPE, HIT_FOUND, HIT_RC, HIT_WINDOW, LIB_PATH, NODE_DTYPE, PregraphGPU, ReadPacker, STEP_DTYPE, STEP_NONE,
+    ARC_DTYPE, DeviceReadPacker, EDGE_COUNTS, EDGE_CYCLE, EDGE_DTYPE, EDGE_PALINDROME, HIT_DTYPE, HIT_FOUND, HIT_RC, HIT_WINDOW, LIB_PATH, NODE_DTYPE, PRUNE_COUNTS, PRUNE_MINOR_TIPS, PRUNE_SINGLE_TIPS, PregraphGPU, ReadPacker, STEP_DTYPE, STEP_NONE,
     SdtGpuError, build_library,
     edge_codes, hash_kmer, hits_numpy, library, nodes_to_records, read_kmersets, steps_numpy,
 )

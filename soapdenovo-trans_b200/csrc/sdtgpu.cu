@@ -10,6 +10,7 @@
 #include "sdt_route.cuh"
 #include "sdt_edges.cuh"
 #include "sdt_paths.cuh"
+#include "sdt_prune.cuh"
 
 #include <algorithm>
 #include <cstdio>
@@ -117,6 +118,10 @@ struct sdtgpu
 	size_t pa_cap[PA_N] = {};	// bytes
 	bool pa_ready = false, pa_arcs = false;	// stamps of the last build (counters zeroed with them); arcs built since
 	u64 pa_n_arcs = 0;
+	// pruning (sdt_prune.cuh): counters, marks and clear masks; grows only, freed by reset and destroy
+	void *pr = nullptr;
+	size_t pr_cap = 0;	// bytes
+	bool pruned = false;	// the table has been pruned since finalize: at most once
 	// sliced build (SDTGPU_F_SLICED): reads of the open epoch are kept in a log and turned into super-k-mer
 	// records in the chains of their slices as they arrive; sliced_flush merges copies and builds the slices
 	bool sliced = false, table_built = false, epoch_open = false, emitted = false, ord_bound_set = false, chains_dropped = false;
@@ -1409,6 +1414,10 @@ int sliced_push (sdtgpu *h, const ReadBatch &rb, u64 upper)
 
 u64 iter_slots (const sdtgpu *h) { return h->sliced ? h->n_store : h->cap; }
 
+// the -d the readers of the table are given (they test deletion as deLowKmer > 0 && L == 0 && R == 0): after a prune
+// every node without a non-zero counter is deleted, whatever -d finalize had
+int deleted_cutoff (const sdtgpu *h) { return h->pruned ? std::max (h->deLowKmer, 1) : h->deLowKmer; }
+
 static_assert (sizeof (Hit) == sizeof (sdtgpu_hit) && SDTGPU_HIT_WINDOW == HIT_WINDOW && SDTGPU_HIT_FOUND == HIT_FOUND && SDTGPU_HIT_RC == HIT_RC, "sdtgpu_hit");
 
 void free_index (sdtgpu *h)
@@ -1479,7 +1488,7 @@ Lookup make_lookup (const sdtgpu *h, sdtgpu_hit *d_out)
 	lk.index = h->index;
 	lk.idx_cap = h->idx_cap;
 	lk.out = reinterpret_cast<Hit *> (d_out);
-	lk.deLowKmer = h->deLowKmer;
+	lk.deLowKmer = deleted_cutoff (h);
 	return lk;
 }
 
@@ -1536,6 +1545,9 @@ void free_edges (sdtgpu *h)
 		h->pa_cap[i] = 0;
 	}
 	h->pa_ready = h->pa_arcs = false;
+	cudaFree (h->pr);
+	h->pr = nullptr;
+	h->pr_cap = 0;
 }
 
 // a finalized table, at most ROUTE_MAX_WORLD ranks, the small count buffers, and the index: a rank that stages
@@ -1667,8 +1679,9 @@ template <int W> int edges_build_t (sdtgpu *h, uint64_t out[8], double *ms)
 	g.idx_cap = h->idx_cap;
 	g.slots = slots;
 	g.K = h->K;
-	g.deLowKmer = h->deLowKmer;
-	g.max_m = 2 * h->h_ctr->n_linear + 2;	// a palindromic edge holds its nodes twice
+	g.deLowKmer = deleted_cutoff (h);
+	// a palindromic edge holds its nodes twice; a prune makes junctions linear, so finalize's linear count no longer bounds
+	g.max_m = 2 * (h->pruned ? h->h_ctr->n_nodes : h->h_ctr->n_linear) + 2;
 	auto bind = [&] () {
 		g.step = static_cast<Step *> (h->ed[ED_STEP]);
 		g.mark = static_cast<unsigned char *> (h->ed[ED_MARK]);
@@ -1930,6 +1943,88 @@ template <int W> int arcs_build_t (sdtgpu *h, uint64_t out[2], double *ms)
 	return SDTGPU_OK;
 }
 
+// ---- pruning (sdt_prune.cuh)
+template <int W> int prune_t (sdtgpu *h, int minor_pct, unsigned flags, uint64_t out[8], double *ms)
+{
+	typedef typename SlotOf<W>::type S;
+	S *tab = static_cast<S *> (h->table);
+	const u64 slots = iter_slots (h);
+	const size_t per = (slots + 3) & ~3ull;	// the masks start on a word
+	int rc = grow_device (h, &h->pr, &h->pr_cap, 0, 8 * sizeof (u64) + 2 * std::max<size_t> (per, 4), "pruning");
+	if (rc)
+		return rc;
+	Prune g = {};
+	g.index = h->index;
+	g.idx_cap = h->idx_cap;
+	g.ctr = static_cast<u64 *> (h->pr);
+	g.mark = reinterpret_cast<unsigned char *> (g.ctr + 8);
+	g.mask = reinterpret_cast<u32 *> (g.mark + per);
+	g.slots = slots;
+	g.K = h->K;
+	g.minor_pct = minor_pct;
+	const unsigned grid = (unsigned) std::min<u64> ((slots + BLOCK - 1) / BLOCK, (u64) h->sm_count * 16);
+	// the table changes from here on: the edge build, its stamps and its arcs describe the old one
+	h->ed_built = false;
+	h->pa_ready = h->pa_arcs = false;
+	h->pruned = true;
+	EdgeSpans sp (h);
+	sp.mark ();
+	CK (h, cudaMemsetAsync (h->pr, 0, 8 * sizeof (u64) + 2 * per, h->stream));
+	// one round: decide from the table as it is, then unlink and apply; phase < 0 only counts
+	auto round = [&] (int phase) -> int {
+		g.phase = std::max (phase, 0);
+		if (grid)
+		{
+			if (phase == 0)
+				prune_decide_kernel<W, 0><<<grid, BLOCK, 0, h->stream>>> (tab, g);
+			else if (phase == 1)
+				prune_decide_kernel<W, 1><<<grid, BLOCK, 0, h->stream>>> (tab, g);
+			else if (phase == 2)
+				prune_decide_kernel<W, 2><<<grid, BLOCK, 0, h->stream>>> (tab, g);
+			if (phase >= 0)
+				prune_unlink_kernel<W><<<grid, BLOCK, 0, h->stream>>> (tab, g);
+		}
+		CK (h, cudaMemsetAsync (g.ctr + 5, 0, 2 * sizeof (u64), h->stream));
+		if (grid)
+			prune_apply_kernel<W><<<grid, BLOCK, 0, h->stream>>> (tab, g);
+		CK (h, cudaGetLastError ());
+		return SDTGPU_OK;
+	};
+	const bool any = minor_pct > 0 || (flags & (SDTGPU_PRUNE_SINGLE_TIPS | SDTGPU_PRUNE_MINOR_TIPS));
+	if ((minor_pct > 0 && (rc = round (0))) || ((flags & SDTGPU_PRUNE_SINGLE_TIPS) && (rc = round (1))) || (!any && (rc = round (-1))))
+		return rc;
+	sp.mark ();
+	u64 c[8] = {}, rounds = 0;
+	auto read = [&] () -> int {
+		CK (h, cudaMemcpyAsync (c, g.ctr, sizeof c, cudaMemcpyDeviceToHost, h->stream));
+		CK (h, cudaStreamSynchronize (h->stream));
+		return SDTGPU_OK;
+	};
+	if ((rc = read ()))
+		return rc;
+	if (flags & SDTGPU_PRUNE_MINOR_TIPS)
+		for (u64 prev = c[3];; prev = c[3])
+		{	// until a round cuts nothing: the host reads the counters after each
+			sp.mark ();
+			if ((rc = round (2)))
+				return rc;
+			sp.mark ();
+			rounds++;
+			if ((rc = read ()))
+				return rc;
+			if (c[3] == prev)
+				break;
+		}
+	for (int i = 0; i < 4; i++)
+		out[i] = c[i];
+	out[4] = rounds;
+	out[5] = c[5];
+	out[6] = c[6];
+	out[7] = c[5] - c[6];
+	*ms = sp.ms ();
+	return SDTGPU_OK;
+}
+
 }	// namespace
 
 // =================================================================================================
@@ -2076,7 +2171,7 @@ int sdtgpu_reset (sdtgpu_t *h)
 		return SDTGPU_EINVAL;
 	CK (h, cudaSetDevice (h->device));
 	Trace tr (h);
-	if (h->index || h->rt_q || h->rt_aq || h->rt_back || h->ed[ED_STEP])
+	if (h->index || h->rt_q || h->rt_aq || h->rt_back || h->ed[ED_STEP] || h->pr)
 	{
 		CK (h, cudaStreamSynchronize (h->stream));	// (a lookup may still be reading them)
 		free_index (h);
@@ -2122,7 +2217,7 @@ int sdtgpu_reset (sdtgpu_t *h)
 		if (rc)
 			return rc;
 	}
-	h->pushed_upper = 0; h->n_reads = 0; h->ord_end = 0; h->finalized = false; h->deLowKmer = 0;
+	h->pushed_upper = 0; h->n_reads = 0; h->ord_end = 0; h->finalized = false; h->deLowKmer = 0; h->pruned = false;
 	if (h->snap_pending)
 		CK (h, cudaEventSynchronize (h->snap_ev));
 	h->snap_pending = false;
@@ -2572,9 +2667,9 @@ int sdtgpu_export_nodes (sdtgpu_t *h, int thrd_num, int sort_by_ordinal, sdtgpu_
 	const unsigned grid = (unsigned) std::min<u64> ((slots + BLOCK - 1) / BLOCK, (u64) h->sm_count * 8);
 	switch (h->W)
 	{
-	case 1: export_kernel<1><<<grid, BLOCK, 0, h->stream>>> (static_cast<const Slot1 *> (h->table), slots, h->key_words, thrd_num, h->deLowKmer, d_out, n, h->d_ctr); break;
-	case 2: export_kernel<2><<<grid, BLOCK, 0, h->stream>>> (static_cast<const Slot2 *> (h->table), slots, h->key_words, thrd_num, h->deLowKmer, d_out, n, h->d_ctr); break;
-	default: export_kernel<4><<<grid, BLOCK, 0, h->stream>>> (static_cast<const Slot4 *> (h->table), slots, h->key_words, thrd_num, h->deLowKmer, d_out, n, h->d_ctr); break;
+	case 1: export_kernel<1><<<grid, BLOCK, 0, h->stream>>> (static_cast<const Slot1 *> (h->table), slots, h->key_words, thrd_num, deleted_cutoff (h), d_out, n, h->d_ctr); break;
+	case 2: export_kernel<2><<<grid, BLOCK, 0, h->stream>>> (static_cast<const Slot2 *> (h->table), slots, h->key_words, thrd_num, deleted_cutoff (h), d_out, n, h->d_ctr); break;
+	default: export_kernel<4><<<grid, BLOCK, 0, h->stream>>> (static_cast<const Slot4 *> (h->table), slots, h->key_words, thrd_num, deleted_cutoff (h), d_out, n, h->d_ctr); break;
 	}
 	h->all_launches++;
 	cudaError_t e = cudaGetLastError ();
@@ -2993,6 +3088,33 @@ int sdtgpu_arcs_clear (sdtgpu_t *h)
 	if (!fresh)	// (stamps just made come with zero counters)
 		CK (h, cudaMemsetAsync (h->pa[PA_CTR], 0, std::max<u64> (h->ed_n_starts, 1) * 16, h->stream));
 	return SDTGPU_OK;
+}
+
+int sdtgpu_prune (sdtgpu_t *h, int minor_pct, unsigned flags, uint64_t out[8], double *ms)
+{
+	if (!h)
+		return SDTGPU_EINVAL;
+	if (!out || !ms)
+		return fail (h, SDTGPU_EINVAL, "sdtgpu_prune: NULL output");
+	if (minor_pct < 0 || minor_pct > 100)
+		return fail (h, SDTGPU_EINVAL, "sdtgpu_prune: minor_pct must be in 0..100");
+	if (flags & ~(SDTGPU_PRUNE_SINGLE_TIPS | SDTGPU_PRUNE_MINOR_TIPS))
+		return fail (h, SDTGPU_EINVAL, "sdtgpu_prune: unknown flag");
+	if (make_route (h).kind != ROUTE_ONE)
+		return fail (h, SDTGPU_EINVAL, "sdtgpu_prune: the handle holds one rank's share of a sharded table");
+	int rc = lookup_prologue (h, nullptr);
+	if (rc)
+		return rc;
+	if (h->pruned)
+		return fail (h, SDTGPU_ESTATE, "sdtgpu_prune: the table has been pruned already");
+	if ((rc = ensure_index (h)))
+		return rc;
+	switch (h->W)
+	{
+	case 1: return prune_t<1> (h, minor_pct, flags, out, ms);
+	case 2: return prune_t<2> (h, minor_pct, flags, out, ms);
+	default: return prune_t<4> (h, minor_pct, flags, out, ms);
+	}
 }
 
 int sdtgpu_host_alloc (void **out, size_t bytes)

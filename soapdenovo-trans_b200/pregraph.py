@@ -35,6 +35,9 @@ STEP_NONE = 0xFFFFFFFF
 ARC_DTYPE = np.dtype([("from", "<u4"), ("to", "<u4"), ("count", "<u4"), ("unused", "<u4")])
 assert ARC_DTYPE.itemsize == 16
 EDGE_COUNTS = ("edges", "palindromes", "cycles", "bases", "vertices", "linear_on_edges", "linear_on_cycles", "dangling")
+# sdtgpu_prune's out[] and flags (include/sdtgpu.h)
+PRUNE_COUNTS = ("minor_branches", "single_tips", "minor_tips", "tips", "rounds", "live", "linear", "vertices")
+PRUNE_SINGLE_TIPS, PRUNE_MINOR_TIPS = 1, 2
 
 F_NKMER = 1
 F_SLICED = 4
@@ -63,7 +66,7 @@ class KmerSet(C.Structure):
 def build_library(force: bool = False) -> str:
     """Compiles csrc/ + host/ for sm_100a into libsdtgpu.so (in-tree, so it travels to the GPU box)."""
     srcs = [os.path.join(PKG_DIR, p) for p in ("csrc/sdtgpu.cu", "csrc/sdt_synth.cu", "csrc/sdt_device.cuh",
-                                               "csrc/sdt_kernels.cuh", "csrc/sdt_sliced.cuh", "csrc/sdt_skm.cuh", "csrc/sdt_build.cuh", "csrc/sdt_lookup.cuh", "csrc/sdt_route.cuh", "csrc/sdt_edges.cuh", "csrc/sdt_paths.cuh", "csrc/sdt_nccl.cu", "csrc/sdt_parse.cu", "host/kmerset_builder.cpp", "host/sdt_readpack.c", "../include/sdtpack.h",
+                                               "csrc/sdt_kernels.cuh", "csrc/sdt_sliced.cuh", "csrc/sdt_skm.cuh", "csrc/sdt_build.cuh", "csrc/sdt_lookup.cuh", "csrc/sdt_route.cuh", "csrc/sdt_edges.cuh", "csrc/sdt_paths.cuh", "csrc/sdt_prune.cuh", "csrc/sdt_nccl.cu", "csrc/sdt_parse.cu", "host/kmerset_builder.cpp", "host/sdt_readpack.c", "../include/sdtpack.h",
                                                "../include/sdtgpu.h")]
     stale = (not os.path.exists(LIB_PATH)) or any(os.path.getmtime(s) > os.path.getmtime(LIB_PATH) for s in srcs)
     if force or stale:
@@ -141,6 +144,7 @@ def library() -> C.CDLL:
     L.sdtgpu_arcs_build.argtypes = [vp, C.POINTER(u64), C.POINTER(C.c_double)]
     L.sdtgpu_arcs_buffers.argtypes = [vp, C.POINTER(vp)]
     L.sdtgpu_arcs_clear.argtypes = [vp]
+    L.sdtgpu_prune.argtypes = [vp, i32, C.c_uint, C.POINTER(u64), C.POINTER(C.c_double)]
     L.sdtgpu_last_ordinals.argtypes = [vp, i32, vp]
     L.sdtgpu_kernel_times.argtypes = [vp, i32, C.POINTER(C.c_double), C.POINTER(u64)]
     L.sdtgpu_phase_times.argtypes = [vp, i32, C.POINTER(C.c_double), C.POINTER(u64)]
@@ -512,6 +516,19 @@ class PregraphGPU:
 
     def arcs_clear(self):
         self._ck(self.L.sdtgpu_arcs_clear(self.h))
+
+    # ---- the table pruned of minor branches and tips (include/sdtgpu.h sdtgpu_prune)
+    def prune(self, minor_pct: int = 5, single_tips=None, minor_tips: bool = True) -> dict:
+        """Prunes the finalized table once, with the reference's defaults -> the eight counts of sdtgpu_prune
+        (PRUNE_COUNTS) and ms, its device time.  single_tips=None: on when finalize had -d 0, as call_pregraph does."""
+        if single_tips is None:
+            single_tips = self.lookup_route()["deLowKmer"] == 0
+        flags = (PRUNE_SINGLE_TIPS if single_tips else 0) | (PRUNE_MINOR_TIPS if minor_tips else 0)
+        out, ms = (C.c_uint64 * 8)(), C.c_double()
+        self._ck(self.L.sdtgpu_prune(self.h, minor_pct, flags, out, C.byref(ms)))
+        res = {k: int(v) for k, v in zip(PRUNE_COUNTS, out)}
+        res["ms"] = float(ms.value)
+        return res
 
     # ---- lookups routed to the rank that owns each k-mer (include/sdtgpu.h sdtgpu_lookup_stage_* ... _exchange)
     def lookup_route(self) -> dict:
